@@ -7,10 +7,12 @@ One "step" = one fused forward/backward/update pass of the hot path over one bat
 cfg2|cfg3|cfg4|cfg5|cfg1`` select BASELINE.json's configs.  At N=1 a short cfg2 (configs[1]) measurement rides along as
 ``extra.cfg2``.
 
-Timing: W warm-up steps, then rounds of EXACTLY K steps (CUDA events on the launching stream, barrier + synchronize on
-both sides, max over ranks) repeated until ``--min-time`` seconds (default 0.5) of device time have been timed;
-``ms_per_step`` / ``value`` are the MEDIAN round.  ``--check`` (default on) runs one step of a small sharded problem
-outside the timed region and compares cost and every parameter's gradient with the float64 oracle (``parity_ok``).
+Timing: W warm-up steps, then one round of EXACTLY K timed steps (CUDA events on the launching stream, barrier +
+synchronize on both sides, max over ranks).  ``--min-time S`` repeats the K-step round until S seconds of device time have
+been timed and reports the MEDIAN round.  ``--check`` (default on) runs one step of a small sharded problem outside the
+timed region and compares cost and every parameter's gradient with the float64 oracle (``parity_ok``).
+``--dump-outputs DIR`` writes the parameters after the last timed step as DIR/<name>.npy (see ``_dump_outputs``); the
+inputs depend on the arguments only, so two builds run with the same arguments can be compared array for array.
 
   python bench.py --gpus N --steps K --warmup W            our arm  (N>1: launched by torch.distributed.run)
   python bench.py --impl reference --gpus N --steps K ...  reference arm: the reference's CPU path (NumPy float64 port of
@@ -311,9 +313,35 @@ def _parity_check(args, rank, world, local_rank, dist):
     return res
 
 
-def _measure(args, wl, wl_name, rank, world, local_rank, dist, steps, warmup, min_time, with_e2e=True, with_phases=True):
+DUMP_MAX_ELEMS = 2 << 20       # per array: 8 MB of float32; at most 7 parameters, so a dump stays under 64 MB
+
+
+def _dump_outputs(out_dir, params, data, neg1, neg2, b, B):
+    """The parameters after the last timed step (what the caller of the training step gets back: they are updated in
+    place) as ``out_dir/<name>.npy``, float32.  Of the row tables only the rows batch ``b`` (the last step's) touched are
+    kept: its feature rows of W, its argument and negative rows of A and Ab.  An array of more than DUMP_MAX_ELEMS
+    elements is cut to a fixed, seeded sample of those rows (tables) or of its elements (dense parameters)."""
+    os.makedirs(out_dir, exist_ok=True)
+    lo, hi = b * B, (b + 1) * B
+    ent = np.concatenate([data.args1[lo:hi], data.args2[lo:hi], neg1[:, lo:hi].ravel(), neg2[:, lo:hi].ravel()])
+    rows = {"W": np.unique(data.indices[data.indptr[lo]:data.indptr[hi]]), "A": np.unique(ent), "Ab": np.unique(ent)}
+    for name, a in params.items():
+        if name in rows:
+            r = rows[name]
+            width = int(np.prod(a.shape[1:]))
+            if r.size * width > DUMP_MAX_ELEMS:
+                r = np.sort(np.random.default_rng(0).choice(r, DUMP_MAX_ELEMS // width, replace=False))
+            a = a[r]
+        elif a.size > DUMP_MAX_ELEMS:
+            a = a.ravel()[np.sort(np.random.default_rng(0).choice(a.size, DUMP_MAX_ELEMS, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float32))
+
+
+def _measure(args, wl, wl_name, rank, world, local_rank, dist, steps, warmup, min_time, with_e2e=True, with_phases=True,
+             dump_dir=None):
     """Throughput of one workload: device-resident, end to end, per-phase.  Returns (line fragment dict, engine params for
-    the CPU leg or None, data tuple)."""
+    the CPU leg or None, data tuple).  With ``dump_dir`` the parameters after the device-resident timed steps are written
+    there (``_dump_outputs``)."""
     import torch
 
     from relation_autoencoder_b200.engine import Engine
@@ -391,6 +419,11 @@ def _measure(args, wl, wl_name, rank, world, local_rank, dist, steps, warmup, mi
     ms_dev, _, rounds_dev = timed(lambda b: eng.train_device(b, want_cost=False), 0, min_time)
     clocks = sampler.stop() if rank == 0 else None
     st = eng.stats()
+    if dump_dir:
+        params_after = eng.get_params_numpy()          # collective for N > 1
+        if rank == 0:
+            _dump_outputs(dump_dir, params_after, data, neg1, neg2, (warmup + len(rounds_dev) * steps - 1) % nb, B)
+        del params_after
     # ---- (2) end to end through the reference-facing call: host negatives in, cost out, every step ----
     ms_e2e = None
     if with_e2e:
@@ -499,7 +532,7 @@ def _run_ours(args, wl, rank, world, local_rank):
     parity = _parity_check(args, rank, world, local_rank, dist) if args.check else None
     tf32_peak = _measure_tf32_peak(dev) if rank == 0 else None
     frag, st, phase_ms, p_cpu, (data, neg1, neg2) = _measure(args, wl, args.workload, rank, world, local_rank, dist, steps, warmup,
-                                                             args.min_time)
+                                                             args.min_time, dump_dir=args.dump_outputs)
     extra = {}
     if world == 1 and args.workload != "cfg2" and not args.no_extra:
         wl2 = dict(SY.WORKLOADS["cfg2"])
@@ -653,7 +686,8 @@ def main():
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", choices=["ours", "reference"], default="ours")
     ap.add_argument("--workload", choices=sorted(SY.WORKLOADS), default="T")
-    ap.add_argument("--min-time", type=float, default=0.5, help="repeat the K-step round until this many seconds are timed")
+    ap.add_argument("--min-time", type=float, default=0.0, help="repeat the K-step round until this many seconds are timed "
+                    "(0: one round, exactly K timed steps)")
     ap.add_argument("--max-rounds", type=int, default=400)
     ap.add_argument("--check", dest="check", action="store_true", default=True, help="parity check of one small sharded step (default)")
     ap.add_argument("--no-check", dest="check", action="store_false")
@@ -665,7 +699,11 @@ def main():
     ap.add_argument("--engine-flags", type=int, default=0, help="extra RAE_FLAG_* bits for the 1-GPU engine (4 = force the SIMT contraction)")
     ap.add_argument("--no-pdl", action="store_true", help="RAE_FLAG_NO_PDL: plain stream-order launches (A/B of programmatic dependent launch)")
     ap.add_argument("--cpu-budget", type=float, default=45.0, help="seconds of CPU work allowed for the CPU legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="write the parameters after the last timed step as "
+                    "DIR/<name>.npy (float32, a fixed sample of the rows the last step touched; under 64 MB in all)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the timed GPU path computed: --impl ours only")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -44,6 +44,38 @@ def test_roofline_terms_and_tensor_table():
     assert b._tensor_kernels(dict(SY.WORKLOADS["cfg4"]), {"tensor_path": 0}, PHASES_T, pk, 740.0) is None
 
 
+def test_dump_outputs_keeps_the_last_batch_rows_under_the_cap(tmp_path, monkeypatch):
+    """--dump-outputs: float32 arrays named after the parameters; the row tables keep the rows the given batch touched,
+    cut to a fixed sample when an array would exceed the per-array cap; two dumps of the same state are identical."""
+    import numpy as np
+    b = _bench()
+    from relation_autoencoder_b200 import synthetic as SY
+    F, N, K, d, S, B = 3000, 700, 6, 5, 3, 40
+    data = SY.make_dataset(4 * B, F, N, 10, seed=3)
+    rng = np.random.RandomState(2)
+    params = SY.init_params(rng, "rescal+sp", F, K, N, d)
+    params["Ab"] = np.arange(N, dtype=np.float32)            # a row's value is its id
+    neg1, neg2 = SY.draw_negatives(rng, data.neg_cum, data.n, S)
+    monkeypatch.setattr(b, "DUMP_MAX_ELEMS", 100)
+    for out in ("a", "b"):
+        b._dump_outputs(str(tmp_path / out), params, data, neg1, neg2, 2, B)
+    lo, hi = 2 * B, 3 * B
+    w_rows = np.unique(data.indices[data.indptr[lo]:data.indptr[hi]])
+    e_rows = np.unique(np.concatenate([data.args1[lo:hi], data.args2[lo:hi], neg1[:, lo:hi].ravel(), neg2[:, lo:hi].ravel()]))
+    assert w_rows.size * K > 100 and e_rows.size > 100
+    got = {n: np.load(str(tmp_path / "a" / (n + ".npy"))) for n in params}
+    for n, a in got.items():
+        assert a.dtype == np.float32 and a.size <= 100, n
+        assert np.array_equal(a, np.load(str(tmp_path / "b" / (n + ".npy")))), n
+    assert got["W"].shape == (100 // K, K) and got["A"].shape == (100 // d, d) and got["Ab"].shape == (100,)
+    # every dumped table row is one the batch touched
+    w_table = {tuple(r) for r in params["W"][w_rows]}
+    assert all(tuple(r) in w_table for r in got["W"])
+    assert set(got["Ab"].astype(np.int64).tolist()) <= set(e_rows.tolist())
+    assert np.array_equal(got["Wb"], params["Wb"]) and got["C"].shape == (100,)
+    assert set(got["C"].tolist()) <= set(params["C"].ravel().tolist())
+
+
 def test_reference_arm_prints_a_complete_line():
     """`bench.py --impl reference` (the NumPy float64 port of the reference's CPU path; the README-size config keeps it short)."""
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--workload", "cfg1", "--steps", "2",
