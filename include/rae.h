@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define RAE_ABI_VERSION 1
+#define RAE_ABI_VERSION 2
 
 /* decoder selection: construct_decoder(model_type, ...) learning/models/decoders/Decoder.py:84-93 */
 #define RAE_MODEL_A 0  /* 'rescal'    Bilinear.py               */
@@ -148,30 +148,17 @@ int rae_train_step_explicit(rae_engine* h, const int32_t* indptr, const int32_t*
                             double* cost_host, void* stream);
 
 /* ---- multi-GPU building blocks (SURVEY 8e): the reference has no counterpart (single process, no device) ----------
- * Data parallel over examples; dense parameters (C, C1, C2, Wb) replicated and their gradients all-reduced by the caller
- * (NCCL) between _begin and _end; W / A / Ab row-sharded by owner = row mod world.  A rank fetches the rows its batch
- * touches into compact tables (rae_gather_rows on the owner + all-to-all), runs the step with RAE_FLAG_EMIT_ONLY so the
- * kernels emit one reduced gradient row per compact row, returns those rows to the owners, and each owner applies them
- * with rae_sparse_rows_apply: stable sort by (row, source rank order), segment-reduce, one optimiser RMW per row. */
+ * The row-sharded step of the peer-memory path below (relation_autoencoder_b200/dist.py) binds a rank's compact gradient
+ * buffers and flat dense gradient with rae_bind_grad_buffers and runs its local step as rae_train_step_begin, then
+ * rae_train_step_end around the dense-gradient all-reduce.  It copies the local cost for the cross-rank sum with
+ * rae_copy_cost and labels a split's rows on their compact feature slots with rae_label_explicit. */
 /* caller-owned output buffers for the emitted gradients: gW[F,K], gA[N,d], gAb[N] (F, N = compact capacities) and the
  * flat dense gradient [C | C1 | C2 | Wb] (rae_dense_grad_size floats).  NULL keeps the internal buffer. */
 int rae_bind_grad_buffers(rae_engine* h, float* gW, float* gA, float* gAb, float* dense);
 int64_t rae_dense_grad_size(const rae_engine* h);
-/* first part of a step on explicit device inputs: everything except the dense-parameter optimiser update; the flat
- * dense gradient is complete when the stream reaches this point (all-reduce it, then call _end). */
-int rae_train_step_begin_explicit(rae_engine* h, const int32_t* indptr, const int32_t* indices, int64_t nnz,
-                                  const int32_t* args1, const int32_t* args2, const int32_t* neg1, const int32_t* neg2,
-                                  int64_t neg_ld, void* stream);
 int rae_train_step_end(rae_engine* h, void* stream);
 /* synchronise and read the last step's (local) cost */
 int rae_read_cost(rae_engine* h, double* cost_host, void* stream);
-/* out[i, :] = table[rows[i], :]  (owner-side fetch of requested rows; width floats per row) */
-int rae_gather_rows(rae_engine* h, const float* table, int64_t width, const int32_t* rows, int64_t n, float* out,
-                    void* stream);
-/* owner-side update: for every distinct r in rows[0..n): g = sum (in input order) of grads[i,:] with rows[i] == r, then the
- * handle's optimiser rule on table[r,:] / acc[r,:] (Optimizers.py:29-32 / :51).  n_table_rows bounds the row ids. */
-int rae_sparse_rows_apply(rae_engine* h, float* table, float* acc, int64_t width, const int32_t* rows, const float* grads,
-                          int64_t n, int64_t n_table_rows, void* stream);
 
 /* ---- peer-memory data path over NVLink / NVSwitch (one process per GPU, one node) ----------------------------------
  * The sharded tables and the per-rank compact gradient buffers live in cudaMalloc'ed memory exported with CUDA IPC, so a
@@ -202,8 +189,8 @@ int rae_pull_apply(rae_engine* h, float* table, float* acc, int64_t width, const
                    const int32_t* ent_src, const int32_t* ent_slot, int64_t n_rows, const void* const* grads, int32_t world,
                    void* stream);
 /* first part of a step on batch `batch_index` of the BOUND train split (cached transposed feature index) with explicit
- * device entity ids: args1/args2 [B], neg1/neg2 [S, neg_ld].  Like rae_train_step_begin_explicit, the dense optimiser
- * update is left to rae_train_step_end. */
+ * device entity ids: args1/args2 [B], neg1/neg2 [S, neg_ld]: everything except the dense-parameter optimiser update, which
+ * is left to rae_train_step_end (the flat dense gradient is complete when the stream reaches this point). */
 int rae_train_step_begin(rae_engine* h, int64_t batch_index, const int32_t* args1, const int32_t* args2, const int32_t* neg1,
                          const int32_t* neg2, int64_t neg_ld, void* stream);
 /* One row-sharded data-parallel step as TWO calls around the caller's dense-gradient all-reduce (everything the host

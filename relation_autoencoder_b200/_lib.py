@@ -13,7 +13,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("RAE_LIB") or os.path.join(HERE, "librae.so")    # RAE_LIB: A/B measurement of two builds
 HEADER_PATH = os.path.join(os.path.dirname(HERE), "include", "rae.h")
 
-RAE_ABI_VERSION = 1
+RAE_ABI_VERSION = 2
 RAE_MODEL_A, RAE_MODEL_C, RAE_MODEL_AC = 0, 1, 2
 RAE_OPT_ADAGRAD, RAE_OPT_SGD = 0, 1
 RAE_P_W, RAE_P_WB, RAE_P_A, RAE_P_AB, RAE_P_C, RAE_P_C1, RAE_P_C2 = range(7)
@@ -82,11 +82,8 @@ _SIGNATURES = {
     "rae_get_step_stats": (C.c_int, [_P, C.POINTER(RaeStepStats)]),
     "rae_bind_grad_buffers": (C.c_int, [_P, _P, _P, _P, _P]),
     "rae_dense_grad_size": (C.c_int64, [_P]),
-    "rae_train_step_begin_explicit": (C.c_int, [_P, _P, _P, C.c_int64, _P, _P, _P, _P, C.c_int64, _P]),
     "rae_train_step_end": (C.c_int, [_P, _P]),
     "rae_read_cost": (C.c_int, [_P, C.POINTER(C.c_double), _P]),
-    "rae_gather_rows": (C.c_int, [_P, _P, C.c_int64, _P, C.c_int64, _P, _P]),
-    "rae_sparse_rows_apply": (C.c_int, [_P, _P, _P, C.c_int64, _P, _P, C.c_int64, C.c_int64, _P]),
     "rae_peer_alloc": (C.c_int, [C.c_int64, C.POINTER(_P), _P]),
     "rae_peer_free": (C.c_int, [_P]),
     "rae_peer_open": (C.c_int, [_P, C.POINTER(_P)]),

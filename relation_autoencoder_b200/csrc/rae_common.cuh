@@ -81,6 +81,16 @@ __device__ __forceinline__ void adagrad_apply(float& p, float& acc, float g, flo
     p = fmaf(-lr * g, inv, p);
 }
 
+// the handle's optimiser rule on one element: AdaGrad (above) or SGD, Optimizers.py:51 (p' = p - lr*g; acc untouched)
+__device__ __forceinline__ void opt_step(float& w, float& a, float g, float lr, int adagrad) {
+    if (adagrad) adagrad_apply(w, a, g, lr);
+    else w -= lr * g;
+}
+__device__ __forceinline__ void opt_step(float4& w, float4& a, const float4& g, float lr, int adagrad) {
+    opt_step(w.x, a.x, g.x, lr, adagrad); opt_step(w.y, a.y, g.y, lr, adagrad);
+    opt_step(w.z, a.z, g.z, lr, adagrad); opt_step(w.w, a.w, g.w, lr, adagrad);
+}
+
 // v[b,j], w[b,j] of the tensor-core contraction from its partial buffers (rae_decoder_tc.cu):
 //   vg [2][B][dp]          DP=128: both epilogue groups hold a half-row partial; DP=64: group j%2; DP=32: group (j/2)%2
 //   wp [slot][2][B][dp]    sum over the NS = tcs_nslots(schedule, b / 128) slots of the example's tile of the group

@@ -736,15 +736,6 @@ int rae_bind_grad_buffers(rae_engine* h, float* gW, float* gA, float* gAb, float
 
 int64_t rae_dense_grad_size(const rae_engine* h) { return h ? h->n_dense : 0; }
 
-int rae_train_step_begin_explicit(rae_engine* h, const int32_t* indptr, const int32_t* indices, int64_t nnz,
-                                  const int32_t* args1, const int32_t* args2, const int32_t* neg1, const int32_t* neg2,
-                                  int64_t neg_ld, void* stream) {
-    int rc = check_ready(h, false, false);
-    if (rc) return rc;
-    if (!indptr || !indices || !args1 || !args2 || nnz < 0) return fail(h, RAE_EINVAL, "rae_train_step_begin_explicit: bad argument");
-    return run_step(h, indptr, indices, nnz, args1, args2, neg1, neg2, neg_ld, nullptr, nullptr, (cudaStream_t)stream, false);
-}
-
 int rae_train_step_begin(rae_engine* h, int64_t batch_index, const int32_t* args1, const int32_t* args2, const int32_t* neg1,
                          const int32_t* neg2, int64_t neg_ld, void* stream) {
     int rc = check_ready(h, true, false);
@@ -786,30 +777,6 @@ int rae_train_step_end(rae_engine* h, void* stream) {
 int rae_read_cost(rae_engine* h, double* cost_host, void* stream) {
     if (!h || !cost_host) return RAE_EINVAL;
     return finish_cost(h, cost_host, (cudaStream_t)stream);
-}
-
-int rae_gather_rows(rae_engine* h, const float* table, int64_t width, const int32_t* rows, int64_t n, float* out,
-                    void* stream) {
-    if (!h || !table || (!rows && n > 0) || (!out && n > 0) || width < 1 || n < 0) return rae::fail(h, RAE_EINVAL, "rae_gather_rows: bad argument");
-    return launch_gather_rows(h, table, width, rows, n, out, (cudaStream_t)stream);
-}
-
-int rae_sparse_rows_apply(rae_engine* h, float* table, float* acc, int64_t width, const int32_t* rows, const float* grads,
-                          int64_t n, int64_t n_table_rows, void* stream) {
-    if (!h || !table || width < 1 || n < 0 || n_table_rows < 1) return rae::fail(h, RAE_EINVAL, "rae_sparse_rows_apply: bad argument");
-    if (h->adagrad && !acc) return rae::fail(h, RAE_EINVAL, "rae_sparse_rows_apply: AdaGrad needs the accumulator table");
-    if (n == 0) return RAE_OK;
-    if (!rows || !grads) return rae::fail(h, RAE_EINVAL, "rae_sparse_rows_apply: null rows/grads");
-    cudaStream_t st = (cudaStream_t)stream;
-    int rc = ensure_feat_capacity(h, n);
-    if (rc) return rc;
-    if ((rc = build_row_keys(h, rows, n, st))) return rc;
-    const int saved_bits = h->feat.key_bits;
-    h->feat.key_bits = bits_for(n_table_rows);
-    rc = sort_pairs(h, h->feat, n, st, h->cub_tmp, h->cub_bytes);
-    h->feat.key_bits = saved_bits;
-    if (rc) return rc;
-    return launch_rows_apply(h, table, acc, (int)width, h->feat.keys_s, h->feat.vals_s, grads, n, st);
 }
 
 int rae_get_probs(rae_engine* h, float* dst, void* stream) {

@@ -257,11 +257,6 @@ int launch_entity_update(rae_engine* h, const uint32_t* keys_s, const uint32_t* 
                          bool apply, cudaStream_t st);
 int launch_w_update(rae_engine* h, const uint32_t* keys_s, const uint32_t* vals_s, int64_t nnz, bool emit_dense,
                     bool apply, cudaStream_t st);
-int build_row_keys(rae_engine* h, const int32_t* rows, int64_t n, cudaStream_t st);      // keys = rows, vals = 0..n-1
-int launch_rows_apply(rae_engine* h, float* table, float* acc, int width, const uint32_t* keys_s, const uint32_t* vals_s,
-                      const float* grads, int64_t n, cudaStream_t st);
-int launch_gather_rows(rae_engine* h, const float* table, int64_t width, const int32_t* rows, int64_t n, float* out,
-                       cudaStream_t st);
 // ---- peer-memory path (rae_peer.cu) ----
 int launch_fetch_rows(rae_engine* h, const void* const* tables, int world, int64_t width, const int32_t* ids, int64_t n,
                       float* out, cudaStream_t st);

@@ -121,13 +121,8 @@ __global__ void __launch_bounds__(256) k_pull_apply(float* __restrict__ table, f
                     for (int u = 0; u < 4; ++u) { g.x += x[u].x; g.y += x[u].y; g.z += x[u].z; g.w += x[u].w; }
                 }
                 if (in) {
-                    if (adagrad) {
-                        adagrad_apply(w.x, a.x, g.x, lr); adagrad_apply(w.y, a.y, g.y, lr);
-                        adagrad_apply(w.z, a.z, g.z, lr); adagrad_apply(w.w, a.w, g.w, lr);
-                        reinterpret_cast<float4*>(acc + rowoff)[q0] = a;
-                    } else {
-                        w.x -= lr * g.x; w.y -= lr * g.y; w.z -= lr * g.z; w.w -= lr * g.w;
-                    }
+                    opt_step(w, a, g, lr, adagrad);
+                    if (adagrad) reinterpret_cast<float4*>(acc + rowoff)[q0] = a;
                     reinterpret_cast<float4*>(table + rowoff)[q0] = w;
                 }
             }
@@ -151,12 +146,8 @@ __global__ void __launch_bounds__(256) k_pull_apply(float* __restrict__ table, f
                     for (int u = 0; u < 4; ++u) g += x[u];
                 }
                 if (in) {
-                    if (adagrad) {
-                        adagrad_apply(w, a, g, lr);
-                        acc[rowoff + k] = a;
-                    } else {
-                        w -= lr * g;
-                    }
+                    opt_step(w, a, g, lr, adagrad);
+                    if (adagrad) acc[rowoff + k] = a;
                     table[rowoff + k] = w;
                 }
             }
@@ -183,14 +174,9 @@ __global__ void __launch_bounds__(256) k_pull_apply_scalars(float* __restrict__ 
             for (int u = 0; u < 4; ++u) g += x[u];
         }
         const int r = rows_local[i];
-        float w = table[r];
-        if (adagrad) {
-            float a = acc[r];
-            adagrad_apply(w, a, g, lr);
-            acc[r] = a;
-        } else {
-            w -= lr * g;
-        }
+        float w = table[r], a = adagrad ? acc[r] : 0.f;
+        opt_step(w, a, g, lr, adagrad);
+        if (adagrad) acc[r] = a;
         table[r] = w;
     }
 }
@@ -289,15 +275,10 @@ __global__ void __launch_bounds__(256) k_dense_apply_peers(DenseSegs segs, PeerP
             for (int k = 0; k < 4; ++k) {
                 if (k < segs.count && i >= segs.s[k].begin && i < segs.s[k].end) {
                     const size_t j = i - segs.s[k].begin;
-                    float4 w = *reinterpret_cast<const float4*>(segs.s[k].p + j);
-                    if (adagrad) {
-                        float4 a = *reinterpret_cast<const float4*>(segs.s[k].acc + j);
-                        adagrad_apply(w.x, a.x, g.x, lr); adagrad_apply(w.y, a.y, g.y, lr);
-                        adagrad_apply(w.z, a.z, g.z, lr); adagrad_apply(w.w, a.w, g.w, lr);
-                        *reinterpret_cast<float4*>(segs.s[k].acc + j) = a;
-                    } else {
-                        w.x -= lr * g.x; w.y -= lr * g.y; w.z -= lr * g.z; w.w -= lr * g.w;
-                    }
+                    float4 w = *reinterpret_cast<const float4*>(segs.s[k].p + j), a = make_float4(0.f, 0.f, 0.f, 0.f);
+                    if (adagrad) a = *reinterpret_cast<const float4*>(segs.s[k].acc + j);
+                    opt_step(w, a, g, lr, adagrad);
+                    if (adagrad) *reinterpret_cast<float4*>(segs.s[k].acc + j) = a;
                     *reinterpret_cast<float4*>(segs.s[k].p + j) = w;
                 }
             }
@@ -316,14 +297,9 @@ __global__ void __launch_bounds__(256) k_dense_apply_peers(DenseSegs segs, PeerP
         for (int k = 0; k < 4; ++k) {
             if (k < segs.count && i >= segs.s[k].begin && i < segs.s[k].end) {
                 const size_t j = i - segs.s[k].begin;
-                float w = segs.s[k].p[j];
-                if (adagrad) {
-                    float a = segs.s[k].acc[j];
-                    adagrad_apply(w, a, g, lr);
-                    segs.s[k].acc[j] = a;
-                } else {
-                    w -= lr * g;
-                }
+                float w = segs.s[k].p[j], a = adagrad ? segs.s[k].acc[j] : 0.f;
+                opt_step(w, a, g, lr, adagrad);
+                if (adagrad) segs.s[k].acc[j] = a;
                 segs.s[k].p[j] = w;
             }
         }

@@ -22,8 +22,12 @@ def record_err(test, name, value):
             f.write(json.dumps({"test": test, "what": name, "err": float(value)}) + "\n")
 
 
-def make_problem(model, B=12, K=5, d=6, S=3, F=40, N=25, fbar=4, seed=0, dup_heavy=False, empty_rows=False):
-    """Random tiny instance: params in reference init order + one batch with injected negatives."""
+def make_problem(model, B=12, K=5, d=6, S=3, F=40, N=25, fbar=4, seed=0, dup_heavy=False, empty_rows=False, hot_rows=False):
+    """Random tiny instance: params in reference init order + one batch with injected negatives.
+
+    hot_rows: feature ids 0-4 and entity ids 0-4 get fixed shares of the batch on top of the random draws - id 0 in every
+    example, id 1 in every 5th, ids 2-4 in every 14th each (at B = 512: 512, ~100 and ~37 occurrences), so that the
+    sparse-row update sees rows cut by one chunk boundary, rows over a few chunks and rows over many chunks."""
     rng = np.random.RandomState(seed)
     p = O.init_params(rng, model, F, K, N, d)
     # make biases / W non-trivial so every term is exercised
@@ -38,6 +42,8 @@ def make_problem(model, B=12, K=5, d=6, S=3, F=40, N=25, fbar=4, seed=0, dup_hea
         if empty_rows and b % 5 == 0:
             n = 0
         feats = np.sort(rng.choice(F, size=min(n, F), replace=False))
+        if hot_rows:
+            feats = np.union1d(feats, _hot_ids(b))
         indices.extend(feats.tolist())
         indptr.append(len(indices))
     hiN = max(2, N // 5) if dup_heavy else N
@@ -45,8 +51,19 @@ def make_problem(model, B=12, K=5, d=6, S=3, F=40, N=25, fbar=4, seed=0, dup_hea
     a2 = rng.randint(0, hiN, size=B).astype(np.int32)
     neg1 = rng.randint(0, hiN, size=(S, B)).astype(np.int32)
     neg2 = rng.randint(0, hiN, size=(S, B)).astype(np.int32)
+    if hot_rows:
+        b = np.arange(B)
+        a1[:] = 0
+        a2[b % 5 == 0] = 1
+        for k in range(3):
+            neg1[0, b % 14 == k] = 2 + k
     return dict(p=p, indptr=np.asarray(indptr, dtype=np.int32), indices=np.asarray(indices, dtype=np.int32),
                 a1=a1, a2=a2, neg1=neg1, neg2=neg2)
+
+
+def _hot_ids(b):
+    """The hot feature ids of example b (make_problem(hot_rows=True))."""
+    return [0] + ([1] if b % 5 == 0 else []) + [2 + k for k in range(3) if b % 14 == k]
 
 
 def torch_reference_cost(model, p, indptr, indices, a1, a2, neg1, neg2, alpha, l1, l2, adj, ext_reg):

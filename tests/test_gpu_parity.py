@@ -32,6 +32,10 @@ SHAPES = {
     "b512d128": dict(B=512, K=100, d=128, S=4, F=3000, N=900, fbar=20),  # 4 example tiles: cluster of 4, operand multicast
     "b256d30": dict(B=256, K=100, d=30, S=5, F=2000, N=700, fbar=30),    # 2 example tiles: cluster of 2
 }
+HOT_SHAPES = {      # batches for make_problem(hot_rows=True)
+    "k100d128": dict(B=512, K=100, d=128, S=4, F=3000, N=900, fbar=20),  # row widths multiples of 4: 16-byte row accesses
+    "k7d33": dict(B=512, K=7, d=33, S=4, F=3000, N=900, fbar=20),        # neither width a multiple of 4
+}
 
 
 def _engine(model, sh, flags=FLAG_DENSE, **kw):
@@ -45,8 +49,8 @@ def _to32(p):
 
 
 def _check_step(model, sh, seed=0, dup_heavy=False, empty_rows=False, l1=0.0, l2=0.0, ext_reg=True, alpha=1.0,
-                optimizer="adagrad", lr=0.1, steps=1, flags=FLAG_DENSE):
-    pr = make_problem(model, seed=seed, dup_heavy=dup_heavy, empty_rows=empty_rows, **sh)
+                optimizer="adagrad", lr=0.1, steps=1, flags=FLAG_DENSE, hot_rows=False):
+    pr = make_problem(model, seed=seed, dup_heavy=dup_heavy, empty_rows=empty_rows, hot_rows=hot_rows, **sh)
     p0 = _to32(pr["p"])
     names = O.param_names(model)
     adj = 0.37
@@ -143,22 +147,46 @@ def test_sgd(model):
     _check_step(model, SHAPES["tiny"], seed=8, optimizer="sgd", steps=2)
 
 
+def _chunk_spans(keys):
+    """Chunks of 32 positions that each row's segment covers in the stable sort by row (the row-update kernels' layout)."""
+    s = np.sort(keys, kind="stable")
+    starts = np.flatnonzero(np.r_[True, s[1:] != s[:-1]])
+    ends = np.r_[starts[1:], len(s)]
+    return (ends - 1) // 32 - starts // 32 + 1
+
+
+@pytest.mark.parametrize("optimizer", ["adagrad", "sgd"])
+@pytest.mark.parametrize("shape", list(HOT_SHAPES))
+@pytest.mark.parametrize("model", O.MODELS)
+def test_hot_rows_take_every_row_update_path(model, shape, optimizer):
+    """Rows of 2 chunks (feature rows: absorbed by level 1), of 3-9 chunks (level 2, one warp) and of 10 or more chunks
+    (level 2, the whole CTA), on both feature and entity rows, held to the oracle."""
+    sh = HOT_SHAPES[shape]
+    pr = make_problem(model, seed=13, hot_rows=True, **sh)
+    feature_keys = pr["indices"]
+    entity_keys = np.concatenate([pr["a1"], pr["a2"], pr["neg1"].reshape(-1), pr["neg2"].reshape(-1)])
+    for keys in (feature_keys, entity_keys):
+        spans = _chunk_spans(keys)
+        assert (spans == 2).any() and ((spans >= 3) & (spans <= 9)).any() and (spans >= 10).any(), np.bincount(spans)
+    _check_step(model, sh, seed=13, hot_rows=True, optimizer=optimizer)
+
+
 @pytest.mark.parametrize("model", O.MODELS)
 def test_production_path_without_dense_grads_matches_debug_path(model):
     """The flag that materialises dense gradients must not change the update (bitwise)."""
-    sh = SHAPES["k100d30"]
-    pr = make_problem(model, seed=9, dup_heavy=True, **sh)
-    res = []
-    for flags in (FLAG_DENSE, 0, 16):       # debug, production (cached feature index n/a for explicit), no cache
-        eng = _engine(model, sh, flags=flags)
-        eng.set_params_numpy(_to32(pr["p"]))
-        c = eng.train_explicit(pr["indptr"], pr["indices"], pr["a1"], pr["a2"], pr["neg1"], pr["neg2"])
-        res.append((c, eng.get_params_numpy(), eng.get_acc_numpy()))
-        eng.close()
-    for c, p, a in res[1:]:
-        assert c == res[0][0]
-        for n in p:
-            assert np.array_equal(p[n], res[0][1][n]) and np.array_equal(a[n], res[0][2][n]), n
+    for sh, pr in ((SHAPES["k100d30"], make_problem(model, seed=9, dup_heavy=True, **SHAPES["k100d30"])),
+                   (HOT_SHAPES["k7d33"], make_problem(model, seed=13, hot_rows=True, **HOT_SHAPES["k7d33"]))):
+        res = []
+        for flags in (FLAG_DENSE, 0, 16):       # debug, production (cached feature index n/a for explicit), no cache
+            eng = _engine(model, sh, flags=flags)
+            eng.set_params_numpy(_to32(pr["p"]))
+            c = eng.train_explicit(pr["indptr"], pr["indices"], pr["a1"], pr["a2"], pr["neg1"], pr["neg2"])
+            res.append((c, eng.get_params_numpy(), eng.get_acc_numpy()))
+            eng.close()
+        for c, p, a in res[1:]:
+            assert c == res[0][0]
+            for n in p:
+                assert np.array_equal(p[n], res[0][1][n]) and np.array_equal(a[n], res[0][2][n]), n
 
 
 def test_sort_segment_layout_is_bit_exact():
