@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define RAE_ABI_VERSION 2
+#define RAE_ABI_VERSION 3
 
 /* decoder selection: construct_decoder(model_type, ...) learning/models/decoders/Decoder.py:84-93 */
 #define RAE_MODEL_A 0  /* 'rescal'    Bilinear.py               */
@@ -69,7 +69,8 @@ extern "C" {
 #define RAE_FLAG_CLUSTER_MULTICAST 64u /* accepted and ignored: the cluster-multicast variant of the tcgen05 path measured no gain on
                                          * B200 (the kernels are not operand-traffic bound) and was removed */
 #define RAE_FLAG_NO_PDL 128u        /* launch the step's kernels in plain stream order (no programmatic dependent launch): A/B measurements */
-#define RAE_FLAG_EMIT_ONLY 32u      /* row-sharded multi-GPU: W/A/Ab are per-step compact copies; emit per-row gradients, apply nothing */
+#define RAE_FLAG_EMIT_ONLY 32u      /* row-sharded multi-GPU: W/A/Ab are per-step compact copies; emit per-row data gradients, apply
+                                      * nothing (with l1/l2 != 0 the owner adds W's regulariser, rae_shard_apply) */
 
 typedef struct rae_config {
     int32_t abi_version; /* RAE_ABI_VERSION */
@@ -188,6 +189,13 @@ int rae_fetch_rows(rae_engine* h, const void* const* tables, int32_t world, int6
 int rae_pull_apply(rae_engine* h, float* table, float* acc, int64_t width, const int32_t* rows_local, const int32_t* ent_off,
                    const int32_t* ent_src, const int32_t* ent_slot, int64_t n_rows, const void* const* grads, int32_t world,
                    void* stream);
+/* rae_pull_apply over EVERY row of a regularised table shard (shard_rows rows, local indices 0..shard_rows-1): for each
+ * element, in the order of the single-GPU dense update, g = the summed contributions when the row is in rows_local
+ * (ascending) else 0, then g += adj*(l1*sgn(p) + 2*l2*p) with the handle's adj / l1 / l2, then the optimiser rule - one
+ * read-modify-write of table and acc per element.  Rows no rank touched move too: the regulariser reaches every row. */
+int rae_shard_apply(rae_engine* h, float* table, float* acc, int64_t width, const int32_t* rows_local, const int32_t* ent_off,
+                    const int32_t* ent_src, const int32_t* ent_slot, int64_t n_rows, const void* const* grads, int32_t world,
+                    int64_t shard_rows, void* stream);
 /* first part of a step on batch `batch_index` of the BOUND train split (cached transposed feature index) with explicit
  * device entity ids: args1/args2 [B], neg1/neg2 [S, neg_ld]: everything except the dense-parameter optimiser update, which
  * is left to rae_train_step_end (the flat dense gradient is complete when the stream reaches this point). */
@@ -218,11 +226,17 @@ typedef struct rae_dist_step {
     const void* const* dense_bufs;                         /* every rank's flat dense gradient [C | C1 | C2 | Wb], or NULL:   */
     int32_t rank;                                          /*   NULL = the caller all-reduced the dense gradient itself      */
     int32_t global_cost;                                   /* 1: flag buffers are int32[RAE_FLAG_WORDS]; the ranks' costs are  */
-} rae_dist_step;                                           /*    summed in rank order (cost_dev, rae_dist_read_cost)           */
+                                                           /*    summed in rank order (cost_dev, rae_dist_read_cost)           */
+    int64_t w_rows;                                        /* rows of this rank's W shard, len(range(rank, F, world)); read    */
+} rae_dist_step;                                           /*    only by a regularised handle (l1 or l2 != 0)                  */
 /* With flag_bufs set, rae_dist_step_end runs: barrier ("every rank has emitted") -> dense update, summing the ranks'
  * dense gradients straight from dense_bufs in rank order when given -> the three pulls -> barrier ("every owner has
  * applied").  The barrier is a one-warp kernel: release-store of the epoch into every peer's flag word, acquire-spin on the
- * own flags (bounded: a rank that never arrives sets the status word instead of hanging the GPU, see rae_peer_status). */
+ * own flags (bounded: a rank that never arrives sets the status word instead of hanging the GPU, see rae_peer_status).
+ * Regularised handle (l1 or l2 != 0, OieModel.py:54-62): before the first barrier the local cost gets adj*(l1*L1 + l2*L2)
+ * of the pre-update W shard (w_rows rows at W) and, on rank 0 with ext_reg, of C | C1 | C2; the dense update adds the
+ * decoder tensors' regulariser term to the summed gradient; and W is applied by rae_shard_apply over the whole shard
+ * instead of pulled row by row. */
 /* Gradient push (optional, once after rae_create with RAE_FLAG_EMIT_ONLY): gw / ga / gab are HOST arrays of `world` device
  * pointers to every rank's RECEIVE buffers, float [world][f_cap][K], [world][n_cap][d], [world][n_cap].  From then on the
  * step's row-update kernels store the reduced gradient row of compact slot j (global row id = f_ids[j] / e_ids[j] of the

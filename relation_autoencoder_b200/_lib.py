@@ -13,7 +13,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("RAE_LIB") or os.path.join(HERE, "librae.so")    # RAE_LIB: A/B measurement of two builds
 HEADER_PATH = os.path.join(os.path.dirname(HERE), "include", "rae.h")
 
-RAE_ABI_VERSION = 2
+RAE_ABI_VERSION = 3
 RAE_MODEL_A, RAE_MODEL_C, RAE_MODEL_AC = 0, 1, 2
 RAE_OPT_ADAGRAD, RAE_OPT_SGD = 0, 1
 RAE_P_W, RAE_P_WB, RAE_P_A, RAE_P_AB, RAE_P_C, RAE_P_C1, RAE_P_C2 = range(7)
@@ -50,7 +50,7 @@ class RaeDistStep(C.Structure):
                 + [("fr_rows", C.c_void_p), ("fr_off", C.c_void_p), ("n_fr", C.c_int64), ("f_src", C.c_void_p), ("f_slot", C.c_void_p)]
                 + [("er_rows", C.c_void_p), ("er_off", C.c_void_p), ("n_er", C.c_int64), ("e_src", C.c_void_p), ("e_slot", C.c_void_p)]
                 + [("cost_dev", C.c_void_p), ("flag_bufs", C.c_void_p), ("dense_bufs", C.c_void_p), ("rank", C.c_int32),
-                   ("global_cost", C.c_int32)])
+                   ("global_cost", C.c_int32), ("w_rows", C.c_int64)])
 
 
 class RaeStepStats(C.Structure):
@@ -90,6 +90,7 @@ _SIGNATURES = {
     "rae_peer_close": (C.c_int, [_P]),
     "rae_fetch_rows": (C.c_int, [_P, _P, C.c_int32, C.c_int64, _P, C.c_int64, _P, _P]),
     "rae_pull_apply": (C.c_int, [_P, _P, _P, C.c_int64, _P, _P, _P, _P, C.c_int64, _P, C.c_int32, _P]),
+    "rae_shard_apply": (C.c_int, [_P, _P, _P, C.c_int64, _P, _P, _P, _P, C.c_int64, _P, C.c_int32, C.c_int64, _P]),
     "rae_train_step_begin": (C.c_int, [_P, C.c_int64, _P, _P, _P, _P, C.c_int64, _P]),
     "rae_dist_step_begin": (C.c_int, [_P, C.POINTER(RaeDistStep), _P]),
     "rae_dist_step_end": (C.c_int, [_P, C.POINTER(RaeDistStep), _P]),

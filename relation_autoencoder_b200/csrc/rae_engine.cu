@@ -224,7 +224,8 @@ static int run_step(rae_engine* h, const int32_t* indptr, const int32_t* indices
     // applied by the same kernel that sums the partials
     if ((rc = launch_dense_finalize(h, st, finish_dense && h->cfg.l1 == 0.0 && h->cfg.l2 == 0.0))) return rc;
     RAE_MARK("dense_finalize", st, 0);
-    RAE_PHASE();   // 13 cost (uses the pre-update parameters for the regulariser value); overlapped order: see phase 5
+    RAE_PHASE();   // 13 cost (uses the pre-update parameters for the regulariser value); overlapped order: see phase 5.
+    // Emit-only: the score part only - rae_dist_step_end adds the regulariser of the own shard and re-runs the cost
     if (!overlap && (rc = launch_cost(h, st))) return rc;
     // emit-only (row-sharded multi-GPU): the tables are per-step compact copies whose every row is touched, so the
     // emitted gradient buffers need no clearing and nothing is applied here (the owner shard applies, rae_pull_apply)
@@ -402,13 +403,12 @@ int rae_create(const rae_config* cfg, rae_engine** out) {
     h->hasSP = cfg->model != RAE_MODEL_A;
     h->quirk = cfg->model == RAE_MODEL_C && !(cfg->flags & RAE_FLAG_FIX_SP_QUIRK);
     h->adagrad = cfg->optimizer == RAE_OPT_ADAGRAD;
-    h->dense_w = (cfg->l1 != 0.0 || cfg->l2 != 0.0);
+    h->reg = (cfg->l1 != 0.0 || cfg->l2 != 0.0);
     h->debug_dense = (cfg->flags & RAE_FLAG_DENSE_GRADS) != 0;
     h->emit_only = (cfg->flags & RAE_FLAG_EMIT_ONLY) != 0;
-    if (h->emit_only && h->dense_w) {
-        delete h;
-        return fail(nullptr, RAE_EINVAL, "RAE_FLAG_EMIT_ONLY (row-sharded tables) does not support l1/l2 != 0 yet");
-    }
+    // row-sharded (emit-only): the step emits W's data gradient only; the owner of each shard adds the regulariser to every
+    // row of it after the cross-rank sum (rae_shard_apply)
+    h->dense_w = h->reg && !h->emit_only;
     h->Z = cfg->z_total > 0 ? (double)cfg->z_total : (double)(4.0 * cfg->B + 2.0 * cfg->B * cfg->S);
 #define RAE_CREATE_CUDA(expr)                                                                                  \
     do {                                                                                                       \

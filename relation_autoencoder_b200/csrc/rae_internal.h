@@ -118,7 +118,10 @@ struct rae_engine {
     rae_config cfg;
     int K, d, S, B;
     int dp;          // d rounded up to a multiple of 4 (row stride of ev)
-    bool hasM, hasSP, quirk, adagrad, dense_w, debug_dense, emit_only;
+    bool hasM, hasSP, quirk, adagrad, debug_dense, emit_only;
+    bool reg;        // l1 or l2 != 0: W (and C | C1 | C2 when ext_reg) carry the regulariser
+    bool dense_w;    // this handle applies the rule to every element of its own W through a dense dW (reg && !emit_only);
+                     // an emit-only handle leaves W's regulariser to the owner's shard pass (rae_shard_apply)
     double Z;        // denominator of the mean
     float* P[RAE_NUM_PARAMS];
     float* ACC[RAE_NUM_PARAMS];
@@ -263,13 +266,19 @@ int launch_fetch_rows(rae_engine* h, const void* const* tables, int world, int64
 int launch_pull_apply(rae_engine* h, float* table, float* acc, int64_t width, const int32_t* rows_local, const int32_t* ent_off,
                       const int32_t* ent_src, const int32_t* ent_slot, int64_t n_rows, const void* const* grads, int world,
                       cudaStream_t st);
+int launch_shard_apply(rae_engine* h, float* table, float* acc, int64_t width, const int32_t* rows_local, const int32_t* ent_off,
+                       const int32_t* ent_src, const int32_t* ent_slot, int64_t n_rows, const void* const* grads, int world,
+                       int64_t shard_rows, cudaStream_t st);
 int launch_peer_barrier(rae_engine* h, const void* const* flag_bufs, int world, int rank, cudaStream_t st, int kind = 0);
 int launch_dense_apply_peers(rae_engine* h, const void* const* dense_bufs, int world, cudaStream_t st, int part = 0);
 int launch_dense_finalize(rae_engine* h, cudaStream_t st, bool fuse_apply);  // sum partials -> dense_grad, or (fused) straight into the optimiser rule
 int launch_dense_apply(rae_engine* h, cudaStream_t st);     // AdaGrad/SGD on C,C1,C2,Wb (+ W when dense_w)
 int stage_host_negatives(rae_engine* h, const int32_t* neg1_host, int64_t ld1, const int32_t* neg2_host, int64_t ld2,
                          cudaStream_t sc, int32_t** d1_out, int32_t** d2_out);   // host [S,B] ids -> device staging, records ev_neg
-int launch_cost(rae_engine* h, cudaStream_t st);            // deterministic loss reduce + regulariser
+// deterministic loss reduce + regulariser.  The norms run over the handle's own W (none on an emit-only handle, whose W is
+// a compact copy) or, when w_shard is given, over w_elems elements there; the decoder tensors' share is added when
+// ext_reg and (not emit-only, or with_dec)
+int launch_cost(rae_engine* h, cudaStream_t st, const float* w_shard = nullptr, int64_t w_elems = 0, bool with_dec = false);
 int launch_zero(rae_engine* h, void* p, size_t bytes, cudaStream_t st);
 
 }  // namespace rae

@@ -8,6 +8,8 @@
 //                                                                      NVLink (or locally), one warp per row, 16-byte lanes
 //   k_pull_apply : owner-side: g = sum_{rank order} grad_rank[slot,:]   remote reads of the ranks' reduced gradient rows,
 //                  then ONE optimiser read-modify-write per row        fixed order -> bitwise reproducible
+//   k_shard_apply: owner-side, l1 / l2 != 0: every row of the W shard  the touched rows' sums as above (0 elsewhere),
+//                  + adj*(l1 sgn w + 2 l2 w), then the rule             one pass over the shard, a pure HBM stream
 //
 // No atomics, no collective: the only synchronisation the sparse path needs is "all ranks have emitted" (given by the
 // dense-gradient all-reduce that precedes the pull) and "all owners have applied" (the end-of-step barrier).
@@ -155,6 +157,153 @@ __global__ void __launch_bounds__(256) k_pull_apply(float* __restrict__ table, f
     }
 }
 
+// regulariser term of one element, added to its (cross-rank summed) data gradient: the expression of k_dense_apply
+// (rae_update.cu), OieModel.py:54-62 with adj folded into r1 = adj*l1, r2 = adj*l2
+__device__ __forceinline__ void add_reg(float& g, float w, float r1, float r2) {
+    const float sgn = (w > 0.f) ? 1.f : ((w < 0.f) ? -1.f : 0.f);
+    g += r1 * sgn + 2.f * r2 * w;
+}
+__device__ __forceinline__ void add_reg(float4& g, const float4& w, float r1, float r2) {
+    add_reg(g.x, w.x, r1, r2); add_reg(g.y, w.y, r1, r2); add_reg(g.z, w.z, r1, r2); add_reg(g.w, w.w, r1, r2);
+}
+
+// Owner-side pass of a regularised W: EVERY row of the rank's shard, not only the rows the batch touched - the regulariser
+// makes every element's gradient non-zero.  Per element, in the order of the single-GPU k_dense_apply: the data gradient
+// (the sum over the row's contributions in rank order, as k_pull_apply, or 0 for a row no rank touched), then
+// adj*(l1 sgn w + 2 l2 w), then the optimiser rule: one read-modify-write of w and acc.
+// A CTA owns the contiguous rows [r0, r0 + rpc).  One binary search finds the first touched row of the range in rows_local
+// (ascending); the touched rows of the range are then merged into a shared per-row table of entry ranges, so the element
+// loop below needs no scratch in global memory.  The element loop is a flat stream over the range's rows * width elements
+// (16-byte units when VEC), SU units per thread in flight.
+constexpr int SHARD_MAX_RPC = 1024;
+template <bool VEC>
+__global__ void __launch_bounds__(256) k_shard_apply(float* __restrict__ table, float* __restrict__ acc, int width, int shard_rows,
+                                                     int rpc, const int32_t* __restrict__ rows_local, const int32_t* __restrict__ ent_off,
+                                                     const int32_t* __restrict__ ent_src, const int32_t* __restrict__ ent_slot,
+                                                     int n_rows, PeerPtrs grads, float lr, int adagrad, float r1, float r2,
+                                                     const int32_t* __restrict__ abort) {
+    __shared__ int s_e0[SHARD_MAX_RPC], s_ne[SHARD_MAX_RPC];
+    __shared__ const float* s_gp[RAE_MAX_PEERS];       // indexed by source rank: from shared, not a local copy of the argument
+    pdl_enter();
+    if (*abort != 0) return;      // a peer barrier of this handle timed out: the peers' gradient rows may be stale
+    const int r0 = blockIdx.x * rpc;
+    const int r1_ = min(r0 + rpc, shard_rows);
+    if (r0 >= r1_) return;
+    for (int j = threadIdx.x; j < r1_ - r0; j += blockDim.x) s_ne[j] = 0;
+    if (threadIdx.x == 0) {
+#pragma unroll
+        for (int r = 0; r < RAE_MAX_PEERS; ++r) s_gp[r] = grads.p[r];
+    }
+    // first touched row >= r0 (every thread finds the same index; rows_local is read through L1)
+    int lo = 0, hi = n_rows;
+    while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if (__ldg(rows_local + mid) < r0) lo = mid + 1;
+        else hi = mid;
+    }
+    __syncthreads();
+    for (int t = lo + threadIdx.x; t < n_rows; t += blockDim.x) {
+        const int r = __ldg(rows_local + t);
+        if (r >= r1_) break;                  // ascending: every later entry is past the range too
+        const int e0 = __ldg(ent_off + t);
+        s_e0[r - r0] = e0;
+        s_ne[r - r0] = __ldg(ent_off + t + 1) - e0;
+    }
+    __syncthreads();
+    constexpr int SU = 4;
+    const int upr = VEC ? width >> 2 : width;            // units per row
+    const int n_units = (r1_ - r0) * upr;
+    float* const tb = table + (size_t)r0 * width;
+    float* const ac = adagrad ? acc + (size_t)r0 * width : nullptr;
+    for (int u0 = threadIdx.x; u0 < n_units; u0 += SU * blockDim.x) {
+        int row[SU], col[SU];
+        bool in[SU];
+        if (VEC) {
+            float4 w[SU], a[SU], g[SU];
+#pragma unroll
+            for (int s = 0; s < SU; ++s) {
+                const int u = u0 + s * blockDim.x;
+                in[s] = u < n_units;
+                row[s] = in[s] ? u / upr : 0;
+                col[s] = u - row[s] * upr;
+                g[s] = make_float4(0.f, 0.f, 0.f, 0.f);
+                w[s] = g[s]; a[s] = g[s];
+                if (in[s]) {
+                    w[s] = reinterpret_cast<const float4*>(tb)[u];
+                    if (adagrad) a[s] = reinterpret_cast<const float4*>(ac)[u];
+                }
+            }
+            // the contributions of the touched rows, entry j of every unit in flight together, added in rank order
+            int ne_max = 0;
+#pragma unroll
+            for (int s = 0; s < SU; ++s) ne_max = max(ne_max, in[s] ? s_ne[row[s]] : 0);
+            for (int j = 0; j < ne_max; ++j) {
+                float4 x[SU];
+#pragma unroll
+                for (int s = 0; s < SU; ++s) {
+                    x[s] = make_float4(0.f, 0.f, 0.f, 0.f);
+                    if (in[s] && j < s_ne[row[s]]) {
+                        const int e = s_e0[row[s]] + j;
+                        x[s] = ld_cv4(reinterpret_cast<const float4*>(s_gp[__ldg(ent_src + e)] + (size_t)__ldg(ent_slot + e) * width) + col[s]);
+                    }
+                }
+#pragma unroll
+                for (int s = 0; s < SU; ++s)
+                    if (in[s] && j < s_ne[row[s]]) { g[s].x += x[s].x; g[s].y += x[s].y; g[s].z += x[s].z; g[s].w += x[s].w; }
+            }
+#pragma unroll
+            for (int s = 0; s < SU; ++s) {
+                if (!in[s]) continue;
+                const int u = u0 + s * blockDim.x;
+                add_reg(g[s], w[s], r1, r2);
+                opt_step(w[s], a[s], g[s], lr, adagrad);
+                if (adagrad) reinterpret_cast<float4*>(ac)[u] = a[s];
+                reinterpret_cast<float4*>(tb)[u] = w[s];
+            }
+        } else {
+            float w[SU], a[SU], g[SU];
+#pragma unroll
+            for (int s = 0; s < SU; ++s) {
+                const int u = u0 + s * blockDim.x;
+                in[s] = u < n_units;
+                row[s] = in[s] ? u / upr : 0;
+                col[s] = u - row[s] * upr;
+                g[s] = 0.f; w[s] = 0.f; a[s] = 0.f;
+                if (in[s]) {
+                    w[s] = tb[u];
+                    if (adagrad) a[s] = ac[u];
+                }
+            }
+            int ne_max = 0;
+#pragma unroll
+            for (int s = 0; s < SU; ++s) ne_max = max(ne_max, in[s] ? s_ne[row[s]] : 0);
+            for (int j = 0; j < ne_max; ++j) {
+                float x[SU];
+#pragma unroll
+                for (int s = 0; s < SU; ++s) {
+                    x[s] = 0.f;
+                    if (in[s] && j < s_ne[row[s]]) {
+                        const int e = s_e0[row[s]] + j;
+                        x[s] = ld_cv(s_gp[__ldg(ent_src + e)] + (size_t)__ldg(ent_slot + e) * width + col[s]);
+                    }
+                }
+#pragma unroll
+                for (int s = 0; s < SU; ++s)
+                    if (in[s] && j < s_ne[row[s]]) g[s] += x[s];
+            }
+#pragma unroll
+            for (int s = 0; s < SU; ++s) {
+                if (!in[s]) continue;
+                const int u = u0 + s * blockDim.x;
+                add_reg(g[s], w[s], r1, r2);
+                opt_step(w[s], a[s], g[s], lr, adagrad);
+                if (adagrad) ac[u] = a[s];
+                tb[u] = w[s];
+            }
+        }
+    }
+}
+
 // width == 1: one thread per row
 __global__ void __launch_bounds__(256) k_pull_apply_scalars(float* __restrict__ table, float* __restrict__ acc,
                                                             const int32_t* __restrict__ rows_local,
@@ -250,8 +399,9 @@ __global__ void __launch_bounds__(256) k_check_negatives(const int32_t* __restri
 }
 
 // dense optimiser step with the ranks' flat dense gradients summed on the fly, in rank order (identical on every rank):
-// replaces "all-reduce, then k_dense_apply" when the gradient is small enough to be read from every peer
-struct DenseSeg { float* p; float* acc; size_t begin, end; };      // [begin, end) of the flat gradient
+// replaces "all-reduce, then k_dense_apply" when the gradient is small enough to be read from every peer.  A regularised
+// segment (C | C1 | C2 when ext_reg) adds adj*(l1 sgn w + 2 l2 w) to the sum before the rule, as k_dense_apply does.
+struct DenseSeg { float* p; float* acc; size_t begin, end; float r1, r2; };      // [begin, end) of the flat gradient
 struct DenseSegs { DenseSeg s[4]; int count; };
 
 __global__ void __launch_bounds__(256) k_dense_apply_peers(DenseSegs segs, PeerPtrs grads, int world, size_t i_begin, size_t i_end,
@@ -277,7 +427,9 @@ __global__ void __launch_bounds__(256) k_dense_apply_peers(DenseSegs segs, PeerP
                     const size_t j = i - segs.s[k].begin;
                     float4 w = *reinterpret_cast<const float4*>(segs.s[k].p + j), a = make_float4(0.f, 0.f, 0.f, 0.f);
                     if (adagrad) a = *reinterpret_cast<const float4*>(segs.s[k].acc + j);
-                    opt_step(w, a, g, lr, adagrad);
+                    float4 gk = g;
+                    if (segs.s[k].r1 != 0.f || segs.s[k].r2 != 0.f) add_reg(gk, w, segs.s[k].r1, segs.s[k].r2);
+                    opt_step(w, a, gk, lr, adagrad);
                     if (adagrad) *reinterpret_cast<float4*>(segs.s[k].acc + j) = a;
                     *reinterpret_cast<float4*>(segs.s[k].p + j) = w;
                 }
@@ -298,7 +450,9 @@ __global__ void __launch_bounds__(256) k_dense_apply_peers(DenseSegs segs, PeerP
             if (k < segs.count && i >= segs.s[k].begin && i < segs.s[k].end) {
                 const size_t j = i - segs.s[k].begin;
                 float w = segs.s[k].p[j], a = adagrad ? segs.s[k].acc[j] : 0.f;
-                opt_step(w, a, g, lr, adagrad);
+                float gk = g;
+                if (segs.s[k].r1 != 0.f || segs.s[k].r2 != 0.f) add_reg(gk, w, segs.s[k].r1, segs.s[k].r2);
+                opt_step(w, a, gk, lr, adagrad);
                 if (adagrad) segs.s[k].acc[j] = a;
                 segs.s[k].p[j] = w;
             }
@@ -362,6 +516,35 @@ int launch_pull_apply(rae_engine* h, float* table, float* acc, int64_t width, co
     return RAE_OK;
 }
 
+int launch_shard_apply(rae_engine* h, float* table, float* acc, int64_t width, const int32_t* rows_local, const int32_t* ent_off,
+                       const int32_t* ent_src, const int32_t* ent_slot, int64_t n_rows, const void* const* grads, int world,
+                       int64_t shard_rows, cudaStream_t st) {
+    if (shard_rows <= 0) return RAE_OK;
+    if (shard_rows >= ((int64_t)1 << 31) || shard_rows * width >= ((int64_t)1 << 40))
+        return fail(h, RAE_EINVAL, "rae_shard_apply: shard of %lld rows is too large", (long long)shard_rows);
+    PeerPtrs pp;
+    int rc = fill_peers(h, grads, world, &pp, "rae_shard_apply");
+    if (rc) return rc;
+    const float lr = (float)h->cfg.lr;
+    const int adagrad = h->adagrad ? 1 : 0;
+    const float r1 = (float)(h->cfg.adj * h->cfg.l1), r2 = (float)(h->cfg.adj * h->cfg.l2);     // as launch_dense_apply
+    // about 16K elements per CTA: a few passes of the element loop, a grid of several waves
+    const int rpc = (int)std::max<int64_t>(1, std::min<int64_t>(SHARD_MAX_RPC, 16384 / width));
+    const int blocks = (int)((shard_rows + rpc - 1) / rpc);
+    bool vec = (width & 3) == 0 && (((uintptr_t)table | (uintptr_t)acc) & 15) == 0;
+    for (int r = 0; r < world; ++r)
+        if ((uintptr_t)pp.p[r] & 15) vec = false;
+    if (vec)
+        launch_pdl(k_shard_apply<true>, dim3(blocks), dim3(256), 0, st, table, acc, (int)width, (int)shard_rows, rpc, rows_local, ent_off,
+                   ent_src, ent_slot, (int)n_rows, pp, lr, adagrad, r1, r2, h->peer_err_dev);
+    else
+        launch_pdl(k_shard_apply<false>, dim3(blocks), dim3(256), 0, st, table, acc, (int)width, (int)shard_rows, rpc, rows_local, ent_off,
+                   ent_src, ent_slot, (int)n_rows, pp, lr, adagrad, r1, r2, h->peer_err_dev);
+    h->launches++;
+    RAE_CUDA(h, cudaGetLastError());
+    return RAE_OK;
+}
+
 // a peer barrier of this handle has timed out (seen through the page-locked status word): every later call fails
 int peer_failed(rae_engine* h) {
     if (*(volatile int32_t*)h->peer_err_pinned == 0) return RAE_OK;
@@ -394,20 +577,23 @@ int launch_dense_apply_peers(rae_engine* h, const void* const* dense_bufs, int w
     PeerPtrs pp;
     int rc = fill_peers(h, dense_bufs, world, &pp, "rae_dist_step_end(dense_bufs)");
     if (rc) return rc;
-    if (h->dense_w) return fail(h, RAE_EINVAL, "peer dense update does not support l1 / l2 != 0");
     DenseSegs segs{};
     bool aligned = true;
-    auto add = [&](int pid, int64_t begin, int64_t n) {
+    // the decoder tensors carry the regulariser when ext_reg (OieModel.py:60-62); Wb never does
+    const bool regdec = h->reg && h->cfg.ext_reg;
+    const float r1 = regdec ? (float)(h->cfg.adj * h->cfg.l1) : 0.f, r2 = regdec ? (float)(h->cfg.adj * h->cfg.l2) : 0.f;
+    auto add = [&](int pid, int64_t begin, int64_t n, bool regularised) {
         if (n <= 0) return;
         DenseSeg& sg = segs.s[segs.count++];
         sg.p = h->P[pid]; sg.acc = h->ACC[pid]; sg.begin = (size_t)begin; sg.end = (size_t)(begin + n);
+        sg.r1 = regularised ? r1 : 0.f; sg.r2 = regularised ? r2 : 0.f;
         if ((begin & 3) || (n & 3) || (((uintptr_t)sg.p | (uintptr_t)sg.acc) & 15)) aligned = false;
     };
     const int64_t dd = h->hasM ? (int64_t)h->d * h->d * h->K : 0, dk = h->hasSP ? (int64_t)h->d * h->K : 0;
-    add(RAE_P_C, h->off_gC, dd);
-    add(RAE_P_C1, h->off_gC1, dk);
-    add(RAE_P_C2, h->off_gC2, dk);
-    add(RAE_P_WB, h->off_gWb, h->K);
+    add(RAE_P_C, h->off_gC, dd, true);
+    add(RAE_P_C1, h->off_gC1, dk, true);
+    add(RAE_P_C2, h->off_gC2, dk, true);
+    add(RAE_P_WB, h->off_gWb, h->K, false);
     for (int r = 0; r < world; ++r)
         if ((uintptr_t)pp.p[r] & 15) aligned = false;
     const size_t i_begin = part == 2 ? (size_t)h->off_gWb : 0, i_end = part == 1 ? (size_t)h->off_gWb : (size_t)h->n_dense;
@@ -489,6 +675,17 @@ int rae_pull_apply(rae_engine* h, float* table, float* acc, int64_t width, const
     if (h->adagrad && !acc) return fail(h, RAE_EINVAL, "rae_pull_apply: AdaGrad needs the accumulator table");
     if (n_rows > 0 && (!rows_local || !ent_off || !ent_src || !ent_slot)) return fail(h, RAE_EINVAL, "rae_pull_apply: null plan arrays");
     return launch_pull_apply(h, table, acc, width, rows_local, ent_off, ent_src, ent_slot, n_rows, grads, world, (cudaStream_t)stream);
+}
+
+int rae_shard_apply(rae_engine* h, float* table, float* acc, int64_t width, const int32_t* rows_local, const int32_t* ent_off,
+                    const int32_t* ent_src, const int32_t* ent_slot, int64_t n_rows, const void* const* grads, int32_t world,
+                    int64_t shard_rows, void* stream) {
+    if (!h || !grads || width < 1 || n_rows < 0 || shard_rows < 0 || (shard_rows > 0 && !table))
+        return fail(h, RAE_EINVAL, "rae_shard_apply: bad argument");
+    if (h->adagrad && shard_rows > 0 && !acc) return fail(h, RAE_EINVAL, "rae_shard_apply: AdaGrad needs the accumulator table");
+    if (n_rows > 0 && (!rows_local || !ent_off || !ent_src || !ent_slot)) return fail(h, RAE_EINVAL, "rae_shard_apply: null plan arrays");
+    return launch_shard_apply(h, table, acc, width, rows_local, ent_off, ent_src, ent_slot, n_rows, grads, world, shard_rows,
+                              (cudaStream_t)stream);
 }
 
 int rae_peer_barrier(rae_engine* h, const void* const* flag_bufs, int32_t world, int32_t rank, void* stream) {
@@ -619,6 +816,14 @@ int rae_dist_step_end(rae_engine* h, const rae_dist_step* d, void* stream) {
     const bool flags = d->flag_bufs != nullptr;
     const bool gcost = flags && d->global_cost != 0;
     FlagPtrs fp;
+    if (h->reg) {
+        // The regulariser's share of this rank, from the parameters before this step's update (every apply of the step is
+        // behind barrier A below): its own W shard, and on rank 0 the decoder tensors, which every rank holds.  The cost is
+        // re-run on the score partials of the local step; the rank-order sum of the local costs is then the global cost.
+        if (d->w_rows < 0 || (d->w_rows > 0 && !d->W)) return fail(h, RAE_EINVAL, "rae_dist_step_end: bad W shard / w_rows");
+        if ((rc = launch_cost(h, st, d->W, d->w_rows * h->K, d->rank == 0))) return rc;
+        RAE_DMARK("reg_cost", st, 0);
+    }
     if (gcost) {
         if (d->world > RAE_MAX_PEERS || d->rank < 0 || d->rank >= d->world) return fail(h, RAE_EINVAL, "rae_dist_step_end: bad world / rank");
         memset(&fp, 0, sizeof(fp));
@@ -666,8 +871,15 @@ int rae_dist_step_end(rae_engine* h, const rae_dist_step* d, void* stream) {
         if ((rc = rae_pull_apply(h, d->Ab, d->accAb, 1, d->er_rows, d->er_off, d->e_src, d->e_slot, d->n_er, d->gab_bufs, d->world, sb))) return rc;
         RAE_DMARK("apply_Ab", sb, side ? 2 : 0);
     }
-    if (d->n_fr > 0 && (rc = rae_pull_apply(h, d->W, d->accW, h->K, d->fr_rows, d->fr_off, d->f_src, d->f_slot, d->n_fr, d->gw_bufs,
-                                            d->world, stream))) return rc;
+    if (h->reg) {
+        // every row of the shard moves: the touched rows' contributions, then the regulariser, then the rule
+        RAE_DMARK("w_shard_begin", st, 0);
+        if ((rc = rae_shard_apply(h, d->W, d->accW, h->K, d->fr_rows, d->fr_off, d->f_src, d->f_slot, d->n_fr, d->gw_bufs, d->world,
+                                  d->w_rows, stream))) return rc;
+    } else if (d->n_fr > 0 && (rc = rae_pull_apply(h, d->W, d->accW, h->K, d->fr_rows, d->fr_off, d->f_src, d->f_slot, d->n_fr,
+                                                   d->gw_bufs, d->world, stream))) {
+        return rc;
+    }
     RAE_DMARK("apply_W", st, 0);
     if (!peer_dense) {
         // the caller all-reduced the dense gradient itself - possibly on another stream, beside the barrier and the applies

@@ -700,7 +700,23 @@ __global__ void __launch_bounds__(256) k_dense_apply(DenseJobs jobs) {
 __global__ void k_reg_norms(const float* __restrict__ p, size_t n, double* __restrict__ part /* [grid][2] */) {
     __shared__ double s1[256], s2[256];
     double a = 0.0, b = 0.0;
-    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
+    // each thread visits i, i + stride, ... in that order; the loads of NU consecutive visits are issued before their adds
+    // (one memory latency per NU elements instead of per element), the summation order is unchanged
+    constexpr int NU = 16;
+    const size_t stride = (size_t)gridDim.x * blockDim.x;
+    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    for (; i + (NU - 1) * stride < n; i += NU * stride) {
+        float x[NU];
+#pragma unroll
+        for (int u = 0; u < NU; ++u) x[u] = p[i + u * stride];
+#pragma unroll
+        for (int u = 0; u < NU; ++u) {
+            const double v = (double)x[u];
+            a += fabs(v);
+            b += v * v;
+        }
+    }
+    for (; i < n; i += stride) {
         const double v = (double)p[i];
         a += fabs(v);
         b += v * v;
@@ -933,7 +949,7 @@ int launch_dense_finalize(rae_engine* h, cudaStream_t st, bool fuse_apply) {
 }
 
 int launch_dense_apply(rae_engine* h, cudaStream_t st) {
-    const bool reg = (h->cfg.l1 != 0.0 || h->cfg.l2 != 0.0);
+    const bool reg = h->reg;
     if (h->dense_fused && !h->dense_w) return RAE_OK;      // applied inside k_dense_finalize
     const bool regdec = reg && h->cfg.ext_reg;
     const size_t dd = (size_t)h->d * h->d * h->K, dk = (size_t)h->d * h->K;
@@ -968,27 +984,28 @@ int launch_dense_apply(rae_engine* h, cudaStream_t st) {
     return RAE_OK;
 }
 
-int launch_cost(rae_engine* h, cudaStream_t st) {
-    const bool reg = (h->cfg.l1 != 0.0 || h->cfg.l2 != 0.0);
+int launch_cost(rae_engine* h, cudaStream_t st, const float* w_shard, int64_t w_elems, bool with_dec) {
     int n_reg = 0;
-    if (reg) {
+    if (h->reg) {
         // fixed grid per tensor -> fixed summation order
-        auto norms = [&](int pid, size_t n) -> int {
+        auto norms = [&](const float* p, size_t n) -> int {
             if (n == 0) return RAE_OK;
             const int blocks = 64;
             if (n_reg + blocks > h->n_reg_part) return fail(h, RAE_EINVAL, "internal: reg_part too small");
-            k_reg_norms<<<blocks, 256, 0, st>>>(h->P[pid], n, h->reg_part + 2 * (size_t)n_reg);
+            k_reg_norms<<<blocks, 256, 0, st>>>(p, n, h->reg_part + 2 * (size_t)n_reg);
             n_reg += blocks;
             h->launches++;
             return RAE_OK;
         };
         int rc;
-        if ((rc = norms(RAE_P_W, (size_t)h->cfg.F * h->K))) return rc;
-        if (h->cfg.ext_reg) {
-            if (h->hasM && (rc = norms(RAE_P_C, (size_t)h->d * h->d * h->K))) return rc;
+        // an emit-only handle's W is the step's compact copy, not the parameter: its norms come from the shard
+        if (!h->emit_only && (rc = norms(h->P[RAE_P_W], (size_t)h->cfg.F * h->K))) return rc;
+        if (w_shard && (rc = norms(w_shard, (size_t)w_elems))) return rc;
+        if (h->cfg.ext_reg && (!h->emit_only || with_dec)) {
+            if (h->hasM && (rc = norms(h->P[RAE_P_C], (size_t)h->d * h->d * h->K))) return rc;
             if (h->hasSP) {
-                if ((rc = norms(RAE_P_C1, (size_t)h->d * h->K))) return rc;
-                if ((rc = norms(RAE_P_C2, (size_t)h->d * h->K))) return rc;
+                if ((rc = norms(h->P[RAE_P_C1], (size_t)h->d * h->K))) return rc;
+                if ((rc = norms(h->P[RAE_P_C2], (size_t)h->d * h->K))) return rc;
             }
         }
     }

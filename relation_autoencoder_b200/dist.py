@@ -17,6 +17,13 @@ a sum over examples divided by the global Z (learning/OieModel.py:90).
     (4) pull    - each OWNER reads the gradient rows of its rows from all ranks' compact gradient buffers, sums them in
                   rank order and applies ONE optimiser read-modify-write per row (``rae_pull_apply``);
     (5) barrier - "every owner has applied", before the next step's fetch.
+* regulariser (l1 / l2 != 0, OieModel.py:54-62, OieInduction.py:131-135): it reaches every element of W (and of C | C1 | C2
+  when ext_reg), touched or not.  The local step emits data gradients only.  Before (3) each rank adds
+  adj*(l1*L1 + l2*L2) of its own pre-update W shard to its local cost, rank 0 also that of the decoder tensors, so the
+  rank-order sum of the local costs is the global batch's cost.  The dense update adds the decoder tensors' term to the
+  summed gradient.  In (4) the owner applies W over its WHOLE shard (``rae_shard_apply``): per element the summed
+  contributions (0 for a row no rank touched), then adj*(l1*sgn + 2*l2*w), then the rule - the order of the single-GPU
+  dense update.
   Fixed orders everywhere: bitwise reproducible for a given world size.  (Backends without peer memory - the NumPy
   backend of the CPU tests - order (3) and (5) with the dense all-reduce and a one-element cost all-reduce.)
 * routing (which rows, which slots, who owns what) depends only on the ids: the plans of ALL batches are built at bind
@@ -203,11 +210,17 @@ class GranularStep:
         self.local_step(b, a1c, a2c, n1c, n2c, neg_ld)
 
     def run_end(self, de, b):
+        # a regularised step (backends implement add_local_regulariser / shard_apply): the regulariser's value is taken
+        # from the parameters before any apply of this step, and W moves over the whole shard, touched rows or not
+        reg = de.l1 != 0.0 or de.l2 != 0.0
+        if reg:
+            self.add_local_regulariser()
         self.dense_apply()
         for name, plan in (("W", de.fplan), ("A", de.eplan), ("Ab", de.eplan)):
             lo, hi = plan.r_off[b], plan.r_off[b + 1]
-            self.pull_apply(name, de.shard[name], de.shard_acc[name], plan.rows_local[lo:hi], plan.ent_off[lo:hi + 1],
-                            plan.ent_src, plan.ent_slot)
+            apply = self.shard_apply if (reg and name == "W") else self.pull_apply
+            apply(name, de.shard[name], de.shard_acc[name], plan.rows_local[lo:hi], plan.ent_off[lo:hi + 1], plan.ent_src,
+                  plan.ent_slot)
         return self.local_cost_tensor()
 
     def plans_changed(self, de):
@@ -266,7 +279,7 @@ class CudaBackend(GranularStep):
         L = self.L
         self.eng = Engine(de.model, de.K, de.d, de.S, de.B, f_cap, n_cap, de.n_train, lr=de.lr, alpha=de.alpha,
                           optimizer=de.optimizer, device=self.device.index, flags=L.RAE_FLAG_EMIT_ONLY, z_total=de.z_total,
-                          adj=de.adj)
+                          adj=de.adj, l1=de.l1, l2=de.l2, ext_reg=de.ext_reg)
         self.h = self.eng._h
         f32 = dict(dtype=torch.float32, device=self.device)
         self.compact = {"W": torch.zeros(f_cap, de.K, **f32), "A": torch.zeros(n_cap, de.d, **f32), "Ab": torch.zeros(n_cap, **f32)}
@@ -327,6 +340,8 @@ class CudaBackend(GranularStep):
         self.eng._check(self.lib.rae_train_step_end(self.h, self._stream), "rae_train_step_end")
 
     def pull_apply(self, name: str, table, acc, rows_local, ent_off, ent_src, ent_slot):
+        if name == "W" and (self.de.l1 != 0.0 or self.de.l2 != 0.0):
+            return self.shard_apply(name, table, acc, rows_local, ent_off, ent_src, ent_slot)   # every row moves
         width = 1 if table.dim() == 1 else table.shape[1]
         n_rows = rows_local.numel()
         if n_rows == 0:
@@ -334,6 +349,13 @@ class CudaBackend(GranularStep):
         self.eng._check(self.lib.rae_pull_apply(self.h, self._p(table), self._p(acc), width, self._p(rows_local), self._p(ent_off),
                                                 self._p(ent_src), self._p(ent_slot), n_rows, self._recv_regions[name],
                                                 self.de.world, self._stream), "rae_pull_apply")
+
+    def shard_apply(self, name: str, table, acc, rows_local, ent_off, ent_src, ent_slot):
+        """The regularised owner-side pass over every row of the shard ``table`` (``rae_shard_apply``)."""
+        width = 1 if table.dim() == 1 else table.shape[1]
+        self.eng._check(self.lib.rae_shard_apply(self.h, self._p(table), self._p(acc), width, self._p(rows_local), self._p(ent_off),
+                                                 self._p(ent_src), self._p(ent_slot), rows_local.numel(), self._recv_regions[name],
+                                                 self.de.world, table.shape[0], self._stream), "rae_shard_apply")
 
     def local_cost_tensor(self) -> torch.Tensor:
         self.eng._check(self.lib.rae_copy_cost(self.h, self._p(self.cost_t), self._stream), "rae_copy_cost")
@@ -374,6 +396,7 @@ class CudaBackend(GranularStep):
             d.dense_bufs = vp(self._grad_arrays["dense"]) if self.peer_dense else None
             d.rank = de.rank
             d.global_cost = 1                     # the ranks' costs are summed over peer memory too: no collective in the step
+            d.w_rows = de.shard["W"].shape[0]     # the handle's F is the compact capacity: the shard's rows come from here
             self.descs.append(d)
 
     def run_begin(self, de, b, a1c, a2c, n1c, n2c, neg_ld):
@@ -443,8 +466,6 @@ class DistributedEngine:
                  device=0, rank: Optional[int] = None, world: Optional[int] = None, backend_factory=None, group=None,
                  peer_dense_max_bytes: int = 16 << 20):
         self.peer_dense_max_bytes = int(peer_dense_max_bytes)
-        if l1 != 0.0 or l2 != 0.0:
-            raise NotImplementedError("row-sharded multi-GPU training supports l1 = l2 = 0 only (the regulariser makes dW dense)")
         from .engine import MODEL_IDS, MODEL_PARAMS
         self.rank = dist.get_rank(group) if rank is None else rank
         self.world = dist.get_world_size(group) if world is None else world
@@ -454,6 +475,7 @@ class DistributedEngine:
         self.model, self.K, self.d, self.S, self.B, self.F, self.N = model, K, d, S, B, F, N
         self.n_train = n_train
         self.lr, self.alpha, self.optimizer = lr, alpha, optimizer
+        self.l1, self.l2, self.ext_reg = float(l1), float(l2), bool(ext_reg)
         self.names = list(MODEL_PARAMS[MODEL_IDS[model]])
         self.dense_names = [n for n in self.names if n not in SPARSE]
         self.z_total = self.world * (4 * B + 2 * B * S)                       # global Z (OieModel.py:90)
