@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define RAE_ABI_VERSION 3
+#define RAE_ABI_VERSION 4
 
 /* decoder selection: construct_decoder(model_type, ...) learning/models/decoders/Decoder.py:84-93 */
 #define RAE_MODEL_A 0  /* 'rescal'    Bilinear.py               */
@@ -152,7 +152,7 @@ int rae_train_step_explicit(rae_engine* h, const int32_t* indptr, const int32_t*
  * The row-sharded step of the peer-memory path below (relation_autoencoder_b200/dist.py) binds a rank's compact gradient
  * buffers and flat dense gradient with rae_bind_grad_buffers and runs its local step as rae_train_step_begin, then
  * rae_train_step_end around the dense-gradient all-reduce.  It copies the local cost for the cross-rank sum with
- * rae_copy_cost and labels a split's rows on their compact feature slots with rae_label_explicit. */
+ * rae_copy_cost and labels a split's rows straight from the owners' W shards with rae_label_shards. */
 /* caller-owned output buffers for the emitted gradients: gW[F,K], gA[N,d], gAb[N] (F, N = compact capacities) and the
  * flat dense gradient [C | C1 | C2 | Wb] (rae_dense_grad_size floats).  NULL keeps the internal buffer. */
 int rae_bind_grad_buffers(rae_engine* h, float* gW, float* gA, float* gAb, float* dense);
@@ -268,9 +268,18 @@ int rae_peer_barrier(rae_engine* h, const void* const* flag_bufs, int32_t world,
 int rae_peer_status(rae_engine* h, void* stream);
 /* copy the last step's (local) cost into a DEVICE double (no synchronisation) */
 int rae_copy_cost(rae_engine* h, double* dst_device, void* stream);
-/* encoder on explicit device inputs (indptr has n_rows+1 entries; n_rows <= B): labels int64[n_rows], probs [n_rows, K] */
-int rae_label_explicit(rae_engine* h, const int32_t* indptr, const int32_t* indices, int64_t n_rows, int64_t* labels,
-                       float* probs, void* stream);
+/* func['label_<split>'] over n_rows rows of a split whose W is row-sharded over `world` ranks: row f of W is
+ * w_shards[f % world] + (f / world) * K (w_shards: HOST array of `world` device pointers, own shard included; world = 1
+ * with the handle's bound W is the single-table case).  indices are GLOBAL feature ids; indptr has n_rows+1 entries and
+ * may start at any offset; n_rows is NOT bounded by B.  Wb is the handle's bound Wb.  labels int64[n_rows] (first max
+ * wins); probs [n_rows, K] or NULL (not written).  The sums run in CSR order, as in rae_label: labels and probs are
+ * bit-identical to those of a single-GPU handle holding the gathered W.
+ * Ordering: the kernel runs on `stream`, the caller's stream of the sharded step.  There rae_dist_step_end ends with the
+ * "every owner has applied" barrier, so the labels see the last step's W on every rank.  The next step cannot overtake
+ * the read either: its W applies sit behind its barrier A ("every rank has emitted"), which every rank issues on its
+ * caller stream behind this kernel. */
+int rae_label_shards(rae_engine* h, const void* const* w_shards, int32_t world, const int32_t* indptr,
+                     const int32_t* indices, int64_t n_rows, int64_t* labels, float* probs, void* stream);
 
 /* ---- negative sampling on the device (replaces NegativeExampleGenerator.get_negative_samples, NegativeExampleGenerator.py:14-32)
  * out[i] = searchsorted(cum, uniform(0, cum_last)) for i in [0, n), bit-exact with the reference's host recipe on a legacy

@@ -13,7 +13,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("RAE_LIB") or os.path.join(HERE, "librae.so")    # RAE_LIB: A/B measurement of two builds
 HEADER_PATH = os.path.join(os.path.dirname(HERE), "include", "rae.h")
 
-RAE_ABI_VERSION = 3
+RAE_ABI_VERSION = 4
 RAE_MODEL_A, RAE_MODEL_C, RAE_MODEL_AC = 0, 1, 2
 RAE_OPT_ADAGRAD, RAE_OPT_SGD = 0, 1
 RAE_P_W, RAE_P_WB, RAE_P_A, RAE_P_AB, RAE_P_C, RAE_P_C1, RAE_P_C2 = range(7)
@@ -101,7 +101,7 @@ _SIGNATURES = {
     "rae_peer_barrier": (C.c_int, [_P, _P, C.c_int32, C.c_int32, _P]),
     "rae_peer_status": (C.c_int, [_P, _P]),
     "rae_copy_cost": (C.c_int, [_P, _P, _P]),
-    "rae_label_explicit": (C.c_int, [_P, _P, _P, C.c_int64, _P, _P, _P]),
+    "rae_label_shards": (C.c_int, [_P, _P, C.c_int32, _P, _P, C.c_int64, _P, _P, _P]),
     "rae_sample_negatives": (C.c_int, [_P, _P, _P, C.c_int64, C.c_double, _P, C.c_int64, _P, _P]),
     "rae_set_profiling": (C.c_int, [_P, C.c_int32]),
     "rae_get_phase_times": (C.c_int, [_P, C.POINTER(C.c_float)]),

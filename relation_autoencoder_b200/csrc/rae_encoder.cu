@@ -8,15 +8,69 @@
 
 namespace rae {
 
-template <int KT>
+// Where row f of W is: a compile-time policy of the encoder bodies below.  The warp of an example reads its feature ids 32
+// at a time (one per lane), turns each into a lookup key, and broadcasts the key of the row it loads next.
+//   DenseTable : one table, row f at W + f*K (the engine's bound W: the single-GPU step and labelling, the compact tables of
+//                the sharded step).  int example index; probs are always written.
+//   ShardTables: W row-sharded over `world` ranks, row f at p[f % world] + (f / world)*K (rae_label_shards).  The <= 16
+//                peer pointers are copied into shared memory at kernel entry, so the lookup never indexes the parameter
+//                space dynamically (no local copy, no stack frame); the key is the row pointer itself.  int64 example
+//                index (a whole split per launch); q == NULL skips the probability stores.
+struct DenseTable {
+    typedef const float* __restrict__ Arg;
+    typedef int Index;
+    typedef int Key;
+    static constexpr bool kOptionalQ = false;
+    const float* W;
+    __device__ __forceinline__ explicit DenseTable(const float* w) : W(w) {}
+    static __device__ __forceinline__ Index example() { return (blockIdx.x * blockDim.x + threadIdx.x) >> 5; }
+    __device__ __forceinline__ Key key(int f, int) const { return f; }
+    static __device__ __forceinline__ Key shfl(Key k, int src) { return __shfl_sync(kFull, k, src); }
+    __device__ __forceinline__ const float* row(Key f, int K) const { return W + (size_t)f * K; }
+};
+
+struct ShardPtrs {
+    const float* p[RAE_MAX_PEERS];
+    int world;
+};
+
+struct ShardTables {
+    typedef ShardPtrs Arg;
+    typedef int64_t Index;
+    typedef const float* Key;
+    static constexpr bool kOptionalQ = true;
+    const float* const* tab;       // shared memory
+    int world;
+    // every thread of the CTA must construct it (one barrier) before any thread leaves
+    __device__ __forceinline__ explicit ShardTables(const ShardPtrs& a) : world(a.world) {
+        __shared__ const float* s_tab[RAE_MAX_PEERS];
+        if (threadIdx.x == 0) {
+#pragma unroll
+            for (int r = 0; r < RAE_MAX_PEERS; ++r) s_tab[r] = a.p[r];
+        }
+        __syncthreads();
+        tab = s_tab;
+    }
+    static __device__ __forceinline__ Index example() {
+        return (Index)(((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5);
+    }
+    __device__ __forceinline__ Key key(int f, int K) const { return tab[f % world] + (size_t)(f / world) * K; }
+    static __device__ __forceinline__ Key shfl(Key k, int src) {
+        return reinterpret_cast<Key>(__shfl_sync(kFull, reinterpret_cast<unsigned long long>(k), src));
+    }
+    __device__ __forceinline__ const float* row(Key k, int) const { return k; }
+};
+
+template <int KT, class Rows = DenseTable>
 __global__ void __launch_bounds__(256) k_encoder_forward(const int32_t* __restrict__ indptr,
                                                          const int32_t* __restrict__ indices,
-                                                         const float* __restrict__ W, const float* __restrict__ Wb,
-                                                         int B, int K, float alpha, float* __restrict__ q,
+                                                         typename Rows::Arg W, const float* __restrict__ Wb,
+                                                         typename Rows::Index B, int K, float alpha, float* __restrict__ q,
                                                          float* __restrict__ logq, float* __restrict__ sc_ent,
                                                          int sc_stride, int64_t* __restrict__ labels) {
+    const Rows rows(W);
     const int lane = threadIdx.x & 31;
-    const int b = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const typename Rows::Index b = Rows::example();
     if (b >= B) return;
     const int beg = indptr[b], end = indptr[b + 1];
     float z[KT];
@@ -27,15 +81,15 @@ __global__ void __launch_bounds__(256) k_encoder_forward(const int32_t* __restri
     }
     constexpr int UNROLL = (KT <= 4) ? 8 : 2;
     for (int base = beg; base < end; base += 32) {
-        const int mine = (base + lane < end) ? indices[base + lane] : 0;
+        const typename Rows::Key mine = rows.key((base + lane < end) ? indices[base + lane] : 0, K);
         const int cnt = min(32, end - base);
         for (int t0 = 0; t0 < cnt; t0 += UNROLL) {
             float v[UNROLL][KT];
 #pragma unroll
             for (int u = 0; u < UNROLL; ++u) {
-                const int f = __shfl_sync(kFull, mine, (t0 + u) & 31);
+                const typename Rows::Key f = Rows::shfl(mine, (t0 + u) & 31);
                 const bool ok = (t0 + u) < cnt;
-                const float* row = W + (size_t)f * K;
+                const float* row = rows.row(f, K);
 #pragma unroll
                 for (int t = 0; t < KT; ++t) {
                     int k = lane + 32 * t;
@@ -78,13 +132,14 @@ __global__ void __launch_bounds__(256) k_encoder_forward(const int32_t* __restri
     s = warp_sum(s);
     const float lse = m + logf(s);
     float ent = 0.f;
+    const bool store_q = !Rows::kOptionalQ || q != nullptr;
 #pragma unroll
     for (int t = 0; t < KT; ++t) {
         int k = lane + 32 * t;
         if (k < K) {
             float lq = z[t] - lse;
             float p = expf(lq);
-            q[(size_t)b * K + k] = p;
+            if (store_q) q[(size_t)b * K + k] = p;
             if (logq != nullptr) logq[(size_t)b * K + k] = lq;
             ent -= p * lq;
         }
@@ -97,16 +152,17 @@ __global__ void __launch_bounds__(256) k_encoder_forward(const int32_t* __restri
 
 // K % 4 == 0: every lane owns QT float4 (16-byte row loads, one instruction per W row for K <= 128) and UNROLL rows
 // are in flight together.
-template <int QT>
+template <int QT, class Rows = DenseTable>
 __global__ void __launch_bounds__(256) k_encoder_forward_v4(const int32_t* __restrict__ indptr,
                                                             const int32_t* __restrict__ indices,
-                                                            const float* __restrict__ W, const float* __restrict__ Wb,
-                                                            int B, int K, float alpha, float* __restrict__ q,
+                                                            typename Rows::Arg W, const float* __restrict__ Wb,
+                                                            typename Rows::Index B, int K, float alpha, float* __restrict__ q,
                                                             float* __restrict__ logq, float* __restrict__ sc_ent,
                                                             int sc_stride, int64_t* __restrict__ labels) {
     pdl_enter();
+    const Rows rows(W);
     const int lane = threadIdx.x & 31;
-    const int b = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const typename Rows::Index b = Rows::example();
     if (b >= B) return;
     const int beg = indptr[b], end = indptr[b + 1];
     const int nq = K >> 2;
@@ -118,15 +174,15 @@ __global__ void __launch_bounds__(256) k_encoder_forward_v4(const int32_t* __res
     }
     constexpr int UNROLL = (QT == 1) ? 16 : (QT == 2 ? 8 : 4);
     for (int base = beg; base < end; base += 32) {
-        const int mine = (base + lane < end) ? indices[base + lane] : 0;
+        const typename Rows::Key mine = rows.key((base + lane < end) ? indices[base + lane] : 0, K);
         const int cnt = min(32, end - base);
         for (int t0 = 0; t0 < cnt; t0 += UNROLL) {
             float4 v[UNROLL][QT];
 #pragma unroll
             for (int u = 0; u < UNROLL; ++u) {
-                const int f = __shfl_sync(kFull, mine, (t0 + u) & 31);
+                const typename Rows::Key f = Rows::shfl(mine, (t0 + u) & 31);
                 const bool ok = (t0 + u) < cnt;
-                const float4* row = reinterpret_cast<const float4*>(W + (size_t)f * K);
+                const float4* row = reinterpret_cast<const float4*>(rows.row(f, K));
 #pragma unroll
                 for (int t = 0; t < QT; ++t) {
                     const int qi = lane + 32 * t;
@@ -175,13 +231,14 @@ __global__ void __launch_bounds__(256) k_encoder_forward_v4(const int32_t* __res
     s = warp_sum(s);
     const float lse = m + logf(s);
     float ent = 0.f;
+    const bool store_q = !Rows::kOptionalQ || q != nullptr;
 #pragma unroll
     for (int t = 0; t < QT; ++t) {
         const int qi = lane + 32 * t;
         if (qi < nq) {
             const float4 lq = make_float4(z[t].x - lse, z[t].y - lse, z[t].z - lse, z[t].w - lse);
             const float4 pr = make_float4(expf(lq.x), expf(lq.y), expf(lq.z), expf(lq.w));
-            reinterpret_cast<float4*>(q + (size_t)b * K)[qi] = pr;
+            if (store_q) reinterpret_cast<float4*>(q + (size_t)b * K)[qi] = pr;
             if (logq != nullptr) reinterpret_cast<float4*>(logq + (size_t)b * K)[qi] = lq;
             ent -= (pr.x * lq.x + pr.y * lq.y) + (pr.z * lq.z + pr.w * lq.w);
         }
@@ -192,22 +249,28 @@ __global__ void __launch_bounds__(256) k_encoder_forward_v4(const int32_t* __res
     }
 }
 
-int launch_encoder_forward(rae_engine* h, const int32_t* indptr, const int32_t* indices, int B, float* q, float* logq,
-                           float* sc_ent, int64_t* labels, cudaStream_t st) {
+namespace {
+
+// One launch of the encoder over n examples with the W lookup of policy Rows.  w_aligned: every row of W starts on 16 bytes
+// when K % 4 == 0 (the 16-byte path also needs Wb, q and log q aligned).
+template <class Rows>
+int launch_encoder(rae_engine* h, const int32_t* indptr, const int32_t* indices, typename Rows::Arg W, bool w_aligned,
+                   typename Rows::Index n, float* q, float* logq, float* sc_ent, int64_t* labels, cudaStream_t st) {
     const int K = h->K;
     const int threads = 256;
-    const int blocks = (B * 32 + threads - 1) / threads;
-    const float* W = h->P[RAE_P_W];
+    const int64_t blocks64 = ((int64_t)n * 32 + threads - 1) / threads;
+    if (blocks64 > 0x7fffffff) return fail(h, RAE_EINVAL, "encoder: %lld rows are too many for one launch", (long long)n);
+    const int blocks = (int)blocks64;
     const float* Wb = h->P[RAE_P_WB];
     const float alpha = (float)h->cfg.alpha;
     const int kt = (K + 31) / 32;
     // 16-byte path: rows of W, q and log q must be 16-byte aligned (K % 4 == 0 and aligned base pointers)
-    const bool vec = (K & 3) == 0 && K <= 512 && (((uintptr_t)W | (uintptr_t)Wb | (uintptr_t)q | (uintptr_t)logq) & 15) == 0;
+    const bool vec = (K & 3) == 0 && K <= 512 && w_aligned && (((uintptr_t)Wb | (uintptr_t)q | (uintptr_t)logq) & 15) == 0;
     if (vec) {
         const int qt = (K / 4 + 31) / 32;
 #define RAE_ENC4(QT)                                                                                                 \
-    launch_pdl(k_encoder_forward_v4<QT>, dim3(blocks), dim3(threads), 0, st, indptr, indices, W, Wb, B, K, alpha, q, logq, sc_ent, SC_N, \
-                                                          labels)
+    launch_pdl(k_encoder_forward_v4<QT, Rows>, dim3(blocks), dim3(threads), 0, st, indptr, indices, W, Wb, n, K, alpha, q, logq, sc_ent, SC_N, \
+               labels)
         if (qt <= 1) RAE_ENC4(1);
         else if (qt <= 2) RAE_ENC4(2);
         else RAE_ENC4(4);
@@ -216,9 +279,8 @@ int launch_encoder_forward(rae_engine* h, const int32_t* indptr, const int32_t* 
         RAE_CUDA(h, cudaGetLastError());
         return RAE_OK;
     }
-#define RAE_ENC(KT)                                                                                              \
-    k_encoder_forward<KT><<<blocks, threads, 0, st>>>(indptr, indices, W, Wb, B, K, alpha, q, logq, sc_ent, SC_N, \
-                                                       labels)
+#define RAE_ENC(KT)                                                                                                  \
+    k_encoder_forward<KT, Rows><<<blocks, threads, 0, st>>>(indptr, indices, W, Wb, n, K, alpha, q, logq, sc_ent, SC_N, labels)
     if (kt <= 1) RAE_ENC(1);
     else if (kt <= 2) RAE_ENC(2);
     else if (kt <= 4) RAE_ENC(4);
@@ -230,6 +292,29 @@ int launch_encoder_forward(rae_engine* h, const int32_t* indptr, const int32_t* 
     h->launches++;
     RAE_CUDA(h, cudaGetLastError());
     return RAE_OK;
+}
+
+}  // namespace
+
+int launch_encoder_forward(rae_engine* h, const int32_t* indptr, const int32_t* indices, int B, float* q, float* logq,
+                           float* sc_ent, int64_t* labels, cudaStream_t st) {
+    const float* W = h->P[RAE_P_W];
+    return launch_encoder<DenseTable>(h, indptr, indices, W, ((uintptr_t)W & 15) == 0, B, q, logq, sc_ent, labels, st);
+}
+
+int launch_label_shards(rae_engine* h, const void* const* w_shards, int world, const int32_t* indptr, const int32_t* indices,
+                        int64_t n_rows, int64_t* labels, float* probs, cudaStream_t st) {
+    if (world < 1 || world > RAE_MAX_PEERS) return fail(h, RAE_EINVAL, "rae_label_shards: world %d out of range [1, %d]", world, RAE_MAX_PEERS);
+    ShardPtrs sp = {};
+    sp.world = world;
+    bool aligned = true;
+    for (int r = 0; r < world; ++r) {
+        if (!w_shards[r]) return fail(h, RAE_EINVAL, "rae_label_shards: null W shard for rank %d", r);
+        sp.p[r] = static_cast<const float*>(w_shards[r]);
+        aligned = aligned && ((uintptr_t)sp.p[r] & 15) == 0;
+    }
+    if (n_rows == 0) return RAE_OK;
+    return launch_encoder<ShardTables>(h, indptr, indices, sp, aligned, n_rows, probs, nullptr, nullptr, labels, st);
 }
 
 }  // namespace rae

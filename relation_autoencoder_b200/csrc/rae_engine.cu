@@ -758,14 +758,13 @@ int rae_copy_cost(rae_engine* h, double* dst_device, void* stream) {
     return RAE_OK;
 }
 
-int rae_label_explicit(rae_engine* h, const int32_t* indptr, const int32_t* indices, int64_t n_rows, int64_t* labels,
-                       float* probs, void* stream) {
+int rae_label_shards(rae_engine* h, const void* const* w_shards, int32_t world, const int32_t* indptr,
+                     const int32_t* indices, int64_t n_rows, int64_t* labels, float* probs, void* stream) {
     if (!h) return RAE_EINVAL;
     if (!h->params_bound) return fail(h, RAE_ENOTBOUND, "parameters are not bound (rae_bind_params)");
-    if (!indptr || !indices || !labels || !probs || n_rows < 0 || n_rows > h->B) return fail(h, RAE_EINVAL, "rae_label_explicit: bad argument");
+    if (!w_shards || !indptr || !indices || !labels || n_rows < 0) return fail(h, RAE_EINVAL, "rae_label_shards: bad argument");
     h->launches = 0;
-    if (n_rows == 0) return RAE_OK;
-    return launch_encoder_forward(h, indptr, indices, (int)n_rows, probs, nullptr, nullptr, labels, (cudaStream_t)stream);
+    return launch_label_shards(h, w_shards, world, indptr, indices, n_rows, labels, probs, (cudaStream_t)stream);
 }
 
 int rae_train_step_end(rae_engine* h, void* stream) {

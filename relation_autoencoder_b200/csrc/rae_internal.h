@@ -213,6 +213,9 @@ int fail(rae_engine* h, int code, const char* fmt, ...);
 // ---- encoder (rae_encoder.cu) ----
 int launch_encoder_forward(rae_engine* h, const int32_t* indptr, const int32_t* indices, int B, float* q, float* logq,
                            float* sc_ent /* sc + SC_ENT, stride SC_N, may be null */, int64_t* labels, cudaStream_t st);
+// the same encoder over n_rows examples whose W is row-sharded over `world` ranks (rae_label_shards); probs may be null
+int launch_label_shards(rae_engine* h, const void* const* w_shards, int world, const int32_t* indptr, const int32_t* indices,
+                        int64_t n_rows, int64_t* labels, float* probs, cudaStream_t st);
 
 // ---- decoder, SIMT contraction (rae_decoder_simt.cu) ----
 int simt_supported(const rae_engine* h, char* why, size_t n);

@@ -24,6 +24,9 @@ a sum over examples divided by the global Z (learning/OieModel.py:90).
   summed gradient.  In (4) the owner applies W over its WHOLE shard (``rae_shard_apply``): per element the summed
   contributions (0 for a row no rank touched), then adj*(l1*sgn + 2*l2*w), then the rule - the order of the single-GPU
   dense update.
+* labelling (``label_rows``): any rows of a split are labelled straight from the owners' W shards with one
+  ``rae_label_shards`` call (no collective), in the single-GPU summation order; it is issued on the caller's stream behind
+  the step's "every owner has applied" barrier, and the next step's applies wait behind its first barrier.
   Fixed orders everywhere: bitwise reproducible for a given world size.  (Backends without peer memory - the NumPy
   backend of the CPU tests - order (3) and (5) with the dense all-reduce and a one-element cost all-reduce.)
 * routing (which rows, which slots, who owns what) depends only on the ids: the plans of ALL batches are built at bind
@@ -225,6 +228,46 @@ class GranularStep:
 
     def plans_changed(self, de):
         pass
+
+    def label_rows(self, de, indptr, indices, lo, hi, probs=True):
+        """Rows [lo, hi) of a split (int32 CSR, global feature ids) labelled on the compact table: per chunk, fetch the
+        chunk's distinct W rows, then label on their compact slots (backends implement fetch / label).  A chunk is at most
+        B rows whose distinct features fit the compact table, so no split is too wide for it.  A backend without peer
+        memory fetches collectively, so every rank issues as many fetches as the rank with the most chunks."""
+        cap = self.compact["W"].shape[0]
+        ip = indptr.to(torch.int64)
+        chunks = []
+        r = lo
+        while r < hi:
+            e = min(r + de.B, hi)
+            while True:
+                u, inv = torch.unique(indices[ip[r]:ip[e]], sorted=True, return_inverse=True)
+                if u.numel() <= cap:
+                    break
+                if e == r + 1:
+                    raise RuntimeError("label: row %d has %d distinct features, more than the %d rows of the compact table"
+                                       % (r, u.numel(), cap))
+                e = r + (e - r) // 2
+            chunks.append((r, e, u, inv))
+            r = e
+        n_fetch = len(chunks)
+        if de.world > 1:
+            t = torch.tensor([n_fetch], dtype=torch.int64, device=de.dev)
+            dist.all_reduce(t, op=dist.ReduceOp.MAX, group=de.group)
+            n_fetch = int(t.item())
+        labels, q = [], []
+        for i in range(n_fetch):
+            if i >= len(chunks):
+                self.fetch("W", torch.zeros(0, dtype=torch.int32, device=de.dev))
+                continue
+            r, e, u, inv = chunks[i]
+            self.fetch("W", u.to(torch.int32).contiguous())
+            lab, pr = self.label((ip[r:e + 1] - ip[r]).to(torch.int32).contiguous(), inv.to(torch.int32).contiguous())
+            labels.append(torch.as_tensor(lab).to(de.dev, torch.int64))
+            q.append(torch.as_tensor(pr).to(de.dev))
+        if not chunks:
+            return torch.zeros(0, dtype=torch.int64, device=de.dev), (torch.zeros((0, de.K), device=de.dev) if probs else None)
+        return torch.cat(labels), (torch.cat(q) if probs else None)
 
 
 class CudaBackend(GranularStep):
@@ -436,13 +479,15 @@ class CudaBackend(GranularStep):
         self.eng._check(self.lib.rae_dist_read_cost(self.h, self.eng._cost_ref), "train()")
         return self.eng._cost.value
 
-    def label(self, indptr: torch.Tensor, indices_compact: torch.Tensor):
-        n = indptr.numel() - 1
+    def label_rows(self, de, indptr, indices, lo, hi, probs=True):
+        """One rae_label_shards call: rows [lo, hi) read their W rows straight from the owners' shards (no collective, no
+        host synchronisation, no capacity limit)."""
+        n = hi - lo
         labels = torch.empty(n, dtype=torch.int64, device=self.device)
-        probs = torch.empty((n, self.de.K), dtype=torch.float32, device=self.device)
-        self.eng._check(self.lib.rae_label_explicit(self.h, self._p(indptr), self._p(indices_compact), n, self._p(labels),
-                                                    self._p(probs), self._stream), "rae_label_explicit")
-        return labels.cpu().numpy(), probs.cpu().numpy()
+        q = torch.empty((n, de.K), dtype=torch.float32, device=self.device) if probs else None
+        self.eng._check(self.lib.rae_label_shards(self.h, self.shard_buf["W"].peer_array(), de.world, C.c_void_p(indptr.data_ptr() + 4 * lo),
+                                                  self._p(indices), n, self._p(labels), self._p(q), self._stream), "rae_label_shards")
+        return labels, q
 
     def close(self):
         if self.eng is not None:
@@ -491,6 +536,7 @@ class DistributedEngine:
         self.nb = 0
         self._ready = False
         self._label_split = {}
+        self._train_csr32 = None
         self._profiling = False
         self._phase_log = []
 
@@ -561,12 +607,19 @@ class DistributedEngine:
             return x.to(self.dev, torch.int64)
         return torch.as_tensor(np.ascontiguousarray(x)).to(self.dev, torch.int64)
 
+    def _i32(self, x):
+        if isinstance(x, torch.Tensor):
+            return x.to(self.dev, torch.int32).contiguous()
+        return torch.as_tensor(np.ascontiguousarray(x)).to(self.dev, torch.int32).contiguous()
+
     def bind_split(self, split: str, indptr, indices, args1=None, args2=None):
         """Local rows of the split.  For 'train' (collective): routing plan of the feature rows of every batch."""
-        ip, ix = self._i64(indptr), self._i64(indices)
         if split != "train":
-            self._label_split[split] = (ip, ix)
+            # every row of the split (labels are per example: any partition of the rows gives the same labels)
+            self._label_split[split] = (self._i32(indptr), self._i32(indices))
             return
+        ip, ix = self._i64(indptr), self._i64(indices)
+        self._train_csr32 = None
         B = self.B
         nb = (ip.numel() - 1) // B
         if self.world > 1:
@@ -719,22 +772,28 @@ class DistributedEngine:
             raise RuntimeError("train(): the negatives passed for batch %d are not the columns of the bound epoch negatives" % b)
         return cost
 
+    def _label_csr(self, split: str):
+        if split != "train":
+            return self._label_split[split]
+        if self._train_csr32 is None:
+            self._train_csr32 = (self.ip.to(torch.int32).contiguous(), self.ix.to(torch.int32).contiguous())
+        return self._train_csr32
+
+    def label_rows(self, split: str, lo: int, hi: int, probs: bool = True):
+        """Labels (device int64 [hi-lo]) and q(r|x) ([hi-lo, K], or None with ``probs=False``) of rows [lo, hi) of the bound
+        split: every row of 'valid' / 'test', this rank's bound rows of 'train'.  The W rows are read from their owners;
+        the CUDA backend needs no collective (one rae_label_shards call)."""
+        ip, ix = self._label_csr(split)
+        lo, hi = int(lo), int(hi)
+        if not (0 <= lo <= hi <= ip.numel() - 1):
+            raise RuntimeError("label_rows(%r, %d, %d): the split has %d rows" % (split, lo, hi, ip.numel() - 1))
+        return self.backend.label_rows(self, ip, ix, lo, hi, probs)
+
     def label(self, split: str, batch_index: int):
-        """func['label_<split>'](batch_index) for this rank's rows: the needed W rows are read from their owners (no
-        collective with the CUDA backend)."""
+        """func['label_<split>'](batch_index) for this rank's rows [b*B, (b+1)*B) of the bound split (label_rows)."""
         B = self.B
-        if split == "train":
-            ip, ix = self.ip, self.ix
-        else:
-            ip, ix = self._label_split[split]
-        lo, hi = int(ip[batch_index * B].item()), int(ip[(batch_index + 1) * B].item())
-        feats = ix[lo:hi]
-        u, inv = torch.unique(feats, sorted=True, return_inverse=True)
-        if u.numel() > self.backend.compact["W"].shape[0]:
-            raise RuntimeError("label(): batch touches more feature rows than the compact table holds")
-        self.backend.fetch("W", u.to(torch.int32).contiguous())
-        return self.backend.label((ip[batch_index * B:(batch_index + 1) * B + 1] - lo).to(torch.int32).contiguous(),
-                                  inv.to(torch.int32).contiguous())
+        labels, q = self.label_rows(split, batch_index * B, (batch_index + 1) * B)
+        return labels.cpu().numpy(), q.cpu().numpy()
 
     # ------------------------------------------------------------------ misc
     def stats(self) -> dict:

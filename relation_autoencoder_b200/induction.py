@@ -83,6 +83,130 @@ def cuda_backend(inducer: "ReconstructInducer") -> Dict[str, Callable]:
     return func
 
 
+def check_global_batch(batch_size: int, world: int):
+    """--batch-size is the GLOBAL batch: every rank trains batch_size / world examples of it."""
+    if batch_size % world != 0:
+        raise ValueError("--batch-size %d is not divisible by the world size %d: each of the %d ranks trains batch-size / "
+                         "world examples of every global batch" % (batch_size, world, world))
+
+
+class _RankEngine(object):
+    """The inducer's handle on this rank's :class:`relation_autoencoder_b200.dist.DistributedEngine`: ``learn()`` hands it
+    the epoch's full negative arrays and global-batch slices, it passes on this rank's columns.  ``version`` counts the
+    parameter changes (steps, loads), so labels gathered for one state are reused until the next change."""
+
+    def __init__(self, de, rows, rank, B):
+        self.de, self.rows, self.rank, self.B = de, rows, rank, B
+        self._rows_dev = None
+        self.version = 0
+
+    def _cols(self, neg):
+        if isinstance(neg, np.ndarray):
+            return neg[:, self.rows]
+        if self._rows_dev is None or self._rows_dev.device != neg.device:
+            import torch
+            self._rows_dev = torch.as_tensor(self.rows, device=neg.device)
+        return neg[:, self._rows_dev]
+
+    def bind_epoch_negatives(self, neg1, neg2):
+        """Collective: the epoch's [S, n_train] arrays, identical on every rank; this rank's columns are bound."""
+        self.de.bind_epoch_negatives(self._cols(neg1), self._cols(neg2))
+
+    def train(self, batch_index, neg1, neg2):
+        """func['train'] on the global batch's [S, Bg] slices: this rank's columns go to the engine, the GLOBAL cost returns."""
+        lo, hi = self.rank * self.B, (self.rank + 1) * self.B
+        self.version += 1
+        return self.de.train(batch_index, neg1[:, lo:hi], neg2[:, lo:hi])
+
+    def train_device(self, batch_index, want_cost=True):
+        self.version += 1
+        return self.de.train_device(batch_index, want_cost)
+
+    def set_params_numpy(self, params, acc=None):
+        self.version += 1
+        self.de.set_params_numpy(params, acc)
+
+    def get_params_numpy(self):
+        return self.de.get_params_numpy()
+
+    def get_acc_numpy(self):
+        return self.de.get_acc_numpy()
+
+    def close(self):
+        self.de.close()
+
+
+def distributed_backend(inducer: "ReconstructInducer", backend_factory=None, group=None) -> Dict[str, Callable]:
+    """The contract of :func:`cuda_backend` on the ranks of a process group (one process per GPU of one node), through
+    :class:`relation_autoencoder_b200.dist.DistributedEngine`.  Collective: every rank calls it, and then the driver, with
+    the same arguments and the same seeded generator.
+
+    The reference's global-batch semantics at any world size: ``batch_size`` is the global batch Bg, each rank trains
+    B = Bg / world rows of it - global batch g is rows [g*Bg, (g+1)*Bg) and rank r trains rows [g*Bg + r*B, g*Bg + (r+1)*B).
+    The tail is dropped as in the reference, adj = Bg / N_train and Z is global.  Every rank draws the same epoch negatives
+    and binds its own columns.  ``func['label_<split>']`` returns the labels of the global batch (probs: None); the first
+    call after a parameter change labels the split's batch_reps * Bg rows, a share per rank (``label_rows``, no collective
+    with the CUDA backend), and all-gathers them into global order, so clustering and B-cubed see the single-process
+    vector.  ``backend_factory``: the local-compute backend of the engine (the CPU tests inject a float64 NumPy one)."""
+    import torch
+    import torch.distributed as dist
+
+    from .dist import DistributedEngine
+    rank, world = dist.get_rank(group), dist.get_world_size(group)
+    Bg = inducer.batch_size
+    check_global_batch(Bg, world)
+    B = Bg // world
+    data = inducer.data
+    tr = data.split['train']
+    nb = inducer.batch_reps['train']
+    rows = (np.arange(nb, dtype=np.int64)[:, None] * Bg + rank * B + np.arange(B, dtype=np.int64)[None, :]).reshape(-1)
+    ip = np.asarray(tr.indptr, dtype=np.int64)
+    counts = ip[rows + 1] - ip[rows]
+    loc_ip = np.zeros(rows.size + 1, dtype=np.int64)
+    loc_ip[1:] = np.cumsum(counts)
+    loc_ix = np.asarray(tr.indices)[np.repeat(ip[rows] - loc_ip[:-1], counts) + np.arange(loc_ip[-1], dtype=np.int64)]
+    de = DistributedEngine(inducer.decoder_type, inducer.relationNum, inducer.embedSize, inducer.neg_sample_num, B,
+                           data.get_dimensionality(), data.get_arg_voc_size(), tr.get_size(), lr=inducer.learningRate,
+                           l1=inducer.lambdaL1, l2=inducer.lambdaL2, alpha=inducer.alpha, optimizer=inducer.optimization,
+                           ext_reg=inducer.extendedReg, device=inducer.device, backend_factory=backend_factory, group=group)
+    de.set_params_numpy(inducer.initial_params, inducer.initial_acc)
+    de.bind_split('train', loc_ip, loc_ix, np.asarray(tr.args1)[rows], np.asarray(tr.args2)[rows])
+    for split in data.generate_split_keys():
+        if split != 'train':
+            de.bind_split(split, data.split[split].indptr, data.split[split].indices)
+    eng = _RankEngine(de, rows, rank, B)
+
+    def gather_labels(split):
+        """This split's labels of rows [0, batch_reps * Bg) in global order, on every rank (collective)."""
+        n_share = inducer.batch_reps[split] * B
+        if split == 'train':                  # this rank's own bound rows: the layout above gives their global order
+            mine, _ = de.label_rows('train', 0, n_share, probs=False)
+        else:
+            mine, _ = de.label_rows(split, rank * n_share, (rank + 1) * n_share, probs=False)
+        parts = [torch.empty_like(mine) for _ in range(world)] if world > 1 else [mine]
+        if world > 1:
+            dist.all_gather(parts, mine, group=group)
+        out = torch.stack(parts)              # [world, n_share]
+        if split == 'train':
+            out = out.reshape(world, -1, B).transpose(0, 1)
+        return out.reshape(-1).cpu().numpy()
+
+    cache = {}
+
+    def label(split, b):
+        if cache.get(split, (None,))[0] != eng.version:
+            cache[split] = (eng.version, gather_labels(split))
+        return cache[split][1][b * Bg:(b + 1) * Bg], None
+
+    func = {'label_' + split: (lambda b, _s=split: label(_s, b)) for split in data.generate_split_keys()}
+    func['train'] = eng.train
+    inducer.engine = eng
+    inducer.get_parameters = eng.get_params_numpy
+    inducer.get_accumulators = eng.get_acc_numpy
+    inducer.sharded, inducer.rank, inducer.world, inducer.dist_group = True, rank, world, group
+    return func
+
+
 class ReconstructInducer(object):
     def __init__(self, data, gold_standard, rng, nb_epochs, learning_rate, batch_size, embed_size, nb_relations,
                  nb_neg_samples, lambda1, lambda2, optimization, model_name, decoder_model, external_embeddings,
@@ -109,6 +233,8 @@ class ReconstructInducer(object):
         self.frequentEval = frequent_eval
         self.alpha = alpha
         self.device = device
+        # distributed_backend: the ranks of a process group (at any world size, 1 included), this process's rank of `world`
+        self.sharded, self.rank, self.world, self.dist_group = False, 0, 1, None
         self.out = out if out is not None else sys.stdout
         self._backend = backend if backend is not None else cuda_backend
         if self.extEmb:
@@ -172,8 +298,9 @@ class ReconstructInducer(object):
         t0 = time.perf_counter()
         self.learn(debug=False)
         train_duration = time.perf_counter() - t0
-        print('Compiling completed in {:.1f}s'.format(compile_duration), file=sys.stderr)
-        print('Training completed in {:.1f}s'.format(train_duration), file=sys.stderr)
+        if self.rank == 0:
+            print('Compiling completed in {:.1f}s'.format(compile_duration), file=sys.stderr)
+            print('Training completed in {:.1f}s'.format(train_duration), file=sys.stderr)
         self._print('Trained for {} epochs. Avg epoch duration: {:.1f}s'.format(self.cur_epoch, train_duration / float(max(1, self.cur_epoch))))
 
     def learn(self, debug=True):
@@ -191,7 +318,8 @@ class ReconstructInducer(object):
             neg_samples1 = self.negativeSampler.get_negative_samples(self.data.split['train'].args1.shape[0], self.neg_sample_num)
             neg_samples2 = self.negativeSampler.get_negative_samples(self.data.split['train'].args2.shape[0], self.neg_sample_num)
             B = self.batch_size
-            if self.device_sampler:
+            if self.device_sampler or self.sharded:
+                # sharded: every rank drew the same arrays and binds its own columns, whichever the sampler
                 self.engine.bind_epoch_negatives(neg_samples1, neg_samples2)
             for batch_ind in range(self.batch_reps['train']):
                 if self.device_sampler:
@@ -254,11 +382,16 @@ class ReconstructInducer(object):
 
     def save(self, directory: Optional[str] = None) -> str:
         """Portable checkpoint ``<models_path>/<model name>.npz``: parameters, AdaGrad accumulators (which the reference's
-        pickle of ``self`` loses, OieInduction.py:110-116 + Optimizers.py:12-15) and the run configuration."""
+        pickle of ``self`` loses, OieInduction.py:110-116 + Optimizers.py:12-15) and the run configuration.  The format
+        does not depend on the world size.  Several ranks: collective (the shards are gathered), rank 0 writes, and every
+        rank returns once the file is complete."""
         directory = directory if directory is not None else models_path
-        os.makedirs(directory, exist_ok=True)
         path = os.path.join(directory, self.modelName + '.npz')
         params, acc = self.get_parameters(), self.get_accumulators()
+        if self.rank != 0:
+            self._barrier()
+            return path
+        os.makedirs(directory, exist_ok=True)
         cfg = dict(decoder=self.decoder_type, relations=self.relationNum, embed_size=self.embedSize, batch_size=self.batch_size,
                    neg_samples=self.neg_sample_num, l1=self.lambdaL1, l2=self.lambdaL2, alpha=self.alpha, optimizer=self.optimization,
                    learning_rate=self.learningRate, epochs_done=self.cur_epoch, model_id=self.modelID, ext_reg=bool(self.extendedReg),
@@ -270,12 +403,19 @@ class ReconstructInducer(object):
         arrays.update(rng_keys=np.asarray(keys, dtype=np.uint32), rng_pos=np.int64(pos), rng_has_gauss=np.int64(has_gauss),
                       rng_cached_gaussian=np.float64(cached))
         np.savez(path, config=np.array(json.dumps(cfg)), **arrays)
+        self._barrier()
         return path
+
+    def _barrier(self):
+        if self.world > 1:
+            import torch.distributed as dist
+            dist.barrier(group=self.dist_group)
 
     def load(self, path: str):
         """Resume from a checkpoint written by :meth:`save`: parameters, AdaGrad accumulators, the epoch counter, the
         error / metric series and the generator state, so that training continues exactly where the saved run stopped
-        (works before or after the functions are compiled)."""
+        (works before or after the functions are compiled).  Any world size resumes a checkpoint of any other: each rank
+        keeps its own rows (collective once compiled on several ranks)."""
         ck = load_model(path)
         if self.engine is None and getattr(self, 'oracle_model', None) is None:
             self.initial_params = {k: v for k, v in ck['params'].items()}
@@ -353,7 +493,7 @@ def get_command_args(program_name, argv=None):
     p.add_argument('--freq-eval', dest='freq_eval', action='store_true', default='False', help='use frequent evaluation')
     p.add_argument('--alpha', type=float, default=1.0, help='the alpha coefficient for scaling the entropy term')
     p.add_argument('--seed', type=int, default=2, help='a seed number')
-    p.add_argument('--device', type=int, default=0, help='CUDA device index')
+    p.add_argument('--device', type=int, default=None, help='CUDA device index (default 0; several ranks use LOCAL_RANK)')
     p.add_argument('--device-sampler', dest='device_sampler', action='store_true',
                    help='draw the negative samples on the GPU (bit-identical ids, same random stream)')
     if argv is None:
@@ -381,17 +521,52 @@ def get_command_args(program_name, argv=None):
 
 
 def main(argv=None, backend=None):
-    print("Relation Learner")
+    """The command line.  Under ``torchrun --nproc-per-node N`` (WORLD_SIZE > 1) every process trains on GPU LOCAL_RANK
+    through :func:`distributed_backend`: NCCL is initialised here (unless the caller already formed the process group),
+    ``--batch-size`` is the global batch, only rank 0 prints the training log and writes the checkpoint, and the process
+    group is destroyed on the way out.  ``backend`` replaces the binding (cuda_backend, or distributed_backend on several
+    ranks).  With WORLD_SIZE unset or 1 this is the single-GPU driver."""
+    world = int(os.environ.get('WORLD_SIZE', '1'))
+    if world <= 1:
+        return _run(argv, backend)
+    import torch
+    import torch.distributed as dist
+    rank, local = int(os.environ['RANK']), int(os.environ.get('LOCAL_RANK', '0'))
+    out = sys.stdout if rank == 0 else open(os.devnull, 'w')
+    own_group = False
+    try:
+        args = get_command_args('induction', argv)
+        if args.device is not None:
+            raise ValueError("--device cannot be combined with several ranks: rank %d uses GPU LOCAL_RANK = %d" % (rank, local))
+        check_global_batch(args.batch_size, world)
+        if not dist.is_initialized():
+            torch.cuda.set_device(local)
+            dist.init_process_group('nccl', device_id=torch.device('cuda', local))
+            own_group = True
+        return _run(argv, backend if backend is not None else distributed_backend, out=out, device=local, rank=rank)
+    finally:
+        if own_group:
+            dist.destroy_process_group()
+        if out is not sys.stdout:
+            out.close()
+
+
+def _run(argv, backend, out=None, device=None, rank=0):
+    out = out if out is not None else sys.stdout
+    print("Relation Learner", file=out)
     args = get_command_args('induction', argv)
     rand = np.random.RandomState(seed=args.seed)
-    indexed_data, gold_standard = load_data(args.dataset, rand, verbose=True)
+    indexed_data, gold_standard = load_data(args.dataset, rand, verbose=rank == 0)
     inducer = ReconstructInducer(indexed_data, gold_standard, rand, args.epochs, args.learning_rate, args.batch_size,
                                  args.embed_size, args.relations, args.neg_samples, args.l1, args.l2, args.optimizer,
                                  args.model_name, args.decoder, args.ext_emb, args.ext_reg, args.freq_eval, args.alpha,
-                                 backend=backend, device=args.device, device_sampler=args.device_sampler)
+                                 backend=backend, device=device if device is not None else (args.device or 0), out=out,
+                                 device_sampler=args.device_sampler)
     inducer.train()
     path = inducer.save()
-    print('Saved', path)
+    print('Saved', path, file=out)
+    if inducer.sharded:
+        inducer._release()                # collective: the peer mappings go before the process group
     return inducer
 
 
