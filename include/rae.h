@@ -280,6 +280,16 @@ int rae_copy_cost(rae_engine* h, double* dst_device, void* stream);
  * caller stream behind this kernel. */
 int rae_label_shards(rae_engine* h, const void* const* w_shards, int32_t world, const int32_t* indptr,
                      const int32_t* indices, int64_t n_rows, int64_t* labels, float* probs, void* stream);
+/* func['label_<split>'] with the k most probable relations per row instead of the argmax (RelationClassifier.py:39-48;
+ * the posteriors of OieInduction.py:240-250 without materialising [n_rows, K]).  W lookup, CSR conventions, n_rows and
+ * stream ordering exactly as rae_label_shards (world = 1 with the handle's bound W is the single-table case).
+ * ids int32 [n_rows, k], row-major: the k highest-scoring relations, score descending, equal scores by ascending relation
+ * id (so ids[:, 0] are rae_label_shards' labels).  probs [n_rows, k] or NULL (not written): their softmax probabilities,
+ * bit-identical to rae_label_shards' probs[i, ids[i, j]].  1 <= k <= min(K, RAE_MAX_TOPK); k, world or a null shard out
+ * of range return RAE_EINVAL before any launch; n_rows = 0 launches nothing. */
+#define RAE_MAX_TOPK 16
+int rae_label_topk(rae_engine* h, const void* const* w_shards, int32_t world, const int32_t* indptr,
+                   const int32_t* indices, int64_t n_rows, int32_t k, int32_t* ids, float* probs, void* stream);
 
 /* ---- negative sampling on the device (replaces NegativeExampleGenerator.get_negative_samples, NegativeExampleGenerator.py:14-32)
  * out[i] = searchsorted(cum, uniform(0, cum_last)) for i in [0, n), bit-exact with the reference's host recipe on a legacy

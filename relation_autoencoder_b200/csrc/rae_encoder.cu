@@ -1,5 +1,5 @@
 // Kernel 1: encoder.  One warp per example: gather-sum of the example's W rows from the binary CSR batch, + Wb,
-// fused K-way softmax, entropy (training) or argmax (labelling).
+// fused K-way softmax, entropy (training), argmax (labelling) or the k best relations (top-k labelling).
 //   reference: sparse.dot(x_feats, W) + Wb ; T.nnet.softmax ; T.argmax   learning/models/encoders/RelationClassifier.py:35-36,45-47
 //              entropy = alpha * -sum(log(q) * q)                       learning/OieModel.py:81
 // HBM-bound: nnz*K*4 bytes of W rows per batch; every lane keeps UNROLL x KT independent row loads in flight.
@@ -61,13 +61,79 @@ struct ShardTables {
     __device__ __forceinline__ const float* row(Key k, int) const { return k; }
 };
 
-template <int KT, class Rows = DenseTable>
+// The warp's row again, read from the special registers at the store: the gather loop of the scalar KT = 8 body keeps
+// every register busy, and a row index kept live across it spills.
+__device__ __forceinline__ size_t row_of_warp() {
+    unsigned cta, tid, ntid;
+    asm volatile("mov.u32 %0, %%ctaid.x;" : "=r"(cta));
+    asm volatile("mov.u32 %0, %%tid.x;" : "=r"(tid));
+    asm volatile("mov.u32 %0, %%ntid.x;" : "=r"(ntid));
+    return ((size_t)cta * ntid + tid) >> 5;
+}
+
+// Top-k output (TopK = true, rae_label_topk): the k best relations of the warp's row b, by score descending and then
+// relation id ascending (the first-max rule of the labels, extended), into ids[b*k ..] and, when q is not NULL, their softmax
+// probabilities expf(z - lse) into q[b*k ..].  e[s] is the score of relation id(s) of this lane: lane + 32s on the scalar
+// path, 4(lane + 32(s/4)) + s%4 on the 16-byte path.  Each lane keeps its best score not taken yet; k rounds of butterfly
+// arg-max pick the winner, and only the lane that owns it marks it in its bitmask and rescans.  Lane j keeps the winner of
+// round j, so a row's k results leave in one coalesced store.  Everything stays in registers: e is only indexed by
+// unrolled (compile-time) s, and slots past K start out taken so that the rescan needs no relation ids.
+template <bool V4>
+__device__ __forceinline__ int topk_id(int lane, int s) { return V4 ? 4 * (lane + 32 * (s >> 2)) + (s & 3) : lane + 32 * s; }
+
+template <int N, bool V4>
+__device__ __forceinline__ void best_untaken(const float (&e)[N], int lane, unsigned taken, float& bv, int& bi) {
+    bv = -INFINITY;
+    int bs = -1;
+#pragma unroll
+    for (int s = 0; s < N; ++s)
+        if (!((taken >> s) & 1u) && e[s] > bv) { bv = e[s]; bs = s; }       // ascending id: first max wins
+    bi = bs < 0 ? 0x7fffffff : topk_id<V4>(lane, bs);
+}
+
+template <int N, bool V4>
+__device__ __forceinline__ void store_topk(const float (&e)[N], int K, int lane, float lse, size_t b, int k,
+                                           int32_t* __restrict__ ids, float* __restrict__ q) {
+    static_assert(N <= 32, "one bit per owned score");
+    unsigned taken = 0u;
+#pragma unroll
+    for (int s = 0; s < N; ++s)
+        if (topk_id<V4>(lane, s) >= K) taken |= 1u << s;
+    float bv;
+    int bi;
+    best_untaken<N, V4>(e, lane, taken, bv, bi);
+    float my_v = 0.f;
+    int my_i = 0;
+    for (int j = 0; j < k; ++j) {
+        float wv = bv;
+        int wi = bi;
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {
+            const float ov = __shfl_xor_sync(kFull, wv, o);
+            const int oi = __shfl_xor_sync(kFull, wi, o);
+            if (ov > wv || (ov == wv && oi < wi)) { wv = ov; wi = oi; }
+        }
+        if (lane == j) { my_v = wv; my_i = wi; }
+        const int owner = V4 ? (wi >> 2) & 31 : wi & 31;
+        if (wi < K && owner == lane) {
+            taken |= 1u << (V4 ? ((wi >> 7) << 2) | (wi & 3) : wi >> 5);
+            best_untaken<N, V4>(e, lane, taken, bv, bi);
+        }
+    }
+    if (lane < k) {
+        ids[b * k + lane] = my_i;
+        if (q != nullptr) q[b * k + lane] = expf(my_v - lse);
+    }
+}
+
+template <int KT, class Rows = DenseTable, bool TopK = false>
 __global__ void __launch_bounds__(256) k_encoder_forward(const int32_t* __restrict__ indptr,
                                                          const int32_t* __restrict__ indices,
                                                          typename Rows::Arg W, const float* __restrict__ Wb,
                                                          typename Rows::Index B, int K, float alpha, float* __restrict__ q,
                                                          float* __restrict__ logq, float* __restrict__ sc_ent,
-                                                         int sc_stride, int64_t* __restrict__ labels) {
+                                                         int sc_stride, int64_t* __restrict__ labels, int topk,
+                                                         int32_t* __restrict__ topk_ids) {
     const Rows rows(W);
     const int lane = threadIdx.x & 31;
     const typename Rows::Index b = Rows::example();
@@ -111,7 +177,7 @@ __global__ void __launch_bounds__(256) k_encoder_forward(const int32_t* __restri
         int k = lane + 32 * t;
         if (k < K && z[t] > m) { m = z[t]; arg = k; }   // ascending k per lane: first max wins
     }
-    if (labels != nullptr) {
+    if (!TopK && labels != nullptr) {
         float bm = m;
         int ba = arg;
 #pragma unroll
@@ -131,6 +197,10 @@ __global__ void __launch_bounds__(256) k_encoder_forward(const int32_t* __restri
     }
     s = warp_sum(s);
     const float lse = m + logf(s);
+    if (TopK) {
+        store_topk<KT, false>(z, K, lane, lse, row_of_warp(), topk, topk_ids, q);
+        return;
+    }
     float ent = 0.f;
     const bool store_q = !Rows::kOptionalQ || q != nullptr;
 #pragma unroll
@@ -152,13 +222,14 @@ __global__ void __launch_bounds__(256) k_encoder_forward(const int32_t* __restri
 
 // K % 4 == 0: every lane owns QT float4 (16-byte row loads, one instruction per W row for K <= 128) and UNROLL rows
 // are in flight together.
-template <int QT, class Rows = DenseTable>
+template <int QT, class Rows = DenseTable, bool TopK = false>
 __global__ void __launch_bounds__(256) k_encoder_forward_v4(const int32_t* __restrict__ indptr,
                                                             const int32_t* __restrict__ indices,
                                                             typename Rows::Arg W, const float* __restrict__ Wb,
                                                             typename Rows::Index B, int K, float alpha, float* __restrict__ q,
                                                             float* __restrict__ logq, float* __restrict__ sc_ent,
-                                                            int sc_stride, int64_t* __restrict__ labels) {
+                                                            int sc_stride, int64_t* __restrict__ labels, int topk,
+                                                            int32_t* __restrict__ topk_ids) {
     pdl_enter();
     const Rows rows(W);
     const int lane = threadIdx.x & 31;
@@ -210,7 +281,7 @@ __global__ void __launch_bounds__(256) k_encoder_forward_v4(const int32_t* __res
                 if (e[c] > m) { m = e[c]; arg = 4 * qi + c; }     // ascending k per lane: first max wins
         }
     }
-    if (labels != nullptr) {
+    if (!TopK && labels != nullptr) {
         float bm = m;
         int ba = arg;
 #pragma unroll
@@ -230,6 +301,15 @@ __global__ void __launch_bounds__(256) k_encoder_forward_v4(const int32_t* __res
     }
     s = warp_sum(s);
     const float lse = m + logf(s);
+    if (TopK) {
+        float e[4 * QT];
+#pragma unroll
+        for (int t = 0; t < QT; ++t) {
+            e[4 * t] = z[t].x; e[4 * t + 1] = z[t].y; e[4 * t + 2] = z[t].z; e[4 * t + 3] = z[t].w;
+        }
+        store_topk<4 * QT, true>(e, K, lane, lse, row_of_warp(), topk, topk_ids, q);
+        return;
+    }
     float ent = 0.f;
     const bool store_q = !Rows::kOptionalQ || q != nullptr;
 #pragma unroll
@@ -252,10 +332,12 @@ __global__ void __launch_bounds__(256) k_encoder_forward_v4(const int32_t* __res
 namespace {
 
 // One launch of the encoder over n examples with the W lookup of policy Rows.  w_aligned: every row of W starts on 16 bytes
-// when K % 4 == 0 (the 16-byte path also needs Wb, q and log q aligned).
-template <class Rows>
+// when K % 4 == 0 (the 16-byte path also needs Wb, q and log q aligned; the top-k output stores q one float per lane, so
+// there only Wb counts and the path is the one rae_label_shards takes with probs NULL or aligned).
+template <class Rows, bool TopK = false>
 int launch_encoder(rae_engine* h, const int32_t* indptr, const int32_t* indices, typename Rows::Arg W, bool w_aligned,
-                   typename Rows::Index n, float* q, float* logq, float* sc_ent, int64_t* labels, cudaStream_t st) {
+                   typename Rows::Index n, float* q, float* logq, float* sc_ent, int64_t* labels, cudaStream_t st,
+                   int topk = 0, int32_t* topk_ids = nullptr) {
     const int K = h->K;
     const int threads = 256;
     const int64_t blocks64 = ((int64_t)n * 32 + threads - 1) / threads;
@@ -265,12 +347,13 @@ int launch_encoder(rae_engine* h, const int32_t* indptr, const int32_t* indices,
     const float alpha = (float)h->cfg.alpha;
     const int kt = (K + 31) / 32;
     // 16-byte path: rows of W, q and log q must be 16-byte aligned (K % 4 == 0 and aligned base pointers)
-    const bool vec = (K & 3) == 0 && K <= 512 && w_aligned && (((uintptr_t)Wb | (uintptr_t)q | (uintptr_t)logq) & 15) == 0;
+    const uintptr_t outs = TopK ? 0 : ((uintptr_t)q | (uintptr_t)logq);
+    const bool vec = (K & 3) == 0 && K <= 512 && w_aligned && (((uintptr_t)Wb | outs) & 15) == 0;
     if (vec) {
         const int qt = (K / 4 + 31) / 32;
 #define RAE_ENC4(QT)                                                                                                 \
-    launch_pdl(k_encoder_forward_v4<QT, Rows>, dim3(blocks), dim3(threads), 0, st, indptr, indices, W, Wb, n, K, alpha, q, logq, sc_ent, SC_N, \
-               labels)
+    launch_pdl(k_encoder_forward_v4<QT, Rows, TopK>, dim3(blocks), dim3(threads), 0, st, indptr, indices, W, Wb, n, K, alpha, q, logq, \
+               sc_ent, SC_N, labels, topk, topk_ids)
         if (qt <= 1) RAE_ENC4(1);
         else if (qt <= 2) RAE_ENC4(2);
         else RAE_ENC4(4);
@@ -280,7 +363,8 @@ int launch_encoder(rae_engine* h, const int32_t* indptr, const int32_t* indices,
         return RAE_OK;
     }
 #define RAE_ENC(KT)                                                                                                  \
-    k_encoder_forward<KT, Rows><<<blocks, threads, 0, st>>>(indptr, indices, W, Wb, n, K, alpha, q, logq, sc_ent, SC_N, labels)
+    k_encoder_forward<KT, Rows, TopK><<<blocks, threads, 0, st>>>(indptr, indices, W, Wb, n, K, alpha, q, logq, sc_ent, SC_N, labels, \
+                                                                 topk, topk_ids)
     if (kt <= 1) RAE_ENC(1);
     else if (kt <= 2) RAE_ENC(2);
     else if (kt <= 4) RAE_ENC(4);
@@ -294,6 +378,20 @@ int launch_encoder(rae_engine* h, const int32_t* indptr, const int32_t* indices,
     return RAE_OK;
 }
 
+// the peer-pointer table of a row-sharded W (rae_label_shards, rae_label_topk); aligned: every shard starts on 16 bytes
+int shard_ptrs(rae_engine* h, const char* who, const void* const* w_shards, int world, ShardPtrs& sp, bool& aligned) {
+    if (world < 1 || world > RAE_MAX_PEERS) return fail(h, RAE_EINVAL, "%s: world %d out of range [1, %d]", who, world, RAE_MAX_PEERS);
+    sp = ShardPtrs{};
+    sp.world = world;
+    aligned = true;
+    for (int r = 0; r < world; ++r) {
+        if (!w_shards[r]) return fail(h, RAE_EINVAL, "%s: null W shard for rank %d", who, r);
+        sp.p[r] = static_cast<const float*>(w_shards[r]);
+        aligned = aligned && ((uintptr_t)sp.p[r] & 15) == 0;
+    }
+    return RAE_OK;
+}
+
 }  // namespace
 
 int launch_encoder_forward(rae_engine* h, const int32_t* indptr, const int32_t* indices, int B, float* q, float* logq,
@@ -304,17 +402,22 @@ int launch_encoder_forward(rae_engine* h, const int32_t* indptr, const int32_t* 
 
 int launch_label_shards(rae_engine* h, const void* const* w_shards, int world, const int32_t* indptr, const int32_t* indices,
                         int64_t n_rows, int64_t* labels, float* probs, cudaStream_t st) {
-    if (world < 1 || world > RAE_MAX_PEERS) return fail(h, RAE_EINVAL, "rae_label_shards: world %d out of range [1, %d]", world, RAE_MAX_PEERS);
-    ShardPtrs sp = {};
-    sp.world = world;
-    bool aligned = true;
-    for (int r = 0; r < world; ++r) {
-        if (!w_shards[r]) return fail(h, RAE_EINVAL, "rae_label_shards: null W shard for rank %d", r);
-        sp.p[r] = static_cast<const float*>(w_shards[r]);
-        aligned = aligned && ((uintptr_t)sp.p[r] & 15) == 0;
-    }
+    ShardPtrs sp;
+    bool aligned;
+    if (int rc = shard_ptrs(h, "rae_label_shards", w_shards, world, sp, aligned)) return rc;
     if (n_rows == 0) return RAE_OK;
     return launch_encoder<ShardTables>(h, indptr, indices, sp, aligned, n_rows, probs, nullptr, nullptr, labels, st);
+}
+
+int launch_label_topk(rae_engine* h, const void* const* w_shards, int world, const int32_t* indptr, const int32_t* indices,
+                      int64_t n_rows, int k, int32_t* ids, float* probs, cudaStream_t st) {
+    if (k < 1 || k > h->K || k > RAE_MAX_TOPK)
+        return fail(h, RAE_EINVAL, "rae_label_topk: k = %d outside [1, min(K = %d, %d)]", k, h->K, RAE_MAX_TOPK);
+    ShardPtrs sp;
+    bool aligned;
+    if (int rc = shard_ptrs(h, "rae_label_topk", w_shards, world, sp, aligned)) return rc;
+    if (n_rows == 0) return RAE_OK;
+    return launch_encoder<ShardTables, true>(h, indptr, indices, sp, aligned, n_rows, probs, nullptr, nullptr, nullptr, st, k, ids);
 }
 
 }  // namespace rae

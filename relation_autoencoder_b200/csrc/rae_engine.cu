@@ -767,6 +767,15 @@ int rae_label_shards(rae_engine* h, const void* const* w_shards, int32_t world, 
     return launch_label_shards(h, w_shards, world, indptr, indices, n_rows, labels, probs, (cudaStream_t)stream);
 }
 
+int rae_label_topk(rae_engine* h, const void* const* w_shards, int32_t world, const int32_t* indptr,
+                   const int32_t* indices, int64_t n_rows, int32_t k, int32_t* ids, float* probs, void* stream) {
+    if (!h) return RAE_EINVAL;
+    if (!h->params_bound) return fail(h, RAE_ENOTBOUND, "parameters are not bound (rae_bind_params)");
+    if (!w_shards || !indptr || !indices || !ids || n_rows < 0) return fail(h, RAE_EINVAL, "rae_label_topk: bad argument");
+    h->launches = 0;
+    return launch_label_topk(h, w_shards, world, indptr, indices, n_rows, k, ids, probs, (cudaStream_t)stream);
+}
+
 int rae_train_step_end(rae_engine* h, void* stream) {
     int rc = check_ready(h, false, false);
     if (rc) return rc;

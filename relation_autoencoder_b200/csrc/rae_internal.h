@@ -216,6 +216,9 @@ int launch_encoder_forward(rae_engine* h, const int32_t* indptr, const int32_t* 
 // the same encoder over n_rows examples whose W is row-sharded over `world` ranks (rae_label_shards); probs may be null
 int launch_label_shards(rae_engine* h, const void* const* w_shards, int world, const int32_t* indptr, const int32_t* indices,
                         int64_t n_rows, int64_t* labels, float* probs, cudaStream_t st);
+// the k best relations per row of the same encoder (rae_label_topk): ids int32 [n_rows, k], probs [n_rows, k] or null
+int launch_label_topk(rae_engine* h, const void* const* w_shards, int world, const int32_t* indptr, const int32_t* indices,
+                      int64_t n_rows, int k, int32_t* ids, float* probs, cudaStream_t st);
 
 // ---- decoder, SIMT contraction (rae_decoder_simt.cu) ----
 int simt_supported(const rae_engine* h, char* why, size_t n);

@@ -211,6 +211,26 @@ class Engine:
                                             self._stream), "rae_label_host")
         return labels, probs
 
+    def label_topk(self, indptr, indices, k: int, probs: bool = True):
+        """The k most probable relations of every row of a host or device int32 CSR (any number of rows, none dropped),
+        from the bound W and Wb in one ``rae_label_topk`` call -> (ids int32 [n, k], probs float32 [n, k] or None).
+        ids run by score descending, equal scores by ascending relation id, so ``ids[:, 0]`` is the argmax label."""
+        if not self.params:
+            raise RuntimeError("label_topk needs bound parameters (bind_params / set_params_numpy)")
+        ip, ix = self._dev_i32(indptr), self._dev_i32(indices)
+        n, k = ip.numel() - 1, int(k)
+        if ix.numel() == 0:                  # rows without features only: the library wants a non-null array
+            ix = torch.zeros(1, dtype=torch.int32, device=self.device)
+        size = max(n * k, 1)                 # non-null outputs for n == 0 too (the call then launches nothing)
+        ids = torch.empty(size, dtype=torch.int32, device=self.device)
+        q = torch.empty(size, dtype=torch.float32, device=self.device) if probs else None
+        w = (C.c_void_p * 1)(self.params["W"].data_ptr())
+        self._check(self.lib.rae_label_topk(self._h, w, 1, _ptr(ip), _ptr(ix), n, k, _ptr(ids), _ptr(q), self._stream),
+                    "rae_label_topk")
+        torch.cuda.synchronize(self.device)
+        ids = ids[:n * k].reshape(n, k).cpu().numpy()
+        return ids, (q[:n * k].reshape(n, k).cpu().numpy() if q is not None else None)
+
     # ------------------------------------------------------------------ introspection
     def last_probs(self) -> np.ndarray:
         out = torch.empty(self.B, self.K, dtype=torch.float32, device=self.device)

@@ -1,0 +1,204 @@
+"""The induced relations of a trained model: which relation each example gets, how confident the model is, and what each
+cluster holds.  This is what the reference's ``learn(debug=True)`` pickles (``OieInduction.py:230-234,395-402``),
+``compute_posteriors`` returns (``:240-250``) and ``Visualizator.print_clusters`` prints (``evaluation/Visuals.py:8-30``).
+
+    python -m relation_autoencoder_b200.export train_products/m.npz sample.pk --out exported/ \\
+        [--split train --split test ...] [--tsv new_sentences.txt ...] [--top-k 3] [--device 0]
+
+Every row of every labelled set is labelled, the tail batch included, by one ``rae_label_topk`` call on one GPU (the
+checkpoint does not depend on the world size it was trained on).  New sentences (``--tsv``) are featurised through the
+dataset's lexicon without changing it, so W still matches.  Per set NAME (a split, or a TSV file's stem) the output
+directory gets ``NAME.labels.npz``, ``NAME.examples.tsv`` and ``NAME.clusters.tsv``, and ``summary.json`` holds the
+checkpoint's configuration and per-set counts and B-cubed scores.
+"""
+from __future__ import annotations
+
+import argparse
+import json
+import os
+import sys
+from collections import Counter
+from typing import Callable, Dict, Optional, Sequence
+
+import numpy as np
+
+from .data import SPLIT_LABELS, unpickle_objects
+from .evaluation import SingleLabelClusterEvaluation
+from .induction import load_model
+from .preprocess import featurize
+
+TRIGGERS_PER_CLUSTER = 10        # settings.py elems_to_visualize: the triggers print_clusters shows per cluster
+GOLD_PER_CLUSTER = 5
+MAX_TOP_K = 16                   # RAE_MAX_TOPK (include/rae.h)
+
+
+def csr_of(examples, F: int):
+    """Binary CSR of the examples' feature ids (duplicates collapse, ascending within a row, as DatasetManager builds it)
+    -> (indptr int32 [n+1], indices int32 [nnz], n_features int32 [n])."""
+    rows = [np.unique(np.asarray(ex.features, dtype=np.int64)) for ex in examples]
+    for i, u in enumerate(rows):
+        if u.size and (u[0] < 0 or u[-1] >= F):
+            raise IndexError("feature id out of range [0, %d) in example %d" % (F, i))
+    n_features = np.array([u.size for u in rows], dtype=np.int32)
+    indptr = np.zeros(len(rows) + 1, dtype=np.int64)
+    np.cumsum(n_features, out=indptr[1:])
+    if indptr[-1] >= 2 ** 31:
+        raise ValueError("%d features in one set: more than an int32 CSR holds" % indptr[-1])
+    indices = np.concatenate(rows).astype(np.int32) if rows else np.zeros(0, np.int32)
+    return indptr.astype(np.int32), indices, n_features
+
+
+def cuda_labeller(ck: dict, device: int = 0):
+    """(labeller, close): ``labeller(indptr, indices, k) -> (ids, probs)`` through :meth:`Engine.label_topk` on the
+    checkpoint's parameters.  Only W and Wb are read, but the engine binds every parameter of the decoder."""
+    from .engine import Engine
+    cfg, p = ck['config'], ck['params']
+    F, K = p['W'].shape
+    N, d = p['A'].shape
+    B = int(cfg.get('batch_size', 1))
+    eng = Engine(cfg['decoder'], K, d, int(cfg.get('neg_samples', 1)), B, F, N, B, device=device)
+    eng.set_params_numpy(p)
+    return (lambda indptr, indices, k: eng.label_topk(indptr, indices, k, probs=True)), eng.close
+
+
+def _b3(gold: Dict[int, list], label: str, ids0: np.ndarray, n_rows: int):
+    """B-cubed of the clustering ids0[:n_rows] against the whole set's gold labels, as the driver scores a split; None
+    when no row of the set has a gold label."""
+    ev = SingleLabelClusterEvaluation(gold, label if label in SPLIT_LABELS else 'test')
+    if not ev.assessableElemSet:
+        return None
+    clusters: Dict[int, set] = {}
+    for i in range(n_rows):
+        clusters.setdefault(int(ids0[i]), set()).add(i)
+    ev.feed_induced_clusters(clusters)
+    f1, pre, rec = ev.compute_metrics()
+    return {'f1': f1, 'precision': pre, 'recall': rec}
+
+
+def _first_gold(gold: Dict[int, list], i: int) -> str:
+    g = gold.get(i) or ['']
+    return g[0]
+
+
+def _top(counter: Counter, n: int) -> str:
+    return ' '.join('%s:%d' % (s, c) for s, c in sorted(counter.items(), key=lambda t: (-t[1], t[0]))[:n])
+
+
+def _write_set(out_dir: str, name: str, examples, gold, ids, probs, n_features):
+    n, k = ids.shape
+    np.savez(os.path.join(out_dir, name + '.labels.npz'), ids=ids, probs=probs, n_features=n_features)
+    with open(os.path.join(out_dir, name + '.examples.tsv'), 'w', encoding='utf-8') as f:
+        f.write('index\targ1\targ2\ttrigger\tgold\trelation\tprob\tn_features\ttopk\n')
+        for i, ex in enumerate(examples):
+            topk = ' '.join('%d:%.6g' % (ids[i, j], probs[i, j]) for j in range(k))
+            f.write('%d\t%s\t%s\t%s\t%s\t%d\t%.6g\t%d\t%s\n' % (i, ex.arg1, ex.arg2, ex.trigger, _first_gold(gold, i),
+                                                              ids[i, 0], probs[i, 0], n_features[i], topk))
+    members: Dict[int, list] = {}
+    for i in range(n):
+        members.setdefault(int(ids[i, 0]), []).append(i)
+    order = sorted(members, key=lambda r: (-len(members[r]), r))
+    with open(os.path.join(out_dir, name + '.clusters.tsv'), 'w', encoding='utf-8') as f:
+        f.write('relation\tsize\tmean_prob\ttriggers\tgold\n')
+        for r in order:
+            m = members[r]
+            trig = Counter(examples[i].trigger for i in m)
+            gl = Counter(g for g in (_first_gold(gold, i) for i in m) if g != '')
+            f.write('%d\t%d\t%.6g\t%s\t%s\n' % (r, len(m), float(np.mean(probs[m, 0], dtype=np.float64)),
+                                                _top(trig, TRIGGERS_PER_CLUSTER), _top(gl, GOLD_PER_CLUSTER)))
+    return len(order)
+
+
+def export(checkpoint: str, dataset: str, out_dir: str, splits: Optional[Sequence[str]] = None, tsv: Sequence[str] = (),
+           k: int = 3, device: int = 0, labeller: Optional[Callable] = None) -> dict:
+    """Labels the requested splits of ``dataset`` (default: all of them) and the sentences of each ``tsv`` file with the
+    k most probable relations of the model in ``checkpoint``, writes the files the module docstring lists into
+    ``out_dir`` and returns the summary.  ``labeller(indptr, indices, k) -> (ids int32 [n, k], probs float32 [n, k])``
+    replaces the CUDA engine (there is no CPU fallback: without a GPU and without a labeller this raises).  The
+    arguments are checked before any GPU work."""
+    try:
+        ck = load_model(checkpoint)
+    except Exception as e:
+        raise ValueError("cannot load the checkpoint %s: %s" % (checkpoint, e)) from e
+    cfg = ck['config']
+    feats, lex, data, gold = unpickle_objects(dataset)
+    F = lex.get_feature_space_dimensionality()
+    W = ck['params'].get('W')
+    K = int(cfg['relations'])
+    if W is None or W.ndim != 2 or W.shape != (F, K):
+        raise ValueError("the checkpoint's W has shape %s, but the dataset's lexicon has F = %d features and the model K = %d "
+                         "relations: W must be (F, K) = (%d, %d); was the dataset extended after training?"
+                         % (None if W is None else tuple(W.shape), F, K, F, K))
+    k = int(k)
+    if not 1 <= k <= min(K, MAX_TOP_K):
+        raise ValueError("top-k %d is outside [1, min(K, %d)] = [1, %d]" % (k, MAX_TOP_K, min(K, MAX_TOP_K)))
+    splits = [s for s in SPLIT_LABELS if s in data] if splits is None else list(splits)
+    missing = [s for s in splits if s not in data]
+    if missing:
+        raise ValueError("split(s) %s are not in %s, which has %s" % (missing, dataset, [s for s in SPLIT_LABELS if s in data]))
+    names = list(splits)
+    for path in tsv:
+        stem = os.path.splitext(os.path.basename(path))[0]
+        if stem in names:
+            raise ValueError("the TSV file %s would be written as set %r, which is already a set of this export" % (path, stem))
+        names.append(stem)
+    sets = [(s, data[s], gold.get(s, {}), True) for s in splits]
+    for path, name in zip(tsv, names[len(splits):]):
+        ex, g = featurize(path, lex, feats)
+        sets.append((name, ex, g, False))
+
+    close = None
+    if labeller is None:
+        labeller, close = cuda_labeller(ck, device)
+    os.makedirs(out_dir, exist_ok=True)
+    B = int(cfg.get('batch_size', 1))
+    summary = {'checkpoint': os.path.abspath(checkpoint),
+               'config': {'decoder': cfg.get('decoder'), 'K': K, 'd': int(ck['params']['A'].shape[1]),
+                          'epochs_done': cfg.get('epochs_done'), 'model_id': cfg.get('model_id')},
+               'k': k, 'sets': {}}
+    try:
+        for name, examples, g, is_split in sets:
+            indptr, indices, n_features = csr_of(examples, F)
+            ids, probs = labeller(indptr, indices, k)
+            ids = np.ascontiguousarray(ids, dtype=np.int32)
+            probs = np.ascontiguousarray(probs, dtype=np.float32)
+            n = len(examples)
+            if ids.shape != (n, k) or probs.shape != (n, k):
+                raise RuntimeError("the labeller returned %s / %s for %d rows and k = %d" % (ids.shape, probs.shape, n, k))
+            n_clusters = _write_set(out_dir, name, examples, g, ids, probs, n_features)
+            entry = {'rows': n, 'rows_without_features': int((n_features == 0).sum()), 'clusters': n_clusters}
+            b3 = _b3(g, name, ids[:, 0], n)
+            if b3 is not None:
+                entry['b3'] = b3
+                if is_split:         # the rows the training log scores: whole batches only (OieInduction.py:96-98)
+                    entry['b3_driver_rows'] = _b3(g, name, ids[:, 0], (n // B) * B)
+            summary['sets'][name] = entry
+    finally:
+        if close is not None:
+            close()
+    with open(os.path.join(out_dir, 'summary.json'), 'w') as f:
+        json.dump(summary, f, indent=1)
+    return summary
+
+
+def main(argv=None):
+    p = argparse.ArgumentParser(prog='export', description='Exports the relations a trained model induces for a dataset '
+                                'and for new sentences: top-k labels, per-example table, cluster summaries, B-cubed.')
+    p.add_argument('checkpoint', help='the .npz checkpoint written by the training command')
+    p.add_argument('dataset', help='the pickled dataset the model was trained on')
+    p.add_argument('--out', required=True, help='output directory')
+    p.add_argument('--split', action='append', default=None, help='a split to label (repeatable; default: every split)')
+    p.add_argument('--tsv', action='append', default=[], help='a file of new sentences in the dataset format (repeatable)')
+    p.add_argument('--top-k', dest='k', type=int, default=3, help='relations kept per example (1 to min(K, 16))')
+    p.add_argument('--device', type=int, default=0, help='CUDA device index')
+    a = p.parse_args(argv)
+    summary = export(a.checkpoint, a.dataset, a.out, splits=a.split, tsv=a.tsv, k=a.k, device=a.device)
+    for name, s in summary['sets'].items():
+        b3 = s.get('b3')
+        print('%s: %d rows, %d without features, %d clusters%s' % (name, s['rows'], s['rows_without_features'], s['clusters'],
+              '' if b3 is None else ', B3 f1 %.4f' % b3['f1']))
+    print('Wrote', os.path.join(a.out, 'summary.json'))
+    return summary
+
+
+if __name__ == '__main__':
+    main(sys.argv[1:])

@@ -10,6 +10,8 @@ Restated here (not on the GPU path; pure string work):
   * the nine default extractors  OieFeatures.py:247-263 -> trigger, entityTypes, arg1_lower, arg2_lower, bow_clean,
                                  entity1Type, entity2Type, lexicalPattern, posPatternPath  (OieFeatures.py:27-44,132-245)
   * lexicon build + thresholding OiePreprocessor.py:113-208,244-287
+  * ``featurize``                new sentences through a trained model's frozen lexicon (export.py; no reference
+                                 counterpart: the reference's preprocessor only grows the lexicon)
 Stated divergences: (1) the reference takes its English stop-word list from NLTK (``OieFeatures.py:19``), which is not
 installed here - the list is embedded below (NLTK's 153-word list of that era); (2) Python 3 strings: ``lower()`` also
 lowers non-ASCII letters, Python 2 byte strings did not; (3) ``--batch-name`` (README.md:33-35 spelling) is accepted next
@@ -198,6 +200,35 @@ def load_features(raw_features_struct, lexicon, feature_extractors, examples_lis
         index += 1
     if verbose:
         print('  Unique thresholded feature keys: {}'.format(lexicon.nextIdPruned))
+
+
+def featurize(input_file, feature_lex, feature_names, verbose=False):
+    """New sentences through a trained model's FROZEN lexicon -> ([OieExample], {index: [gold tokens]}).
+
+    Same 9-field file as :func:`read_examples`; the extractors are the defaults named by the dataset's object 1
+    (``feature_names``: names or the stored extractor objects).  Every extracted 'name#value' string keeps the pruned id
+    the lexicon gave it and is dropped when it has none, so the feature space (F) stays the one the model was trained
+    on.  The lexicon is only read.  A line whose strings are all unknown gives an example without features."""
+    names = [getattr(f, '__name__', f) for f in feature_names]
+    unknown = [n for n in names if n not in FEATURE_FUNCTION_NAMES]
+    if unknown:
+        raise ValueError('feature extractors %r are not among the defaults %s: new text cannot be featurised like the dataset'
+                         % (unknown, sorted(FEATURE_FUNCTION_NAMES)))
+    by_name = {f.__name__: f for f in getBasicCleanFeatures()}
+    extractors = [by_name[n] for n in names]
+    examples, gold = [], {}
+    for index, feats in enumerate(read_examples(input_file, verbose=verbose)):
+        ids = []
+        for f in extractors:
+            res = f(_info(feats), feats[2], feats[3])
+            if res is not None:
+                for feat_el in generate_feature_element(res):
+                    feat_id = feature_lex.str2IdPruned.get(f.__name__ + "#" + feat_el)
+                    if feat_id is not None:
+                        ids.append(feat_id)
+        examples.append(OieExample(feats[2], feats[3], ids, feats[5], relation=feats[9]))
+        gold[index] = feats[-1].strip().split(' ')
+    return examples, gold
 
 
 def preprocess(input_file, pickled_dataset, batch='train', threshold=0, verbose=True):
