@@ -290,6 +290,26 @@ int rae_label_shards(rae_engine* h, const void* const* w_shards, int32_t world, 
 #define RAE_MAX_TOPK 16
 int rae_label_topk(rae_engine* h, const void* const* w_shards, int32_t world, const int32_t* indptr,
                    const int32_t* indices, int64_t n_rows, int32_t k, int32_t* ids, float* probs, void* stream);
+/* Argument prediction: rank every row's true arguments against all N entities under the bound model (no gold relation
+ * labels needed).  For row i with posterior q (RelationClassifier.py:39-48; a row without features scores Wb alone) and
+ * the decoder's vectors v = M A[args2], w = M^T A[args1], M = sum_r q_r C[:,:,r], c1 = C1 q, c2 = C2 q (v = w = 0 for
+ * model C, c1 = c2 = 0 for model A; Bilinear.py:33,58-59, SelectionalPreferences.py:31-32, BilinearPlusSP.py:35-37,68-72),
+ * the candidate scores of the reference's negative samples (Bilinear.py:36,47 and their SP / A+SP counterparts) are
+ *   slot 1 (x replaces args1): s1(x) = A[x].(v + c1) + Ab[x],   slot 2 (x replaces args2): s2(x) = A[x].(w + c2) + Ab[x]
+ * up to terms that do not depend on x, and rank_s[i] = 1 + #{x in [0, N), x != true_s : s_s(x) > s_s(true_s)}.  The true
+ * argument is scored by the same formula as every other entity: for model C under the args1 quirk of
+ * SelectionalPreferences.py:35 the slot-2 positive term of the cost never reads A[args2], so the slot-2 threshold is not
+ * the cost's u2; RAE_FLAG_FIX_SP_QUIRK changes only x-independent terms and so no rank.  Scores are fp32-accurate (FP16
+ * pair split on the tensor cores); an entity whose score ties the true one within rounding may count either way.
+ * indptr / indices / args1 / args2 follow rae_label_shards: device arrays, indptr has n_rows+1 entries and may start at
+ * any offset, indices are feature ids into the bound W; rank1 / rank2 int32 [n_rows] (device).  n_rows is NOT bounded by
+ * B; n_rows = 0 launches nothing.  Unbound parameters, an emit-only handle, null pointers or n_rows < 0 are refused
+ * before any launch.  Ids are not range-checked here (Engine.rank_arguments checks them on the host).
+ * The call runs the forward pass in chunks of B rows through the handle's per-batch scratch: afterwards rae_get_probs
+ * returns the posteriors of the last chunk, not those of the last training step.  It allocates (stream-ordered) a
+ * workspace of about 512 * N * ceil16(d) bytes for the scaled FP16 image of A plus the query images of up to 131072 rows. */
+int rae_rank_arguments(rae_engine* h, const int32_t* indptr, const int32_t* indices, const int32_t* args1,
+                       const int32_t* args2, int64_t n_rows, int32_t* rank1, int32_t* rank2, void* stream);
 
 /* ---- negative sampling on the device (replaces NegativeExampleGenerator.get_negative_samples, NegativeExampleGenerator.py:14-32)
  * out[i] = searchsorted(cum, uniform(0, cum_last)) for i in [0, n), bit-exact with the reference's host recipe on a legacy

@@ -2189,4 +2189,398 @@ int tc_gather_lr(rae_engine* h, const int32_t* a1, const int32_t* a2, cudaStream
     return RAE_OK;
 }
 
+namespace {
+// ------------------------------------------------------------------------------------------------------------
+// argument ranking (rae_rank_arguments): every held-out example's true argument against all N entities, per slot
+//   s1(x) = A[x].(v + c1) + Ab[x],  s2(x) = A[x].(w + c2) + Ab[x]      (+ terms that do not depend on x)
+//   rank = 1 + #{x != true : s(x) > s(true)}
+// The scores form the GEMM D[query, x] = U[query] . A[x] with fp32 accuracy through the FP16 pair split of the forward
+// contraction (hi.hi + hi.lo + lo.hi, power-of-two operand scales): the queries are the A operand, resident in TMEM,
+// 128 per tile; the candidates stream through shared memory in 128-row chunks, each ONE bulk copy of a pre-split image
+// that also carries the chunk's 128 biases (-inf for the padding rows beyond N).  The epilogue compares every
+// accumulator against the query's fp32 threshold t = U . A[true] + Ab[true] and counts in a register: no score is
+// stored.  Chain length per accumulator: 3 ceil(d / 16) <= 48 MMAs.
+// ------------------------------------------------------------------------------------------------------------
+constexpr int RK_WORKERS = 8;          // epilogue warps 0..7 (group g = warp / 4 takes accumulator columns [64 g, 64 g + 64))
+constexpr int RK_THREADS = 384;        // 8 epilogue + MMA issuer + producer + TMEM allocator + idle
+constexpr uint32_t RK_ACOL = 256;      // TMEM: accumulator stages [0, 256) (2 x 128 columns), query operand hi / lo from 256
+constexpr int RK_MAX_STAGES = 4;
+constexpr int RK_PASS_ROWS = 131072;   // examples per ranking launch (query image: 2 x 131072 x DH x 4 bytes)
+
+// bytes of one candidate chunk image: [hi/lo][kq < DH/8][row < 128] x 16 B, then float Ab[128]
+__host__ __device__ constexpr size_t rank_chunk_bytes(int DH) { return (size_t)512 * DH + 512; }
+
+// A -> candidate chunk images, scaled by pow2_scale(|max A|) (*amax, from k_tc_absmax).  Thread = (chunk, kq, row): it
+// reads 8 consecutive columns of one row of A and writes its 16-byte hi and lo units (consecutive threads: consecutive rows)
+__global__ void __launch_bounds__(256) k_rank_prep_a(const float* __restrict__ A, const float* __restrict__ Ab, int64_t N, int d,
+                                                     int DH, int NC, const uint32_t* __restrict__ amax, uint8_t* __restrict__ img) {
+    pdl_enter();
+    const float sA = pow2_scale(*amax);
+    const int KQ8 = DH / 8;
+    const size_t total = (size_t)NC * KQ8 * 128;
+    for (size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (size_t)gridDim.x * blockDim.x) {
+        const int r = (int)(idx & 127);
+        const int kq = (int)((idx >> 7) % KQ8);
+        const int64_t c = (int64_t)(idx / ((size_t)128 * KQ8));
+        const int64_t n = c * 128 + r;
+        const float* src = A + (size_t)n * d;
+        uint32_t hi[4], lo[4];
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+            const int j = 8 * kq + 2 * u;
+            const float x0 = (n < N && j < d) ? src[j] * sA : 0.f;
+            const float x1 = (n < N && j + 1 < d) ? src[j + 1] * sA : 0.f;
+            split_h2(x0, x1, hi[u], lo[u]);
+        }
+        uint8_t* base = img + (size_t)c * rank_chunk_bytes(DH);
+        uint4* u4 = reinterpret_cast<uint4*>(base);
+        u4[(size_t)kq * 128 + r] = make_uint4(hi[0], hi[1], hi[2], hi[3]);
+        u4[(size_t)(KQ8 + kq) * 128 + r] = make_uint4(lo[0], lo[1], lo[2], lo[3]);
+        if (kq == 0) reinterpret_cast<float*>(base + (size_t)512 * DH)[r] = n < N ? Ab[n] : -INFINITY;
+    }
+}
+
+// the rows of a partial last chunk, padded to B with empty rows and entity 0 (their ranks are not stored)
+__global__ void __launch_bounds__(256) k_rank_pad(const int32_t* __restrict__ indptr, const int32_t* __restrict__ a1,
+                                                  const int32_t* __restrict__ a2, int m, int B, int32_t* __restrict__ ip_out,
+                                                  int32_t* __restrict__ a1_out, int32_t* __restrict__ a2_out) {
+    pdl_enter();
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i <= B; i += gridDim.x * blockDim.x) {
+        ip_out[i] = indptr[min(i, m)];
+        if (i < B) { a1_out[i] = i < m ? a1[i] : 0; a2_out[i] = i < m ? a2[i] : 0; }
+    }
+}
+
+// query vectors of one forward chunk (ev after the contraction: v, w, c1, c2) -> the ranking kernel's operand image.
+// One warp per (example i < m, slot s); query index s * Rpad + off + i.  Per query: its own power-of-two scale
+// (pow2_scale(|max U|)), the unscale factor 1 / (s_U s_A), the fp32 threshold U . A[true] + Ab[true] and the true id.
+// Image: [query tile][word w < DH][row < 128] uint32, words w < DH/2 the hi FP16 pairs (columns 2w, 2w + 1), then lo.
+struct RankQArgs {
+    const float* ev; const float* A; const float* Ab; const int32_t* a1; const int32_t* a2; const uint32_t* amaxA;
+    uint32_t* qimg; float* qinv; float* qthr; int32_t* qtrue;
+    int m, off, Rpad, d, dp, DH, hasM, hasSP;
+};
+__global__ void __launch_bounds__(256) k_rank_queries(RankQArgs p) {
+    pdl_enter();
+    const int lane = threadIdx.x & 31;
+    const int gw = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    if (gw >= 2 * p.m) return;
+    const int s = gw & 1, i = gw >> 1;
+    const float* evb = p.ev + (size_t)i * E_NV * p.dp;
+    const float* vs = evb + (s == 0 ? E_V1 : E_V2) * p.dp;
+    const float* cs = evb + (s == 0 ? E_C1 : E_C2) * p.dp;
+    auto u_at = [&](int j) -> float {
+        if (j >= p.d) return 0.f;
+        float x = p.hasM ? vs[j] : 0.f;
+        if (p.hasSP) x += cs[j];
+        return x;
+    };
+    const int tru = s == 0 ? p.a1[i] : p.a2[i];
+    const float* Ar = p.A + (size_t)tru * p.d;
+    float dot = 0.f, amax = 0.f;
+    for (int j = lane; j < p.d; j += 32) {
+        const float x = u_at(j);
+        dot = fmaf(x, Ar[j], dot);
+        amax = fmaxf(amax, fabsf(x));
+    }
+    dot = warp_sum(dot);
+    amax = warp_max(amax);
+    const float sU = pow2_scale(__float_as_uint(amax));
+    const int q = s * p.Rpad + p.off + i;
+    if (lane == 0) {
+        p.qthr[q] = dot + p.Ab[tru];
+        p.qinv[q] = 1.f / (sU * pow2_scale(*p.amaxA));
+        p.qtrue[q] = tru;
+    }
+    uint32_t* img = p.qimg + (size_t)(q >> 7) * p.DH * 128 + (q & 127);
+    const int half = p.DH / 2;
+    for (int c = lane; c < half; c += 32) {
+        uint32_t hi, lo;
+        split_h2(u_at(2 * c) * sU, u_at(2 * c + 1) * sU, hi, lo);
+        img[(size_t)c * 128] = hi;
+        img[(size_t)(half + c) * 128] = lo;
+    }
+}
+
+struct RankArgs {
+    const uint8_t* aimg;        // candidate chunk images (k_rank_prep_a)
+    const uint32_t* qimg; const float* qinv; const float* qthr; const int32_t* qtrue;   // k_rank_queries
+    int32_t* out1; int32_t* out2;   // ranks of the pass's first example, zeroed; counts are added with integer atomics
+    int NC, DH, nbs;
+    int Rpad, nr;               // queries of slot s at [s Rpad, s Rpad + nr)
+    int n_tiles, splits;        // work item = (query tile, candidate range); item = tile * splits + split
+};
+
+// Persistent: CTA x takes items x, x + G, ...  When the query tiles outnumber the SMs every CTA sweeps ALL candidate
+// chunks in the same order at the same rate, so the CTAs resident together read each chunk from L2 (A is read from HBM
+// about once per wave instead of once per query tile).  With fewer tiles than SMs the candidates are split into ranges.
+__global__ void __launch_bounds__(RK_THREADS, 1) k_tc_rank(RankArgs p) {
+    pdl_enter();
+    extern __shared__ __align__(128) uint8_t smem_raw[];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const uint32_t CB = (uint32_t)rank_chunk_bytes(p.DH);
+    const uint32_t KQ8 = (uint32_t)p.DH / 8u;
+    const uint32_t HALF = (uint32_t)p.DH / 2u;         // TMEM columns of one query plane (two fp16 per column)
+    const int nbs = p.nbs;
+    uint8_t* smB = smem_raw;
+    uint64_t* bars = reinterpret_cast<uint64_t*>(smem_raw + (size_t)nbs * CB);
+    uint64_t* a_full = bars;                           // 8 epilogue-warp arrivals per item: query operand is in TMEM
+    uint64_t* b_full = bars + 1;                       // [RK_MAX_STAGES]
+    uint64_t* b_empty = b_full + RK_MAX_STAGES;        // [RK_MAX_STAGES] MMA commit + 8 epilogue warps (they read the biases)
+    uint64_t* t_full = b_empty + RK_MAX_STAGES;        // [2]
+    uint64_t* t_empty = t_full + 2;                    // [2] 8 epilogue-warp arrivals
+    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(t_empty + 2);
+    if (threadIdx.x == 0) {
+        mbar_init(a_full, RK_WORKERS);
+        for (int s = 0; s < nbs; ++s) { mbar_init(&b_full[s], 1); mbar_init(&b_empty[s], 1 + RK_WORKERS); }
+        for (int s = 0; s < 2; ++s) { mbar_init(&t_full[s], 1); mbar_init(&t_empty[s], RK_WORKERS); }
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    if (warp == RK_WORKERS + 2) {
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(512u) : "memory");
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    }
+    tc_fence_before();
+    __syncthreads();
+    tc_fence_after();
+    const uint32_t tmem_base = *tmem_slot;
+    const int n_items = p.n_tiles * p.splits;
+    auto range = [&](int item, int& c0, int& c1) {
+        const int split = item % p.splits;
+        c0 = (int)((long long)split * p.NC / p.splits);
+        c1 = (int)((long long)(split + 1) * p.NC / p.splits);
+    };
+
+    if (warp == RK_WORKERS + 1) {
+        // ===== producer: one bulk copy per candidate chunk =====
+        if (lane == 0) {
+            int it = 0;
+            for (int item = blockIdx.x; item < n_items; item += gridDim.x) {
+                int c0, c1;
+                range(item, c0, c1);
+                for (int c = c0; c < c1; ++c, ++it) {
+                    const int s = it % nbs;
+                    mbar_wait(&b_empty[s], ((it / nbs) & 1) ^ 1);
+                    mbar_expect_tx(&b_full[s], CB);
+                    bulk_g2s_pieces(smB + (size_t)s * CB, p.aimg + (size_t)c * CB, CB, &b_full[s]);
+                }
+            }
+        }
+    } else if (warp == RK_WORKERS) {
+        // ===== MMA issuer (one elected thread); k-loop unrolled so every descriptor is the stage base + a constant =====
+        if (elect_one()) {
+            const uint32_t idesc = make_idesc_f16(TC_M, 128);
+            const uint32_t a_hi = tmem_base + RK_ACOL, a_lo = a_hi + HALF;
+            const int ksteps = p.DH / 16;              // 1 .. 16
+            int it = 0, k = 0;
+            for (int item = blockIdx.x; item < n_items; item += gridDim.x, ++k) {
+                int c0, c1;
+                range(item, c0, c1);
+                mbar_wait(a_full, k & 1);
+                tc_fence_after();
+                for (int c = c0; c < c1; ++c, ++it) {
+                    const int s = it % nbs, ts = it & 1;
+                    mbar_wait(&t_empty[ts], ((it >> 1) & 1) ^ 1);
+                    mbar_wait(&b_full[s], (it / nbs) & 1);
+                    tc_fence_after();
+                    const uint32_t b_hi = smem_u32(smB + (size_t)s * CB);
+                    const uint64_t h0 = make_desc(b_hi, 128u * 16u, 128u);
+                    const uint64_t l0 = make_desc(b_hi + KQ8 * 128u * 16u, 128u * 16u, 128u);
+                    const uint32_t d0 = tmem_base + (uint32_t)(ts * 128);
+#pragma unroll
+                    for (int ks = 0; ks < 16; ++ks) {
+                        if (ks < ksteps) {
+                            const uint64_t hk = desc_advance(h0, (uint32_t)ks * 2u * 128u * 16u);
+                            const uint64_t lk = desc_advance(l0, (uint32_t)ks * 2u * 128u * 16u);
+                            tc_mma_f16_ts(d0, a_hi + 8u * ks, hk, idesc, ks > 0 ? 1u : 0u);   // hi * hi
+                            tc_mma_f16_ts(d0, a_hi + 8u * ks, lk, idesc, 1u);                 // hi * lo
+                            tc_mma_f16_ts(d0, a_lo + 8u * ks, hk, idesc, 1u);                 // lo * hi
+                        }
+                    }
+                    tc_commit(&b_empty[s]);
+                    tc_commit(&t_full[ts]);
+                }
+            }
+        }
+        __syncwarp();
+    } else if (warp < RK_WORKERS) {
+        // ===== query operand -> TMEM, then the counting epilogue =====
+        const int g = warp >> 2, q4 = warp & 3;
+        const int row = q4 * 32 + lane;
+        const uint32_t lane_base = tmem_base + ((uint32_t)(q4 * 32) << 16);
+        int it = 0;
+        for (int item = blockIdx.x; item < n_items; item += gridDim.x) {
+            const int tile = item / p.splits, split = item % p.splits;
+            int c0, c1;
+            range(item, c0, c1);
+            {
+                // group g writes plane g (hi, lo) of its 32 rows.  After the first item this warp has seen t_full of the
+                // previous item's last chunk: every MMA that read the old operand is done.
+                const uint32_t* src = p.qimg + ((size_t)tile * p.DH + g * HALF) * 128 + row;
+                for (uint32_t w0 = 0; w0 < HALF; w0 += 32) {
+                    uint32_t w[4][8];
+#pragma unroll
+                    for (int u = 0; u < 4; ++u)
+#pragma unroll
+                        for (int e = 0; e < 8; ++e) w[u][e] = (w0 + 8 * u < HALF) ? __ldg(src + (size_t)(w0 + 8 * u + e) * 128) : 0u;
+#pragma unroll
+                    for (int u = 0; u < 4; ++u)
+                        if (w0 + 8 * u < HALF) tc_st8u(lane_base + RK_ACOL + g * HALF + w0 + 8 * u, w[u]);
+                }
+                tc_wait_st();
+                tc_fence_before();
+                __syncwarp();
+                if (lane == 0) mbar_arrive(a_full);
+            }
+            const int qi = tile * 128 + row;
+            const int slot = qi >= p.Rpad ? 1 : 0, r = qi - slot * p.Rpad;
+            const bool valid = r < p.nr;
+            const float thr = valid ? p.qthr[qi] : INFINITY;     // padding rows count nothing
+            const float inv = valid ? p.qinv[qi] : 0.f;
+            const int tru = valid ? p.qtrue[qi] : -1;
+            int cnt = 0;
+            for (int c = c0; c < c1; ++c, ++it) {
+                const int s = it % nbs, ts = it & 1;
+                mbar_wait(&t_full[ts], (it >> 1) & 1);
+                mbar_wait(&b_full[s], (it / nbs) & 1);         // the biases: this phase cannot complete again before our b_empty arrival
+                tc_fence_after();
+                const float* ab = reinterpret_cast<const float*>(smB + (size_t)s * CB + (size_t)512 * p.DH) + 64 * g;
+#pragma unroll
+                for (int hf = 0; hf < 2; ++hf) {
+                    float t[32];
+                    tc_ld32(lane_base + (uint32_t)(ts * 128 + 64 * g + 32 * hf), t);
+                    if (hf == 1) {
+                        tc_fence_before();
+                        __syncwarp();
+                        if (lane == 0) mbar_arrive(&t_empty[ts]);
+                    }
+                    float a[32];
+#pragma unroll
+                    for (int x = 0; x < 32; x += 4) {
+                        const float4 v = *reinterpret_cast<const float4*>(ab + 32 * hf + x);
+                        a[x] = v.x; a[x + 1] = v.y; a[x + 2] = v.z; a[x + 3] = v.w;
+                    }
+                    const int tcol = tru - (c * 128 + 64 * g + 32 * hf);   // the true entity's column in these 32, if any
+                    if (__any_sync(kFull, (unsigned)tcol < 32u)) {
+#pragma unroll
+                        for (int x = 0; x < 32; ++x) cnt += (fmaf(t[x], inv, a[x]) > thr && x != tcol) ? 1 : 0;
+                    } else {
+#pragma unroll
+                        for (int x = 0; x < 32; ++x) cnt += fmaf(t[x], inv, a[x]) > thr ? 1 : 0;
+                    }
+                }
+                __syncwarp();
+                if (lane == 0) mbar_arrive(&b_empty[s]);
+            }
+            if (valid) atomicAdd((slot ? p.out2 : p.out1) + r, cnt + ((g == 0 && split == 0) ? 1 : 0));
+        }
+    }
+    tc_fence_before();
+    __syncthreads();
+    if (warp == RK_WORKERS + 2) {
+        tc_fence_after();
+        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
+    }
+}
+}  // namespace
+
+int launch_rank_arguments(rae_engine* h, const int32_t* indptr, const int32_t* indices, const int32_t* a1, const int32_t* a2,
+                          int64_t n_rows, int32_t* rank1, int32_t* rank2, cudaStream_t st) {
+    if (n_rows == 0) return RAE_OK;
+    const int B = h->B, d = h->d, DH = (d + 15) & ~15;
+    const int64_t N = h->cfg.N;
+    if (N > ((int64_t)1 << 31) - 256) return fail(h, RAE_EINVAL, "rae_rank_arguments: N = %lld entities are too many", (long long)N);
+    const int NC = (int)((N + 127) / 128);
+    const size_t CB = rank_chunk_bytes(DH);
+    const int nbs = (int)std::min<size_t>(RK_MAX_STAGES, ((size_t)h->max_smem_optin - 256) / CB);
+    if (nbs < 1) return fail(h, RAE_EINVAL, "rae_rank_arguments: d = %d needs %zu bytes per candidate stage", d, CB);
+    // more than half the shared memory: one CTA per SM, so no CTA waits in tcgen05.alloc for another's 512 columns
+    const size_t smem = std::max<size_t>((size_t)nbs * CB + 256, (size_t)h->max_smem_optin / 2 + 1024);
+    const int64_t cpp = std::max<int64_t>(1, RK_PASS_ROWS / B);              // forward chunks of B rows per ranking pass
+    const int64_t pass_rows = std::min<int64_t>(cpp, (n_rows + B - 1) / B) * B;
+    const int64_t Rmax = (pass_rows + 127) / 128 * 128;
+    auto al = [](size_t x) { return (x + 255) & ~(size_t)255; };
+    const size_t b_img = al((size_t)NC * CB), b_q = al((size_t)2 * Rmax * DH * 4), b_m = al((size_t)2 * Rmax * 4),
+                 b_pad = al((size_t)(B + 1) * 4), b_a = al((size_t)B * 4);
+    const size_t total = 256 + b_img + b_q + 3 * b_m + b_pad + 2 * b_a;
+    uint8_t* ws = nullptr;
+    cudaError_t e = cudaMallocAsync((void**)&ws, total, st);
+    if (e != cudaSuccess) return fail(h, RAE_ENOMEM, "rae_rank_arguments: %zu bytes of workspace: %s", total, cudaGetErrorString(e));
+    uint32_t* amax = reinterpret_cast<uint32_t*>(ws);
+    uint8_t* cur = ws + 256;
+    auto take = [&](size_t b) { uint8_t* r = cur; cur += b; return r; };
+    uint8_t* aimg = take(b_img);
+    uint32_t* qimg = reinterpret_cast<uint32_t*>(take(b_q));
+    float* qinv = reinterpret_cast<float*>(take(b_m));
+    float* qthr = reinterpret_cast<float*>(take(b_m));
+    int32_t* qtrue = reinterpret_cast<int32_t*>(take(b_m));
+    int32_t* pad_ip = reinterpret_cast<int32_t*>(take(b_pad));
+    int32_t* pad_a1 = reinterpret_cast<int32_t*>(take(b_a));
+    int32_t* pad_a2 = reinterpret_cast<int32_t*>(take(b_a));
+    auto body = [&]() -> int {
+        int rc;
+        RAE_CUDA(h, cudaMemsetAsync(rank1, 0, sizeof(int32_t) * (size_t)n_rows, st));
+        RAE_CUDA(h, cudaMemsetAsync(rank2, 0, sizeof(int32_t) * (size_t)n_rows, st));
+        RAE_CUDA(h, cudaMemsetAsync(amax, 0, sizeof(uint32_t), st));
+        launch_pdl(k_tc_absmax, dim3(h->num_sms * 8), dim3(256), 0, st, (const float*)h->P[RAE_P_A], (size_t)N * d, (const float*)nullptr,
+                   (size_t)0, (const float*)nullptr, (size_t)0, amax);
+        {
+            const size_t items = (size_t)NC * (DH / 8) * 128;
+            const int blocks = (int)std::min<size_t>((items + 255) / 256, (size_t)h->num_sms * 16);
+            launch_pdl(k_rank_prep_a, dim3(blocks), dim3(256), 0, st, (const float*)h->P[RAE_P_A], (const float*)h->P[RAE_P_AB], N, d, DH, NC,
+                       (const uint32_t*)amax, aimg);
+        }
+        h->launches += 2;
+        RAE_CUDA(h, cudaGetLastError());
+        if (h->use_tc && (rc = tc_prepare_c(h, st))) return rc;
+        RAE_CUDA(h, cudaFuncSetAttribute(k_tc_rank, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        for (int64_t row0 = 0; row0 < n_rows; row0 += pass_rows) {
+            const int nr = (int)std::min<int64_t>(pass_rows, n_rows - row0);
+            const int Rpad = (nr + 127) / 128 * 128;
+            for (int off = 0; off < nr; off += B) {
+                const int m = std::min(B, nr - off);
+                const int64_t r = row0 + off;
+                const int32_t* ip = indptr + r;
+                const int32_t* x1 = a1 + r;
+                const int32_t* x2 = a2 + r;
+                if (m < B) {
+                    launch_pdl(k_rank_pad, dim3((B + 256) / 256), dim3(256), 0, st, ip, x1, x2, m, B, pad_ip, pad_a1, pad_a2);
+                    h->launches++;
+                    RAE_CUDA(h, cudaGetLastError());
+                    ip = pad_ip; x1 = pad_a1; x2 = pad_a2;
+                }
+                if ((rc = launch_encoder_forward(h, ip, indices, B, h->q, h->logq, nullptr, nullptr, st))) return rc;
+                if (h->use_tc) {
+                    if ((rc = tc_prepare_p(h, x1, x2, st))) return rc;
+                    if ((rc = tc_forward(h, st))) return rc;
+                } else if ((rc = launch_bilinear_forward_simt(h, x1, x2, st))) {
+                    return rc;
+                }
+                RankQArgs q{};
+                q.ev = h->ev; q.A = h->P[RAE_P_A]; q.Ab = h->P[RAE_P_AB]; q.a1 = x1; q.a2 = x2; q.amaxA = amax;
+                q.qimg = qimg; q.qinv = qinv; q.qthr = qthr; q.qtrue = qtrue;
+                q.m = m; q.off = off; q.Rpad = Rpad; q.d = d; q.dp = h->dp; q.DH = DH; q.hasM = h->hasM; q.hasSP = h->hasSP;
+                launch_pdl(k_rank_queries, dim3((2 * m + 7) / 8), dim3(256), 0, st, q);
+                h->launches++;
+                RAE_CUDA(h, cudaGetLastError());
+            }
+            RankArgs p{};
+            p.aimg = aimg; p.qimg = qimg; p.qinv = qinv; p.qthr = qthr; p.qtrue = qtrue;
+            p.out1 = rank1 + row0; p.out2 = rank2 + row0;
+            p.NC = NC; p.DH = DH; p.nbs = nbs; p.Rpad = Rpad; p.nr = nr;
+            p.n_tiles = 2 * Rpad / 128;
+            // fewer query tiles than SMs: split the candidates, at least 8 chunks per range
+            p.splits = (int)std::max<int64_t>(1, std::min<int64_t>(h->num_sms / p.n_tiles, NC / 8));
+            const int G = std::min(h->num_sms, p.n_tiles * p.splits);
+            launch_pdl(k_tc_rank, dim3(G), dim3(RK_THREADS), smem, st, p);
+            h->launches++;
+            RAE_CUDA(h, cudaGetLastError());
+        }
+        return RAE_OK;
+    };
+    const int rc = body();
+    cudaFreeAsync(ws, st);
+    return rc;
+}
+
 }  // namespace rae

@@ -241,6 +241,9 @@ int tc_backward_recompute(rae_engine* h, cudaStream_t st);
 int tc_backward_dq(rae_engine* h, cudaStream_t st);
 int tc_backward_finish(rae_engine* h, cudaStream_t st);
 int tc_grad_dense(rae_engine* h, cudaStream_t st);
+// rae_rank_arguments: forward in chunks of B rows, query packing, one tcgen05 ranking launch per pass (rae_decoder_tc.cu)
+int launch_rank_arguments(rae_engine* h, const int32_t* indptr, const int32_t* indices, const int32_t* a1, const int32_t* a2,
+                          int64_t n_rows, int32_t* rank1, int32_t* rank2, cudaStream_t st);
 
 // ---- sort / segment / updates (rae_update.cu) ----
 size_t segwork_temp_bytes(int64_t n);

@@ -255,6 +255,15 @@ def generate_args(oie_dataset):
                 yield ex.arg2
 
 
+def entity_index(oie_dataset):
+    """(entity_freqs, id2Arg, arg2Id) of a dataset's entity strings (OieData.py:54,139-144): ids in the order of the strings'
+    first occurrence in ``generate_args``.  The one indexing of entities: DatasetManager trains with it and the export
+    ranks arguments with it."""
+    entity_freqs = Counter(generate_args(oie_dataset))
+    id2_arg, arg2_id = DatasetManager._index_elements(entity_freqs)
+    return entity_freqs, id2_arg, arg2_id
+
+
 class DatasetManager(object):
     def __init__(self, oie_dataset, feature_lex, rng, neg_sampling_distr_power=0.75, verbose=False):
         if 'train' not in oie_dataset:
@@ -263,10 +272,9 @@ class DatasetManager(object):
         self.rng = rng
         self.featureLex = feature_lex
         self.split: Dict[str, DatasetSplit] = {}
-        entity_freqs = Counter(generate_args(oie_dataset))
+        entity_freqs, self.id2Arg, self.arg2Id = entity_index(oie_dataset)
         if verbose:
             print('  feature space size: {}\n  number of unique entities: {}'.format(self.get_dimensionality(), len(entity_freqs)))
-        self.id2Arg, self.arg2Id = self._index_elements(entity_freqs)
         powered = [entity_freqs[self.id2Arg[i]] ** self.negSamplingDistrPower for i in range(len(self.id2Arg))]
         norm1 = float(sum(powered))                                   # OieData.py:57 (left-to-right python sum)
         self.negSamplingDistr = [x / norm1 for x in powered]          # :58

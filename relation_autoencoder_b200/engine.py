@@ -231,6 +231,45 @@ class Engine:
         ids = ids[:n * k].reshape(n, k).cpu().numpy()
         return ids, (q[:n * k].reshape(n, k).cpu().numpy() if q is not None else None)
 
+    def rank_arguments(self, indptr, indices, args1, args2):
+        """Entity ranks of every row's true arguments under the bound model, from one ``rae_rank_arguments`` call ->
+        (rank1 int32 [n], rank2 int32 [n]).  rank_s = 1 + the number of other entities whose candidate score in slot s
+        (the decoder's negative-sample score with that argument replaced) exceeds the true one's.  Host or device int32
+        CSR and argument ids of any length; entity ids must lie in [0, N) and feature ids in [0, F).  The call reuses the
+        handle's per-batch scratch, so ``last_probs`` afterwards no longer shows the last training step."""
+        if not self.params:
+            raise RuntimeError("rank_arguments needs bound parameters (bind_params / set_params_numpy)")
+        ip_h = np.asarray(indptr.cpu() if isinstance(indptr, torch.Tensor) else indptr, dtype=np.int64)
+        ix_h = np.asarray(indices.cpu() if isinstance(indices, torch.Tensor) else indices, dtype=np.int64)
+        a1_h = np.asarray(args1.cpu() if isinstance(args1, torch.Tensor) else args1, dtype=np.int64)
+        a2_h = np.asarray(args2.cpu() if isinstance(args2, torch.Tensor) else args2, dtype=np.int64)
+        n = ip_h.size - 1
+        if n < 0 or a1_h.shape != (n,) or a2_h.shape != (n,):
+            raise ValueError("rank_arguments: indptr has %d entries, args1 %s and args2 %s; expected n+1, (n,), (n,)"
+                             % (ip_h.size, a1_h.shape, a2_h.shape))
+        if n > 0 and (np.any(np.diff(ip_h) < 0) or ip_h[0] < 0 or ip_h[-1] > ix_h.size):
+            raise ValueError("rank_arguments: indptr is not a non-decreasing offset array into %d indices" % ix_h.size)
+        for name, a in (("args1", a1_h), ("args2", a2_h)):
+            if a.size and (a.min() < 0 or a.max() >= self.N):
+                raise ValueError("rank_arguments: %s holds entity ids outside [0, N = %d): min %d, max %d"
+                                 % (name, self.N, a.min(), a.max()))
+        used = ix_h[ip_h[0]:ip_h[-1]] if n > 0 else ix_h[:0]
+        if used.size and (used.min() < 0 or used.max() >= self.F):
+            raise ValueError("rank_arguments: indices hold feature ids outside [0, F = %d): min %d, max %d"
+                             % (self.F, used.min(), used.max()))
+        ip, ix = self._dev_i32(indptr), self._dev_i32(indices)
+        a1, a2 = self._dev_i32(args1), self._dev_i32(args2)
+        if ix.numel() == 0:                  # rows without features only: the library wants a non-null array
+            ix = torch.zeros(1, dtype=torch.int32, device=self.device)
+        if n == 0:
+            a1 = a2 = torch.zeros(1, dtype=torch.int32, device=self.device)
+        r1 = torch.empty(max(n, 1), dtype=torch.int32, device=self.device)
+        r2 = torch.empty(max(n, 1), dtype=torch.int32, device=self.device)
+        self._check(self.lib.rae_rank_arguments(self._h, _ptr(ip), _ptr(ix), _ptr(a1), _ptr(a2), n, _ptr(r1), _ptr(r2),
+                                                self._stream), "rae_rank_arguments")
+        torch.cuda.synchronize(self.device)
+        return r1[:n].cpu().numpy(), r2[:n].cpu().numpy()
+
     # ------------------------------------------------------------------ introspection
     def last_probs(self) -> np.ndarray:
         out = torch.empty(self.B, self.K, dtype=torch.float32, device=self.device)

@@ -3,13 +3,19 @@ cluster holds.  This is what the reference's ``learn(debug=True)`` pickles (``Oi
 ``compute_posteriors`` returns (``:240-250``) and ``Visualizator.print_clusters`` prints (``evaluation/Visuals.py:8-30``).
 
     python -m relation_autoencoder_b200.export train_products/m.npz sample.pk --out exported/ \\
-        [--split train --split test ...] [--tsv new_sentences.txt ...] [--top-k 3] [--device 0]
+        [--split train --split test ...] [--tsv new_sentences.txt ...] [--top-k 3] [--rank-arguments] [--device 0]
 
 Every row of every labelled set is labelled, the tail batch included, by one ``rae_label_topk`` call on one GPU (the
 checkpoint does not depend on the world size it was trained on).  New sentences (``--tsv``) are featurised through the
 dataset's lexicon without changing it, so W still matches.  Per set NAME (a split, or a TSV file's stem) the output
 directory gets ``NAME.labels.npz``, ``NAME.examples.tsv`` and ``NAME.clusters.tsv``, and ``summary.json`` holds the
 checkpoint's configuration and per-set counts and B-cubed scores.
+
+With ``--rank-arguments`` the decoder is measured as well, without gold labels: every example's true arguments are
+ranked against all entities (``rae_rank_arguments``: rank 1 + the number of entities whose score in that argument slot
+beats the true one's).  Per set, ``NAME.argranks.npz`` holds ``rank1`` and ``rank2`` (-1 for a row whose entity strings
+the dataset never saw: such rows cannot be ranked and are left out of the metrics), and ``summary.json`` gets
+``sets[NAME]['arguments']``: rows ranked and skipped, and MRR, mean rank and Hits@1/3/10 per slot and over both slots.
 """
 from __future__ import annotations
 
@@ -22,7 +28,7 @@ from typing import Callable, Dict, Optional, Sequence
 
 import numpy as np
 
-from .data import SPLIT_LABELS, unpickle_objects
+from .data import SPLIT_LABELS, entity_index, unpickle_objects
 from .evaluation import SingleLabelClusterEvaluation
 from .induction import load_model
 from .preprocess import featurize
@@ -30,6 +36,7 @@ from .preprocess import featurize
 TRIGGERS_PER_CLUSTER = 10        # settings.py elems_to_visualize: the triggers print_clusters shows per cluster
 GOLD_PER_CLUSTER = 5
 MAX_TOP_K = 16                   # RAE_MAX_TOPK (include/rae.h)
+HITS_AT = (1, 3, 10)
 
 
 def csr_of(examples, F: int):
@@ -59,6 +66,54 @@ def cuda_labeller(ck: dict, device: int = 0):
     eng = Engine(cfg['decoder'], K, d, int(cfg.get('neg_samples', 1)), B, F, N, B, device=device)
     eng.set_params_numpy(p)
     return (lambda indptr, indices, k: eng.label_topk(indptr, indices, k, probs=True)), eng.close
+
+
+def cuda_ranker(ck: dict, device: int = 0):
+    """(ranker, close): ``ranker(indptr, indices, args1, args2) -> (rank1, rank2)`` through :meth:`Engine.rank_arguments`
+    on the checkpoint's parameters, with the checkpoint's batch size as the forward pass's chunk."""
+    from .engine import Engine
+    cfg, p = ck['config'], ck['params']
+    F, K = p['W'].shape
+    N, d = p['A'].shape
+    B = int(cfg.get('batch_size', 1))
+    eng = Engine(cfg['decoder'], K, d, int(cfg.get('neg_samples', 1)), B, F, N, B, device=device)
+    eng.set_params_numpy(p)
+    return eng.rank_arguments, eng.close
+
+
+def rank_metrics(ranks: np.ndarray) -> dict:
+    """MRR, mean rank and Hits@1/3/10 of 1-based ranks (float64 means)."""
+    r = np.asarray(ranks, dtype=np.float64)
+    m = {'mrr': float(np.mean(1.0 / r)), 'mean_rank': float(np.mean(r))}
+    for k in HITS_AT:
+        m['hits@%d' % k] = float(np.mean(r <= k))
+    return m
+
+
+def _rank_set(out_dir: str, name: str, examples, arg2id: Dict[str, int], F: int, ranker) -> dict:
+    """Ranks the arguments of the rows whose two entity strings are in the dataset, writes NAME.argranks.npz and returns
+    the summary entry."""
+    n = len(examples)
+    a1 = np.array([arg2id.get(ex.arg1, -1) for ex in examples], dtype=np.int64)
+    a2 = np.array([arg2id.get(ex.arg2, -1) for ex in examples], dtype=np.int64)
+    ok = np.flatnonzero((a1 >= 0) & (a2 >= 0))
+    rank1 = np.full(n, -1, dtype=np.int32)
+    rank2 = np.full(n, -1, dtype=np.int32)
+    if ok.size:
+        indptr, indices, _ = csr_of([examples[i] for i in ok], F)
+        r1, r2 = ranker(indptr, indices, a1[ok].astype(np.int32), a2[ok].astype(np.int32))
+        r1 = np.asarray(r1, dtype=np.int32)
+        r2 = np.asarray(r2, dtype=np.int32)
+        if r1.shape != (ok.size,) or r2.shape != (ok.size,):
+            raise RuntimeError("the ranker returned %s / %s for %d rows" % (r1.shape, r2.shape, ok.size))
+        rank1[ok], rank2[ok] = r1, r2
+    np.savez(os.path.join(out_dir, name + '.argranks.npz'), rank1=rank1, rank2=rank2)
+    entry = {'rows_ranked': int(ok.size), 'rows_skipped': int(n - ok.size)}
+    if ok.size:
+        entry['arg1'] = rank_metrics(rank1[ok])
+        entry['arg2'] = rank_metrics(rank2[ok])
+        entry['both'] = rank_metrics(np.concatenate([rank1[ok], rank2[ok]]))
+    return entry
 
 
 def _b3(gold: Dict[int, list], label: str, ids0: np.ndarray, n_rows: int):
@@ -109,12 +164,15 @@ def _write_set(out_dir: str, name: str, examples, gold, ids, probs, n_features):
 
 
 def export(checkpoint: str, dataset: str, out_dir: str, splits: Optional[Sequence[str]] = None, tsv: Sequence[str] = (),
-           k: int = 3, device: int = 0, labeller: Optional[Callable] = None) -> dict:
+           k: int = 3, device: int = 0, labeller: Optional[Callable] = None, rank_arguments: bool = False,
+           ranker: Optional[Callable] = None) -> dict:
     """Labels the requested splits of ``dataset`` (default: all of them) and the sentences of each ``tsv`` file with the
     k most probable relations of the model in ``checkpoint``, writes the files the module docstring lists into
     ``out_dir`` and returns the summary.  ``labeller(indptr, indices, k) -> (ids int32 [n, k], probs float32 [n, k])``
-    replaces the CUDA engine (there is no CPU fallback: without a GPU and without a labeller this raises).  The
-    arguments are checked before any GPU work."""
+    replaces the CUDA engine (there is no CPU fallback: without a GPU and without a labeller this raises).  With
+    ``rank_arguments`` every set's arguments are ranked as well (module docstring); ``ranker(indptr, indices, args1,
+    args2) -> (rank1 int32 [n], rank2 int32 [n])`` replaces the CUDA engine there in the same way.  The arguments are
+    checked before any GPU work."""
     try:
         ck = load_model(checkpoint)
     except Exception as e:
@@ -141,6 +199,13 @@ def export(checkpoint: str, dataset: str, out_dir: str, splits: Optional[Sequenc
         if stem in names:
             raise ValueError("the TSV file %s would be written as set %r, which is already a set of this export" % (path, stem))
         names.append(stem)
+    arg2id = None
+    if rank_arguments:
+        _, _, arg2id = entity_index(data)
+        A = ck['params'].get('A')
+        if A is None or A.ndim != 2 or A.shape[0] != len(arg2id):
+            raise ValueError("the checkpoint's A has %s rows, but the dataset has %d entities: the model was not trained on "
+                             "this dataset" % (None if A is None else A.shape[0], len(arg2id)))
     sets = [(s, data[s], gold.get(s, {}), True) for s in splits]
     for path, name in zip(tsv, names[len(splits):]):
         ex, g = featurize(path, lex, feats)
@@ -149,6 +214,9 @@ def export(checkpoint: str, dataset: str, out_dir: str, splits: Optional[Sequenc
     close = None
     if labeller is None:
         labeller, close = cuda_labeller(ck, device)
+    close_ranker = None
+    if rank_arguments and ranker is None:
+        ranker, close_ranker = cuda_ranker(ck, device)
     os.makedirs(out_dir, exist_ok=True)
     B = int(cfg.get('batch_size', 1))
     summary = {'checkpoint': os.path.abspath(checkpoint),
@@ -171,10 +239,14 @@ def export(checkpoint: str, dataset: str, out_dir: str, splits: Optional[Sequenc
                 entry['b3'] = b3
                 if is_split:         # the rows the training log scores: whole batches only (OieInduction.py:96-98)
                     entry['b3_driver_rows'] = _b3(g, name, ids[:, 0], (n // B) * B)
+            if rank_arguments:
+                entry['arguments'] = _rank_set(out_dir, name, examples, arg2id, F, ranker)
             summary['sets'][name] = entry
     finally:
         if close is not None:
             close()
+        if close_ranker is not None:
+            close_ranker()
     with open(os.path.join(out_dir, 'summary.json'), 'w') as f:
         json.dump(summary, f, indent=1)
     return summary
@@ -189,13 +261,17 @@ def main(argv=None):
     p.add_argument('--split', action='append', default=None, help='a split to label (repeatable; default: every split)')
     p.add_argument('--tsv', action='append', default=[], help='a file of new sentences in the dataset format (repeatable)')
     p.add_argument('--top-k', dest='k', type=int, default=3, help='relations kept per example (1 to min(K, 16))')
+    p.add_argument('--rank-arguments', action='store_true',
+                   help='also rank every example\'s true arguments against all entities (MRR, mean rank, Hits@1/3/10)')
     p.add_argument('--device', type=int, default=0, help='CUDA device index')
     a = p.parse_args(argv)
-    summary = export(a.checkpoint, a.dataset, a.out, splits=a.split, tsv=a.tsv, k=a.k, device=a.device)
+    summary = export(a.checkpoint, a.dataset, a.out, splits=a.split, tsv=a.tsv, k=a.k, device=a.device,
+                     rank_arguments=a.rank_arguments)
     for name, s in summary['sets'].items():
         b3 = s.get('b3')
-        print('%s: %d rows, %d without features, %d clusters%s' % (name, s['rows'], s['rows_without_features'], s['clusters'],
-              '' if b3 is None else ', B3 f1 %.4f' % b3['f1']))
+        args = s.get('arguments', {}).get('both')
+        print('%s: %d rows, %d without features, %d clusters%s%s' % (name, s['rows'], s['rows_without_features'], s['clusters'],
+              '' if b3 is None else ', B3 f1 %.4f' % b3['f1'], '' if args is None else ', argument MRR %.4f' % args['mrr']))
     print('Wrote', os.path.join(a.out, 'summary.json'))
     return summary
 
