@@ -51,8 +51,10 @@ namespace rae {
 namespace {
 
 // optional in-kernel timeline (build with -DRAE_TRACE, never part of the shipped library): SM cycle counter of CTA-local
-// milestones, [CTA][64] slots; forward kernel slots 0.., dq 16.., dC 32.. (see profiles/trace_tc.py)
+// milestones, [CTA][TC_TRACE_STRIDE] slots; forward kernel slots 0.., dq 16.., dC 32.., recompute pass 64.. (the forward
+// kernel's slots + 64), dq segment / selectional-preference stamps 96.. (see profiles/trace_tc.py)
 #ifdef RAE_TRACE
+constexpr int TC_TRACE_STRIDE = 128;
 __device__ unsigned long long* g_tc_trace = nullptr;
 // knock-out switches of the MEASUREMENT build only (profiles/trace_tc.py): 1 = the producer arrives without copying after
 // the first fills, 2 = the MMA thread commits without issuing MMAs, 4 = the row-owning warps skip their arithmetic
@@ -62,7 +64,24 @@ __device__ int g_tc_knock = 0;
 #define TC_TRACE_INIT_IF(cond) unsigned long long* const tc_trace_ptr_ = (cond) ? g_tc_trace : nullptr
 #define TC_TRACE(slot)                                                                                         \
     do {                                                                                                       \
-        if (tc_trace_ptr_ != nullptr && (slot) < 64) tc_trace_ptr_[(size_t)blockIdx.x * 64 + (slot)] = clock64(); \
+        if (tc_trace_ptr_ != nullptr && (slot) < TC_TRACE_STRIDE) tc_trace_ptr_[(size_t)blockIdx.x * TC_TRACE_STRIDE + (slot)] = clock64(); \
+    } while (0)
+// a value instead of a clock (segment count, tile-end flag)
+#define TC_TRACE_VAL(slot, v)                                                                                  \
+    do {                                                                                                       \
+        if (tc_trace_ptr_ != nullptr) tc_trace_ptr_[(size_t)blockIdx.x * TC_TRACE_STRIDE + (slot)] = (unsigned long long)(v); \
+    } while (0)
+// the forward kernel's slot base: 0 for the forward pass, 64 for the recompute pass (the one without C1 / C2 rows)
+#define TC_TRACE_BASE(with_sp) const int tc_tb_ = (with_sp) ? 0 : 64
+// this CTA's segment count and whether one of its segments ends a tile (its range holds the tile's last unit)
+#define TC_TRACE_SEGS(sch, slot_n, slot_end)                                                                   \
+    do {                                                                                                       \
+        TcSegIter si_(sch, blockIdx.x);                                                                        \
+        TcSeg sg_;                                                                                             \
+        int n_ = 0, e_ = 0;                                                                                    \
+        while (si_.next(sg_)) { ++n_; e_ |= sg_.u1 == (sch).upt; }                                             \
+        TC_TRACE_VAL(slot_n, n_);                                                                              \
+        TC_TRACE_VAL(slot_end, e_);                                                                            \
     } while (0)
 // wall-clock stamp (ns, synchronised across SMs): kernel duration and the SM clock actually held under tensor load
 #define TC_TRACE_NS(slot)                                                                                      \
@@ -70,11 +89,14 @@ __device__ int g_tc_knock = 0;
         if (tc_trace_ptr_ != nullptr) {                                                                        \
             unsigned long long ns_;                                                                            \
             asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(ns_));                                            \
-            tc_trace_ptr_[(size_t)blockIdx.x * 64 + (slot)] = ns_;                                             \
+            tc_trace_ptr_[(size_t)blockIdx.x * TC_TRACE_STRIDE + (slot)] = ns_;                                \
         }                                                                                                      \
     } while (0)
 #else
 #define TC_KNOCK(bit) false
+#define TC_TRACE_VAL(slot, v) do { } while (0)
+#define TC_TRACE_BASE(with_sp) do { } while (0)
+#define TC_TRACE_SEGS(sch, slot_n, slot_end) do { } while (0)
 #define TC_TRACE_NS(slot) do { } while (0)
 #define TC_TRACE_INIT() do { } while (0)
 #define TC_TRACE_INIT_IF(cond) do { } while (0)
@@ -405,13 +427,39 @@ __global__ void __launch_bounds__(256) k_tc_prep_c(const float* __restrict__ C, 
 // blockIdx.y == 0: dC B operand, q transposed: [chunk of 32 examples][hi/lo][bq 0..7][krow 0..NK-1] = (q[32c+4bq+0..3][krow]),
 //                  nbc chunks (an even number: the kernels consume two per stage; examples >= B are zero)
 // blockIdx.y == 1: L = A[a1], R = A[a2] (A[a1] with the model-C quirk) -> ev, one warp per example
+// blockIdx.y == 2: P operand of the forward / recompute contraction (k_tc_bilinear): per 128-example tile
+//                  [hi/lo][kq 0..NK/8-1][row 0..127] x 16 B = the FP16 pairs of q[b][8 kq .. 8 kq + 7] scaled by 2^12, i.e. TMEM
+//                  columns 4 kq .. 4 kq + 3 of the row's P planes (one B-operand stage per tile, bulk-copied per segment)
+// blockIdx.y == 3: the two-tile dC kernel's operand (below)
 __global__ void __launch_bounds__(256) k_tc_prep_qt(const float* __restrict__ q, int B, int K, int NK, int nbc, float4* __restrict__ out,
                                                     const float* __restrict__ A, const int32_t* __restrict__ a1,
                                                     const int32_t* __restrict__ a2, int d, int dp, int quirk, float* __restrict__ ev,
-                                                    uint32_t* __restrict__ scal, uint4* __restrict__ out4) {
+                                                    uint32_t* __restrict__ scal, uint4* __restrict__ out4, uint4* __restrict__ pimg) {
     pdl_enter();
     if (blockIdx.x == 0 && blockIdx.y == 0 && threadIdx.x < 2) scal[TS_AMAX_L + threadIdx.x] = 0u;   // the transposes that follow accumulate
     if (blockIdx.y == 2) {
+        const int KQ8 = NK / 8;
+        const size_t totalp = (size_t)((B + TC_M - 1) / TC_M) * KQ8 * TC_M;
+        for (size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x; idx < totalp; idx += (size_t)gridDim.x * blockDim.x) {
+            const int r = (int)(idx % TC_M);
+            const int kq = (int)((idx / TC_M) % KQ8);
+            const size_t tile = idx / ((size_t)TC_M * KQ8);
+            const int b = (int)tile * TC_M + r;
+            uint32_t hi[4], lo[4];
+#pragma unroll
+            for (int u = 0; u < 4; ++u) {
+                const int k = 8 * kq + 2 * u;
+                const float x0 = (b < B && k < K) ? q[(size_t)b * K + k] * TC_QSCALE : 0.f;
+                const float x1 = (b < B && k + 1 < K) ? q[(size_t)b * K + k + 1] * TC_QSCALE : 0.f;
+                split_h2(x0, x1, hi[u], lo[u]);
+            }
+            uint4* base = pimg + tile * 2 * KQ8 * TC_M;
+            base[(size_t)kq * TC_M + r] = make_uint4(hi[0], hi[1], hi[2], hi[3]);
+            base[(size_t)(KQ8 + kq) * TC_M + r] = make_uint4(lo[0], lo[1], lo[2], lo[3]);
+        }
+        return;
+    }
+    if (blockIdx.y == 3) {
         // FP16 pair operand of the two-tile dC kernel: [stage of 64 examples][hi/lo][oct 0..7][krow 0..NK-1] x 16 B = examples
         // 64 st + 8 oct + 0..7 at relation krow, q scaled by 2^12
         const size_t total4 = (size_t)(nbc / 2) * 8 * NK;
@@ -476,8 +524,8 @@ __global__ void __launch_bounds__(256) k_tc_prep_qt(const float* __restrict__ q,
 // way; k_tc_combine transposes / sums them back into the row-major per-example vectors.  (Reading ev[b][...] directly
 // costs one L1 wavefront per lane, ~66 cycles per warp instruction: measured as 2/3 of the kernel's time.)
 struct TcArgs {
-    const float* qT;        // [K][B]  q transposed
     const float4* bop;      // B operand chunks
+    const uint8_t* pimg;    // P operand images, one B-operand stage per example tile (k_tc_prep_qt)
     const float* LT;        // [dp][B]  left vectors transposed  (L forward, a for the recompute pass)
     const float* RT;        // [dp][B]  right vectors transposed (R forward, c for the recompute pass)
     float* spT;             // [2][dp][B]        c1, c2 (the accumulator rows of the C1 / C2 half chunks), transposed
@@ -498,6 +546,7 @@ __global__ void __launch_bounds__(TC_FWD_THREADS, 1) k_tc_bilinear(TcArgs p) {
     extern __shared__ __align__(128) uint8_t smem_raw[];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     TC_TRACE_INIT();
+    TC_TRACE_BASE(p.n_sp_half > 0);
     const uint32_t KQ8 = (uint32_t)p.KH / 8u;               // 16-byte planes (8 relations each) per hi / lo half of a chunk
     const uint32_t B_BYTES = 2u * KQ8 * TC_N * 16u;
     const uint32_t KC = (uint32_t)p.KH / 2u;                // TMEM columns of one P plane (two fp16 per column)
@@ -510,7 +559,7 @@ __global__ void __launch_bounds__(TC_FWD_THREADS, 1) k_tc_bilinear(TcArgs p) {
     uint64_t* t_full = b_empty + 4;                         // [TC_TSTAGES]
     uint64_t* t_empty = t_full + TC_TSTAGES;                // [TC_TSTAGES] 8 epilogue-warp arrivals
     uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(t_empty + TC_TSTAGES);
-    if (threadIdx.x == 0) { TC_TRACE(0); TC_TRACE_NS(14); }
+    if (threadIdx.x == 0) { TC_TRACE(tc_tb_ + 0); TC_TRACE_NS(tc_tb_ + 14); TC_TRACE_SEGS(p.sch, tc_tb_ + 57, tc_tb_ + 62); }
 
     if (threadIdx.x == 0) {
         mbar_init(a_full, 8);
@@ -526,27 +575,29 @@ __global__ void __launch_bounds__(TC_FWD_THREADS, 1) k_tc_bilinear(TcArgs p) {
     __syncthreads();
     tc_fence_after();
     const uint32_t tmem_base = *tmem_slot;
-    if (threadIdx.x == 0) TC_TRACE(1);
+    if (threadIdx.x == 0) TC_TRACE(tc_tb_ + 1);
 
     if (warp >= TC_FWD_WORKERS) {
         asm volatile("setmaxnreg.dec.sync.aligned.u32 40;" ::: "memory");
     }
     if (warp == TC_FWD_WORKERS + 1) {
-        // ===== producer: the chunk sequence of all segments, one bulk copy per chunk =====
+        // ===== producer: per segment the P image of its tile, then its chunks; one bulk copy per ring stage =====
         if (lane == 0) {
             TcSegIter si(p.sch, blockIdx.x);
             TcSeg sg;
             int it = 0;
+            auto fill = [&](const uint8_t* src) {
+                const int s = it % nbs;
+                const uint32_t ph = (it / nbs) & 1;
+                mbar_wait(&b_empty[s], ph ^ 1);
+                if (TC_KNOCK(1) && it >= nbs) { mbar_arrive(&b_full[s]); ++it; return; }
+                mbar_expect_tx(&b_full[s], B_BYTES);
+                bulk_g2s_pieces(smB + (size_t)s * B_BYTES, src, B_BYTES, &b_full[s]);
+                ++it;
+            };
             while (si.next(sg)) {
-                for (int c = sg.u0; c < sg.u1; ++c, ++it) {
-                    const int s = it % nbs;
-                    const uint32_t ph = (it / nbs) & 1;
-                    mbar_wait(&b_empty[s], ph ^ 1);
-                    if (TC_KNOCK(1) && it >= nbs) { mbar_arrive(&b_full[s]); continue; }
-                    mbar_expect_tx(&b_full[s], B_BYTES);
-                    bulk_g2s_pieces(smB + (size_t)s * B_BYTES, reinterpret_cast<const uint8_t*>(p.bop) + (size_t)c * B_BYTES, B_BYTES,
-                                    &b_full[s]);
-                }
+                fill(p.pimg + (size_t)sg.tile * B_BYTES);
+                for (int c = sg.u0; c < sg.u1; ++c) fill(reinterpret_cast<const uint8_t*>(p.bop) + (size_t)c * B_BYTES);
             }
         }
     } else if (warp == TC_FWD_WORKERS) {
@@ -570,6 +621,9 @@ __global__ void __launch_bounds__(TC_FWD_THREADS, 1) k_tc_bilinear(TcArgs p) {
             while (si.next(sg)) {
                 mbar_wait(a_full, seg & 1);                 // this segment's P rows are in TMEM
                 tc_fence_after();
+                if (seg == 1) TC_TRACE(tc_tb_ + 59);
+                mbar_arrive(&b_empty[s]);                   // ... so the epilogue warps are done with its P image's stage
+                if (++s == nbs) { s = 0; sp ^= 1; }
                 for (int c = sg.u0; c < sg.u1; ++c, ++it) {
                     if (!ready) {
                         mbar_wait(&t_empty[ts], tp ^ 1);
@@ -577,8 +631,8 @@ __global__ void __launch_bounds__(TC_FWD_THREADS, 1) k_tc_bilinear(TcArgs p) {
                         tc_fence_after();
                     }
                     ready = false;
-                    if (it == 4) TC_TRACE(6);
-                    if (it == 12) TC_TRACE(10);
+                    if (it == 4) TC_TRACE(tc_tb_ + 6);
+                    if (it == 12) TC_TRACE(tc_tb_ + 10);
                     const uint32_t b_hi = smem_u32(smB + (size_t)s * B_BYTES);
                     const uint64_t h0 = make_desc(b_hi, TC_N * 16u, 128u);
                     const uint64_t l0 = make_desc(b_hi + KQ8 * TC_N * 16u, TC_N * 16u, 128u);
@@ -606,13 +660,14 @@ __global__ void __launch_bounds__(TC_FWD_THREADS, 1) k_tc_bilinear(TcArgs p) {
                     }
                     tc_commit(&b_empty[s]);      // the stage is reusable once these MMAs have read it
                     tc_commit(&t_full[ts]);      // accumulators complete
-                    if (it == 4) TC_TRACE(7);
-                    if (it == 12) TC_TRACE(11);
+                    if (it == 4) TC_TRACE(tc_tb_ + 7);
+                    if (it == 12) TC_TRACE(tc_tb_ + 11);
+                    if (seg == 1 && c == sg.u0) TC_TRACE(tc_tb_ + 60);
                     s = s1; sp = sp1; ts = ts1; tp = tp1;
                 }
                 ++seg;
             }
-            TC_TRACE(3);
+            TC_TRACE(tc_tb_ + 3);
         }
         __syncwarp();
     } else if (warp < TC_FWD_WORKERS) {
@@ -626,34 +681,37 @@ __global__ void __launch_bounds__(TC_FWD_THREADS, 1) k_tc_bilinear(TcArgs p) {
         const float inv = 1.f / (TC_QSCALE * pow2_scale(p.scal[TS_AMAX_C]));      // undoes the operand scales (a power of two)
         TcSegIter si(p.sch, blockIdx.x);
         TcSeg sg;
-        int it = 0;
+        int it = 0, seg = 0;
         while (si.next(sg)) {
             const int b = sg.tile * TC_M + row;
             const bool ok = b < p.B;
+            if (ew == 0 && lane == 0 && seg == 1) TC_TRACE(tc_tb_ + 58);
+            // R (c) rows first: their loads are in flight while the P operand is copied
+            float Rr[RW], Wr[RW];
+            const float* rp = p.RT + (ok ? b : 0);
+            // re-read per segment (opaque to the compiler): otherwise the 64 clamped offsets are hoisted out of the segment
+            // loop and spilled across it
+            int jlast;
+            asm volatile("mov.b32 %0, %1;" : "=r"(jlast) : "r"(p.dp - 1));
+#pragma unroll
+            for (int c = 0; c < RW; ++c) Rr[c] = ldg_stream(rp + (size_t)min(jbase + c, jlast) * p.B);
+            if (ew == 0 && lane == 0 && it == 0) TC_TRACE(tc_tb_ + 12);
             {
-                // q row (scaled by 2^12) -> FP16 hi / lo planes of the A operand in TMEM, two relations per column.  Group g
-                // converts relations [56 g, 56 g + 56): all of a thread's loads are issued before the first conversion (one
-                // memory latency).  Segments after the first: this warp has seen t_full of the previous segment's last
-                // chunk, so every MMA that read the old rows is done.
-                const int kb = 56 * g;
-                float qh[56];
-                if (ew == 0 && lane == 0 && it == 0) TC_TRACE(12);
-                {
-                    const float* qp = p.qT + (ok ? b : 0);
-                    const int klast = p.K - 1;
-#pragma unroll
-                    for (int i = 0; i < 56; ++i) qh[i] = ldg_stream(qp + (size_t)min(kb + i, klast) * p.B);     // clamped: always a valid address
-#pragma unroll
-                    for (int i = 0; i < 56; ++i) qh[i] = (ok && kb + i < p.K) ? qh[i] * TC_QSCALE : 0.f;
-                }
-                if (ew == 0 && lane == 0 && it == 0 && qh[0] != -1.f) TC_TRACE(13);
-                const uint32_t a_hi_col = lane_base + TC_FWD_ACOL + (uint32_t)(kb / 2), a_lo_col = a_hi_col + KC;
+                // the segment's P operand (q rows x 2^12 as FP16 hi / lo planes, two relations per column: k_tc_prep_qt's
+                // image of the tile, streamed into the operand ring ahead of the segment's chunks) -> TMEM.  Group g copies
+                // columns [28 g, 28 g + 28) of each plane.  Segments after the first: this warp has seen t_full of the
+                // previous segment's last chunk, so every MMA that read the old rows is done.
+                const int r = it + seg;                        // ring stages filled before this one: chunks and P images
+                mbar_wait(&b_full[r % nbs], (r / nbs) & 1);
+                if (ew == 0 && lane == 0 && it == 0) TC_TRACE(tc_tb_ + 13);
+                const uint4* img = reinterpret_cast<const uint4*>(smB + (size_t)(r % nbs) * B_BYTES) + row;
+                const uint32_t a_hi_col = lane_base + TC_FWD_ACOL + 28u * g, a_lo_col = a_hi_col + KC;
 #pragma unroll
                 for (int c4 = 0; c4 < 7; ++c4) {
-                    if ((uint32_t)(kb / 2 + 4 * c4) < KC) {
-                        uint32_t hi[4], lo[4];
-#pragma unroll
-                        for (int u = 0; u < 4; ++u) split_h2(qh[8 * c4 + 2 * u], qh[8 * c4 + 2 * u + 1], hi[u], lo[u]);
+                    const uint32_t kq = 7u * g + c4;
+                    if (kq < KQ8) {
+                        const uint4 h = img[kq * TC_M], l = img[(KQ8 + kq) * TC_M];
+                        const uint32_t hi[4] = {h.x, h.y, h.z, h.w}, lo[4] = {l.x, l.y, l.z, l.w};
                         tc_st4u(a_hi_col + 4u * c4, hi);
                         tc_st4u(a_lo_col + 4u * c4, lo);
                     }
@@ -662,21 +720,16 @@ __global__ void __launch_bounds__(TC_FWD_THREADS, 1) k_tc_bilinear(TcArgs p) {
                 tc_fence_before();
                 __syncwarp();
                 if (lane == 0) mbar_arrive(a_full);
-                if (ew == 0 && lane == 0 && it == 0) TC_TRACE(2);
+                if (ew == 0 && lane == 0 && it == 0) TC_TRACE(tc_tb_ + 2);
+                if (ew == 0 && lane == 0 && seg == 1) TC_TRACE(tc_tb_ + 63);
             }
-            float Rr[RW], Wr[RW];
-            {
-                const float* rp = p.RT + (ok ? b : 0);
-                const int jlast = p.dp - 1;
 #pragma unroll
-                for (int c = 0; c < RW; ++c) Rr[c] = ldg_stream(rp + (size_t)min(jbase + c, jlast) * p.B);
-#pragma unroll
-                for (int c = 0; c < RW; ++c) {
-                    if (!(ok && jbase + c < p.dp)) Rr[c] = 0.f;
-                    Wr[c] = 0.f;
-                }
+            for (int c = 0; c < RW; ++c) {
+                if (!(ok && jbase + c < p.dp)) Rr[c] = 0.f;
+                Wr[c] = 0.f;
             }
-            if (ew == 0 && lane == 0 && it == 0 && Rr[0] != -1.f) TC_TRACE(8);
+            if (ew == 0 && lane == 0 && it == 0 && Rr[0] != -1.f) TC_TRACE(tc_tb_ + 8);
+            if (ew == 0 && lane == 0 && seg == 1 && Rr[0] != -1.f) TC_TRACE(tc_tb_ + 61);
             for (int c = sg.u0; c < sg.u1; ++c, ++it) {
                 const int ts = it % TC_TSTAGES;
                 const uint32_t tph = (it / TC_TSTAGES) & 1;
@@ -692,10 +745,10 @@ __global__ void __launch_bounds__(TC_FWD_THREADS, 1) k_tc_bilinear(TcArgs p) {
                     if (DP == 32 && ok && i0 + 1 < p.d) L1 = p.LT[(size_t)(i0 + 1) * p.B + b];
                 }
                 const bool etr = ew == 0 && lane == 0 && it == 8;
-                if (etr) TC_TRACE(53);
+                if (etr) TC_TRACE(tc_tb_ + 53);
                 mbar_wait(&t_full[ts], tph);
                 tc_fence_after();
-                if (etr) TC_TRACE(54);
+                if (etr) TC_TRACE(tc_tb_ + 54);
                 if (!bil && !sp) {                             // padding half chunk: nothing to read
                     __syncwarp();
                     if (lane == 0) mbar_arrive(&t_empty[ts]);
@@ -712,7 +765,7 @@ __global__ void __launch_bounds__(TC_FWD_THREADS, 1) k_tc_bilinear(TcArgs p) {
                         tc_fence_before();
                         __syncwarp();
                         if (lane == 0) mbar_arrive(&t_empty[ts]);     // this group is done with the accumulator stage
-                        if (etr) TC_TRACE(55);
+                        if (etr) TC_TRACE(tc_tb_ + 55);
                     }
                     if (TC_KNOCK(4)) continue;
                     if (bil) {
@@ -747,7 +800,7 @@ __global__ void __launch_bounds__(TC_FWD_THREADS, 1) k_tc_bilinear(TcArgs p) {
                     }
                 }
                 if (DP >= 64 && bil && ok && i0 < p.d) p.vT[((size_t)g * p.dp + i0) * p.B + b] = inv * vsum;
-                if (etr) TC_TRACE(56);
+                if (etr) TC_TRACE(tc_tb_ + 56);
             }
             if (ok) {
                 float* wo = p.wT + ((size_t)sg.slot * 2 + g) * p.dp * p.B + b;
@@ -757,13 +810,14 @@ __global__ void __launch_bounds__(TC_FWD_THREADS, 1) k_tc_bilinear(TcArgs p) {
                     if (j < p.dp) wo[(size_t)j * p.B] = inv * Wr[c];
                 }
             }
-            if (ew == 0 && lane == 0 && it <= (sg.u1 - sg.u0)) TC_TRACE(9);     // first segment done
+            if (ew == 0 && lane == 0 && it <= (sg.u1 - sg.u0)) TC_TRACE(tc_tb_ + 9);     // first segment done
+            ++seg;
         }
-        if (ew == 0 && lane == 0) TC_TRACE(4);
+        if (ew == 0 && lane == 0) TC_TRACE(tc_tb_ + 4);
     }
     tc_fence_before();
     __syncthreads();
-    if (threadIdx.x == 0) { TC_TRACE(5); TC_TRACE_NS(15); }
+    if (threadIdx.x == 0) { TC_TRACE(tc_tb_ + 5); TC_TRACE_NS(tc_tb_ + 15); }
     if (warp == TC_FWD_WORKERS + 2) {
         tc_fence_after();
         asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
@@ -1075,7 +1129,7 @@ __global__ void __launch_bounds__(TC_BWD_THREADS, 1) k_tc_dq(TcDqArgs p) {
     const uint32_t ST_BYTES = 2u * 16u * (uint32_t)p.NK * 16u;
     uint8_t* smB = smem_raw;
     uint32_t tmem_base;
-    if (threadIdx.x == 0) { TC_TRACE(16); TC_TRACE_NS(30); }
+    if (threadIdx.x == 0) { TC_TRACE(16); TC_TRACE_NS(30); TC_TRACE_SEGS(p.sch, 96, 103); }
     const BwdBars br = bwd_setup(smem_raw, ST_BYTES, warp, tmem_base);
     if (threadIdx.x == 0) TC_TRACE(17);
 
@@ -1101,6 +1155,7 @@ __global__ void __launch_bounds__(TC_BWD_THREADS, 1) k_tc_dq(TcDqArgs p) {
                 if (seg > 0) {                                   // the previous segment's accumulator has been drained
                     mbar_wait(br.acc_empty, (seg - 1) & 1);
                     tc_fence_after();
+                    if (seg == 1) TC_TRACE(99);
                 }
                 dq_mma_segment(br, smB, ST_BYTES, p.NK, tmem_base, sg.u1 - sg.u0, it);
                 it += sg.u1 - sg.u0;
@@ -1134,6 +1189,8 @@ __global__ void __launch_bounds__(TC_BWD_THREADS, 1) k_tc_dq(TcDqArgs p) {
             const int b = sg.tile * TC_M + row;
             const bool ok = b < p.B;
             const float* scb = p.sc + (size_t)(ok ? b : 0) * SC_N;
+            [[maybe_unused]] const bool tr0 = gw == 0 && lane == 0;
+            if (tr0 && seg == 1) TC_TRACE(97);
             // register cache of the thread's 32 columns of R and Y2 (coalesced loads from the transposed copies)
             float X[32], Y[32];
             {
@@ -1150,6 +1207,7 @@ __global__ void __launch_bounds__(TC_BWD_THREADS, 1) k_tc_dq(TcDqArgs p) {
                     if (!(ok && j0 + u < p.dp)) { X[u] = 0.f; Y[u] = 0.f; }
             }
             if (gw == 0 && lane == 0 && it == 0 && X[0] != -1.f) TC_TRACE(29);
+            if (tr0 && seg == 1 && X[0] != -1.f) TC_TRACE(98);
             const int st0 = sg.u0, st1 = sg.u1, nst = st1 - st0;
             const int nbil = max(0, min(st1, n_bil_st) - st0);
             float ai_n = 0.f, li_n = 0.f;
@@ -1184,6 +1242,7 @@ __global__ void __launch_bounds__(TC_BWD_THREADS, 1) k_tc_dq(TcDqArgs p) {
                 bwd_publish(br, as, lane);
                 if (tr) TC_TRACE(26);
                 if (gw == 0 && lane == 0 && git == 0) TC_TRACE(18);
+                if (tr0 && seg == 1 && lt == 0) TC_TRACE(104);
             }
             // selectional-preference rows (at most two stages per tile): coalesced loads from the transposed copies
             for (; lt < nst; ++lt) {
@@ -1193,6 +1252,7 @@ __global__ void __launch_bounds__(TC_BWD_THREADS, 1) k_tc_dq(TcDqArgs p) {
                 const float* sx = which == 0 ? p.aT : p.cT;
                 const float* sy = which == 0 ? p.LT : p.RT;
                 const float s2 = (ok && which < 2) ? sG * (which == 0 ? scb[SC_G2] : scb[SC_G1]) : 0.f;
+                if (tr0 && lt == nbil) TC_TRACE(100);
                 mbar_wait(&br.a_empty[as], ((git / NAS) & 1) ^ 1);
                 tc_fence_after();
 #pragma unroll
@@ -1207,12 +1267,14 @@ __global__ void __launch_bounds__(TC_BWD_THREADS, 1) k_tc_dq(TcDqArgs p) {
                     dq_store16(lane_base, as, 16 * cg + 8 * h, g);
                 }
                 bwd_publish(br, as, lane);
+                if (tr0 && lt == nst - 1) TC_TRACE(101);
             }
             it += nst;
             if (gw < 4) {
                 // ===== epilogue: accumulator row -> dq partial of this segment's slot =====
                 mbar_wait(br.acc_full, seg & 1);
                 tc_fence_after();
+                if (tr0 && seg == 0) TC_TRACE(102);
                 float* o = p.dqT + (size_t)sg.slot * p.NK * p.B + (ok ? b : 0);
                 for (int c0 = 0; c0 < p.NK; c0 += 32) {
                     float t[32];
@@ -1964,13 +2026,13 @@ int tc_init(rae_engine* h) {
     cudaError_t e;
     const size_t vec = (size_t)h->dp * h->B * sizeof(float);
     if ((e = cudaMalloc((void**)&t.bop, (size_t)t.n_chunks_fwd * b_bytes)) != cudaSuccess ||
+        (e = cudaMalloc((void**)&t.pimg, (size_t)t.ntile * b_bytes)) != cudaSuccess ||
         (e = cudaMalloc((void**)&t.vT, 2 * vec)) != cudaSuccess ||
         (e = cudaMalloc((void**)&t.wT, 2 * t.slots_vw * vec)) != cudaSuccess ||
         (e = cudaMalloc((void**)&t.spT, 2 * vec)) != cudaSuccess ||
         (e = cudaMalloc((void**)&t.bop2, (size_t)n_st * st_bytes)) != cudaSuccess ||
         (e = cudaMalloc((void**)&t.dqT, (size_t)t.slots_dq * h->B * t.NK * sizeof(float))) != cudaSuccess ||
         (e = cudaMalloc((void**)&t.pop3, (size_t)t.n_bst * st_bytes)) != cudaSuccess ||
-        (e = cudaMalloc((void**)&t.qT, (size_t)t.KH * h->B * sizeof(float))) != cudaSuccess ||
         (e = cudaMalloc((void**)&t.aT, vec + 256)) != cudaSuccess || (e = cudaMalloc((void**)&t.LT, vec + 256)) != cudaSuccess ||
         (e = cudaMemset(t.aT, 0, vec + 256)) != cudaSuccess || (e = cudaMemset(t.LT, 0, vec + 256)) != cudaSuccess ||
         (e = cudaMalloc((void**)&t.pop4, (size_t)t.n_bst * 2 * 8 * t.NK * 16)) != cudaSuccess ||
@@ -2006,8 +2068,8 @@ int tc_init(rae_engine* h) {
 
 void tc_free(rae_engine* h) {
     TcState& t = h->tc;
-    cudaFree(t.bop); cudaFree(t.vT); cudaFree(t.wT); cudaFree(t.spT); cudaFree(t.bop2); cudaFree(t.dqT); cudaFree(t.pop3); cudaFree(t.scal); cudaFree(t.pop4); cudaFree(t.Rimg); cudaFree(t.Yimg); cudaFree(t.tile_slots);
-    cudaFree(t.qT); cudaFree(t.aT); cudaFree(t.LT); cudaFree(t.RT); cudaFree(t.cT); cudaFree(t.Y2T);
+    cudaFree(t.bop); cudaFree(t.pimg); cudaFree(t.vT); cudaFree(t.wT); cudaFree(t.spT); cudaFree(t.bop2); cudaFree(t.dqT); cudaFree(t.pop3); cudaFree(t.scal); cudaFree(t.pop4); cudaFree(t.Rimg); cudaFree(t.Yimg); cudaFree(t.tile_slots);
+    cudaFree(t.aT); cudaFree(t.LT); cudaFree(t.RT); cudaFree(t.cT); cudaFree(t.Y2T);
     t = TcState{};
 }
 
@@ -2029,7 +2091,7 @@ int tc_prepare_c(rae_engine* h, cudaStream_t st) {
 
 namespace {
 // img_slot >= 0: that slot is ALSO written as the stack of stage images the two-tile dC kernel fetches
-int tc_transpose_slots(rae_engine* h, int n, const int* slots, float* const* dst, const int* amax_word, bool with_q, int img_slot,
+int tc_transpose_slots(rae_engine* h, int n, const int* slots, float* const* dst, const int* amax_word, int img_slot,
                        float* img_dst, cudaStream_t st) {
     TcState& t = h->tc;
     TrJobs jobs{};
@@ -2038,10 +2100,6 @@ int tc_transpose_slots(rae_engine* h, int n, const int* slots, float* const* dst
     for (int i = 0; i < n; ++i) {
         jobs.j[nj++] = TrJob{h->ev + (size_t)slots[i] * h->dp, (size_t)E_NV * h->dp, h->d, h->dp, dst[i], t.scal + amax_word[i], 0};
         maxc = std::max(maxc, h->dp);
-    }
-    if (with_q) {
-        jobs.j[nj++] = TrJob{h->q, (size_t)h->K, h->K, h->K, t.qT, nullptr, 0};
-        maxc = std::max(maxc, h->K);
     }
     if (img_slot >= 0 && t.dc2) {
         jobs.j[nj++] = TrJob{h->ev + (size_t)img_slot * h->dp, (size_t)E_NV * h->dp, h->d, t.DP, img_dst, nullptr, 1};
@@ -2054,20 +2112,21 @@ int tc_transpose_slots(rae_engine* h, int n, const int* slots, float* const* dst
 }
 }  // namespace
 
-// q-dependent operand of the dC contraction (after the encoder) + L / R gather, then the transposed views qT, LT, RT
+// q-dependent operands of the dC and forward / recompute contractions (after the encoder) + L / R gather, then the
+// transposed views LT, RT
 int tc_prepare_p(rae_engine* h, const int32_t* a1, const int32_t* a2, cudaStream_t st) {
     TcState& t = h->tc;
     const int nbc = 2 * t.n_bst;
     const size_t total3 = (size_t)nbc * 8 * t.NK;
     const int blocks3 = (int)std::min<size_t>((total3 + 255) / 256, (size_t)h->num_sms * 8);
-    launch_pdl(k_tc_prep_qt, dim3(blocks3, t.dc2 ? 3 : 2), dim3(256), 0, st, h->q, h->B, h->K, t.NK, nbc, t.pop3, h->P[RAE_P_A], a1, a2, h->d, h->dp,
-                                                              h->quirk ? 1 : 0, h->ev, t.scal, reinterpret_cast<uint4*>(t.pop4));
+    launch_pdl(k_tc_prep_qt, dim3(blocks3, t.dc2 ? 4 : 3), dim3(256), 0, st, h->q, h->B, h->K, t.NK, nbc, t.pop3, h->P[RAE_P_A], a1, a2, h->d, h->dp,
+                                                              h->quirk ? 1 : 0, h->ev, t.scal, reinterpret_cast<uint4*>(t.pop4), t.pimg);
     h->launches++;
     RAE_CUDA(h, cudaGetLastError());
     const int slots[2] = {E_L, E_R};
     float* const dst[2] = {t.LT, t.RT};
     const int words[2] = {TS_AMAX_L, TS_AMAX_R};
-    return tc_transpose_slots(h, 2, slots, dst, words, true, E_R, t.Rimg, st);
+    return tc_transpose_slots(h, 2, slots, dst, words, E_R, t.Rimg, st);
 }
 
 // the q-dependent operand alone (only the dC contraction at the end of the step needs it: prepared off the critical path)
@@ -2077,7 +2136,7 @@ int tc_prepare_qt(rae_engine* h, cudaStream_t st) {
     const size_t total3 = (size_t)nbc * 8 * t.NK;
     const int blocks3 = (int)std::min<size_t>((total3 + 255) / 256, (size_t)h->num_sms * 8);
     launch_pdl(k_tc_prep_qt, dim3(blocks3, 1), dim3(256), 0, st, h->q, h->B, h->K, t.NK, nbc, t.pop3, h->P[RAE_P_A], nullptr, nullptr, h->d, h->dp,
-                                                   h->quirk ? 1 : 0, h->ev, t.scal, nullptr);
+                                                   h->quirk ? 1 : 0, h->ev, t.scal, nullptr, nullptr);
     h->launches++;
     RAE_CUDA(h, cudaGetLastError());
     return RAE_OK;
@@ -2088,7 +2147,7 @@ int tc_prepare_qt(rae_engine* h, cudaStream_t st) {
 int tc_contract(rae_engine* h, const float* LT_in, const float* RT_in, int slotV, int slotW, bool with_sp, cudaStream_t st) {
     TcState& t = h->tc;
     TcArgs p{};
-    p.qT = t.qT; p.bop = t.bop; p.LT = LT_in; p.RT = RT_in; p.spT = t.spT; p.vT = t.vT; p.wT = t.wT; p.scal = t.scal;
+    p.bop = t.bop; p.pimg = reinterpret_cast<const uint8_t*>(t.pimg); p.LT = LT_in; p.RT = RT_in; p.spT = t.spT; p.vT = t.vT; p.wT = t.wT; p.scal = t.scal;
     p.B = h->B; p.K = h->K; p.d = h->d; p.dp = h->dp; p.KH = t.KH;
     p.n_bil_half = t.n_bil_half; p.n_sp_half = with_sp ? t.n_sp_half : 0;
     p.nbs = t.fwd_stages;
@@ -2114,7 +2173,7 @@ int tc_backward_recompute(rae_engine* h, cudaStream_t st) {
     const int slots[3] = {E_A, E_CV, E_Y2};
     float* const dst[3] = {t.aT, t.cT, t.Y2T};
     const int words[3] = {TS_AMAX_A, TS_AMAX_CV, TS_AMAX_Y2};
-    int rc = tc_transpose_slots(h, 3, slots, dst, words, false, E_Y2, t.Yimg, st);
+    int rc = tc_transpose_slots(h, 3, slots, dst, words, E_Y2, t.Yimg, st);
     if (rc) return rc;
     return tc_contract(h, t.aT, t.cT, E_GA1, E_GA2, false, st);
 }

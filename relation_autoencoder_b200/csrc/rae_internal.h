@@ -95,6 +95,7 @@ struct TcState {
     TcSched sch_fwd{}, sch_rec{}, sch_dq{}, sch_dc{}, sch_dc2{};
     int slots_vw = 0, slots_dq = 0, slots_dc = 0;   // partial-result slots per tile (maximum over tiles)
     float4* bop = nullptr; // forward B operand chunks [chunk][hi/lo][KQ][128]
+    uint4* pimg = nullptr; // forward / recompute P operand images [tile][hi/lo][KQ][128] (q x 2^12 as FP16 pairs)
     float* vT = nullptr;   // [2][dp][B]            v partials, transposed (lane = example)
     float* wT = nullptr;   // [slots_vw][2][dp][B]  w partials, transposed
     float* spT = nullptr;  // [2][dp][B]            c1, c2, transposed
@@ -107,7 +108,6 @@ struct TcState {
     float4* pop4 = nullptr; float* Rimg = nullptr; float* Yimg = nullptr;     // its q^T operand and the stage images of R, Y2
     int32_t* tile_slots = nullptr;   // [n_ntiles] partial slots of every 128-row tile of dC (device; k_dense_finalize)
     float4* pop3 = nullptr; // q^T chunks [bc][hi/lo][8][NK]
-    float* qT = nullptr;    // [4 KQ][B]  q transposed
     float* aT = nullptr; float* LT = nullptr; float* RT = nullptr; float* cT = nullptr; float* Y2T = nullptr;   // [dp][B] views
 };
 
