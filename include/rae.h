@@ -310,6 +310,23 @@ int rae_label_topk(rae_engine* h, const void* const* w_shards, int32_t world, co
  * workspace of about 512 * N * ceil16(d) bytes for the scaled FP16 image of A plus the query images of up to 131072 rows. */
 int rae_rank_arguments(rae_engine* h, const int32_t* indptr, const int32_t* indices, const int32_t* args1,
                        const int32_t* args2, int64_t n_rows, int32_t* rank1, int32_t* rank2, void* stream);
+/* Argument prediction: the k most likely entities of each argument slot of every row, with the candidate scores s1 / s2 of
+ * rae_rank_arguments (the fp32 value that call compares with its threshold).  ids1 / ids2 int32 [n_rows, k] and
+ * scores1 / scores2 float [n_rows, k] (device, row-major): per row and slot the k entities of [0, N) with the highest
+ * score, score descending, equal scores by ascending entity id.  The true argument is not excluded: its position in the
+ * list, if any, shows where it landed.  The scores are the x-dependent part of the decoder's negative-sample score, so
+ * they order a row's candidates exactly but are not comparable across rows.
+ * A slot's list never reads the argument it predicts: slot 1 depends on the posterior and A[args2] only, slot 2 on the
+ * posterior and A[args1] only (model C: on the posterior only), bit for bit, so a caller may pass any valid id (e.g. 0)
+ * for an argument that is unknown and predict it.  The lists do not depend on how the candidates are split over the SMs.
+ * CSR, n_rows, stream, scratch and ordering conventions as rae_rank_arguments; 1 <= k <= min(N, RAE_MAX_TOPK).
+ * Unbound parameters, an emit-only handle, null pointers, n_rows < 0 or k out of range are refused before any launch;
+ * n_rows = 0 launches nothing.  Workspace: that of rae_rank_arguments plus the partial top-kt lists (kt = k rounded up
+ * to a power of two), 2 x kt x 8 bytes per query and candidate range: at most about 67 MB (2 x 131072 queries x 2 x
+ * 16 x 8 B) on top of what ranking allocates. */
+int rae_predict_arguments(rae_engine* h, const int32_t* indptr, const int32_t* indices, const int32_t* args1,
+                          const int32_t* args2, int64_t n_rows, int32_t k, int32_t* ids1, float* scores1, int32_t* ids2,
+                          float* scores2, void* stream);
 
 /* ---- negative sampling on the device (replaces NegativeExampleGenerator.get_negative_samples, NegativeExampleGenerator.py:14-32)
  * out[i] = searchsorted(cum, uniform(0, cum_last)) for i in [0, n), bit-exact with the reference's host recipe on a legacy

@@ -105,6 +105,7 @@ _SIGNATURES = {
     "rae_label_shards": (C.c_int, [_P, _P, C.c_int32, _P, _P, C.c_int64, _P, _P, _P]),
     "rae_label_topk": (C.c_int, [_P, _P, C.c_int32, _P, _P, C.c_int64, C.c_int32, _P, _P, _P]),
     "rae_rank_arguments": (C.c_int, [_P, _P, _P, _P, _P, C.c_int64, _P, _P, _P]),
+    "rae_predict_arguments": (C.c_int, [_P, _P, _P, _P, _P, C.c_int64, C.c_int32, _P, _P, _P, _P, _P]),
     "rae_sample_negatives": (C.c_int, [_P, _P, _P, C.c_int64, C.c_double, _P, C.c_int64, _P, _P]),
     "rae_set_profiling": (C.c_int, [_P, C.c_int32]),
     "rae_get_phase_times": (C.c_int, [_P, C.POINTER(C.c_float)]),

@@ -2368,12 +2368,67 @@ struct RankArgs {
     int NC, DH, nbs;
     int Rpad, nr;               // queries of slot s at [s Rpad, s Rpad + nr)
     int n_tiles, splits;        // work item = (query tile, candidate range); item = tile * splits + split
+    float* ps; int32_t* pi;     // TopK: partial lists, [item][group][KT][128 rows] scores / ids
+};
+
+// Epilogue policies of the ranking GEMM.  step() sees 32 consecutive candidate columns [col0, col0 + 32) of one query
+// row: t the raw accumulators, a the biases; the score is fmaf(t, inv, a).  finish() runs once per work item.
+struct RankCount {               // rank: count the candidates above the true argument's threshold (no score is stored)
+    int cnt = 0;
+    __device__ __forceinline__ void step(const float (&t)[32], const float (&a)[32], float inv, float thr, int tru, int col0) {
+        const int tcol = tru - col0;   // the true entity's column in these 32, if any
+        if (__any_sync(kFull, (unsigned)tcol < 32u)) {
+#pragma unroll
+            for (int x = 0; x < 32; ++x) cnt += (fmaf(t[x], inv, a[x]) > thr && x != tcol) ? 1 : 0;
+        } else {
+#pragma unroll
+            for (int x = 0; x < 32; ++x) cnt += fmaf(t[x], inv, a[x]) > thr ? 1 : 0;
+        }
+    }
+    __device__ __forceinline__ void finish(const RankArgs& p, bool valid, int slot, int r, int g, int, int split, int) {
+        if (valid) atomicAdd((slot ? p.out2 : p.out1) + r, cnt + ((g == 0 && split == 0) ? 1 : 0));
+    }
+};
+
+// predict: keep the KT best (score, id) of the row's candidates, score descending then id ascending, sorted in registers.
+// A thread sees its ids in ascending order, so the strict > keeps the lower id on equal scores.  The -inf padding rows
+// never enter (k <= N real candidates exist, the merge drops the -inf / INT_MAX fillers).
+template <int KT>
+struct RankTopK {
+    float s[KT];
+    int id[KT];
+    __device__ __forceinline__ RankTopK() {
+#pragma unroll
+        for (int j = 0; j < KT; ++j) { s[j] = -INFINITY; id[j] = 0x7fffffff; }
+    }
+    __device__ __forceinline__ void step(const float (&t)[32], const float (&a)[32], float inv, float, int, int col0) {
+#pragma unroll
+        for (int x = 0; x < 32; ++x) {
+            const float v = fmaf(t[x], inv, a[x]);
+            if (v > s[KT - 1]) {
+#pragma unroll
+                for (int j = KT - 1; j > 0; --j) {
+                    const bool up = v > s[j - 1];
+                    const bool here = !up && v > s[j];
+                    s[j] = up ? s[j - 1] : (here ? v : s[j]);
+                    id[j] = up ? id[j - 1] : (here ? col0 + x : id[j]);
+                }
+                if (v > s[0]) { s[0] = v; id[0] = col0 + x; }
+            }
+        }
+    }
+    __device__ __forceinline__ void finish(const RankArgs& p, bool, int, int, int g, int item, int, int row) {
+        const size_t base = ((size_t)item * 2 + g) * KT * 128 + row;
+#pragma unroll
+        for (int j = 0; j < KT; ++j) { p.ps[base + (size_t)j * 128] = s[j]; p.pi[base + (size_t)j * 128] = id[j]; }
+    }
 };
 
 // Persistent: CTA x takes items x, x + G, ...  When the query tiles outnumber the SMs every CTA sweeps ALL candidate
 // chunks in the same order at the same rate, so the CTAs resident together read each chunk from L2 (A is read from HBM
 // about once per wave instead of once per query tile).  With fewer tiles than SMs the candidates are split into ranges.
-__global__ void __launch_bounds__(RK_THREADS, 1) k_tc_rank(RankArgs p) {
+template <class Epi>
+__device__ __forceinline__ void tc_rank_body(const RankArgs& p) {
     pdl_enter();
     extern __shared__ __align__(128) uint8_t smem_raw[];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -2497,7 +2552,7 @@ __global__ void __launch_bounds__(RK_THREADS, 1) k_tc_rank(RankArgs p) {
             const float thr = valid ? p.qthr[qi] : INFINITY;     // padding rows count nothing
             const float inv = valid ? p.qinv[qi] : 0.f;
             const int tru = valid ? p.qtrue[qi] : -1;
-            int cnt = 0;
+            Epi epi;
             for (int c = c0; c < c1; ++c, ++it) {
                 const int s = it % nbs, ts = it & 1;
                 mbar_wait(&t_full[ts], (it >> 1) & 1);
@@ -2519,19 +2574,12 @@ __global__ void __launch_bounds__(RK_THREADS, 1) k_tc_rank(RankArgs p) {
                         const float4 v = *reinterpret_cast<const float4*>(ab + 32 * hf + x);
                         a[x] = v.x; a[x + 1] = v.y; a[x + 2] = v.z; a[x + 3] = v.w;
                     }
-                    const int tcol = tru - (c * 128 + 64 * g + 32 * hf);   // the true entity's column in these 32, if any
-                    if (__any_sync(kFull, (unsigned)tcol < 32u)) {
-#pragma unroll
-                        for (int x = 0; x < 32; ++x) cnt += (fmaf(t[x], inv, a[x]) > thr && x != tcol) ? 1 : 0;
-                    } else {
-#pragma unroll
-                        for (int x = 0; x < 32; ++x) cnt += fmaf(t[x], inv, a[x]) > thr ? 1 : 0;
-                    }
+                    epi.step(t, a, inv, thr, tru, c * 128 + 64 * g + 32 * hf);
                 }
                 __syncwarp();
                 if (lane == 0) mbar_arrive(&b_empty[s]);
             }
-            if (valid) atomicAdd((slot ? p.out2 : p.out1) + r, cnt + ((g == 0 && split == 0) ? 1 : 0));
+            epi.finish(p, valid, slot, r, g, item, split, row);
         }
     }
     tc_fence_before();
@@ -2541,18 +2589,106 @@ __global__ void __launch_bounds__(RK_THREADS, 1) k_tc_rank(RankArgs p) {
         asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
     }
 }
-}  // namespace
 
-int launch_rank_arguments(rae_engine* h, const int32_t* indptr, const int32_t* indices, const int32_t* a1, const int32_t* a2,
-                          int64_t n_rows, int32_t* rank1, int32_t* rank2, cudaStream_t st) {
+__global__ void __launch_bounds__(RK_THREADS, 1) k_tc_rank(RankArgs p) { tc_rank_body<RankCount>(p); }
+
+template <int KT>
+__global__ void __launch_bounds__(RK_THREADS, 1) k_tc_predict(RankArgs p) { tc_rank_body<RankTopK<KT>>(p); }
+
+// the 2 * splits partial lists of a query -> its first k entries under (score descending, id ascending).  One warp per
+// query: each lane keeps the best KT of the entries lane, lane + 32, ..., then k rounds of a butterfly arg-best over the
+// lanes' heads, the owning lane popping its head.  Ids are unique, so the result does not depend on how the candidates
+// were split; no floating-point arithmetic is done.
+struct PredictMergeArgs {
+    const float* ps; const int32_t* pi;
+    int32_t* ids1; float* sc1; int32_t* ids2; float* sc2;   // [nr, k] of the pass's first example
+    int nr, Rpad, splits, k;
+};
+__device__ __forceinline__ bool pred_before(float v, int x, float w, int y) { return v > w || (v == w && x < y); }
+
+template <int KT>
+__global__ void __launch_bounds__(256) k_predict_merge(PredictMergeArgs p) {
+    pdl_enter();
+    const int lane = threadIdx.x & 31;
+    const int gw = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    if (gw >= 2 * p.nr) return;
+    const int slot = gw >= p.nr ? 1 : 0, r = gw - slot * p.nr;
+    const int qi = slot * p.Rpad + r, tile = qi >> 7, row = qi & 127;
+    float s[KT];
+    int id[KT];
+#pragma unroll
+    for (int j = 0; j < KT; ++j) { s[j] = -INFINITY; id[j] = 0x7fffffff; }
+    const int n = 2 * p.splits * KT;
+    const size_t base = (size_t)tile * p.splits * 2 * KT * 128 + row;   // lists (split, group) of the tile's items
+    for (int e = lane; e < n; e += 32) {
+        const float v = p.ps[base + (size_t)e * 128];
+        const int x = p.pi[base + (size_t)e * 128];
+        if (pred_before(v, x, s[KT - 1], id[KT - 1])) {
+#pragma unroll
+            for (int j = KT - 1; j > 0; --j) {
+                const bool up = pred_before(v, x, s[j - 1], id[j - 1]);
+                const bool here = !up && pred_before(v, x, s[j], id[j]);
+                s[j] = up ? s[j - 1] : (here ? v : s[j]);
+                id[j] = up ? id[j - 1] : (here ? x : id[j]);
+            }
+            if (pred_before(v, x, s[0], id[0])) { s[0] = v; id[0] = x; }
+        }
+    }
+    int32_t* ids = (slot ? p.ids2 : p.ids1) + (size_t)r * p.k;
+    float* sc = (slot ? p.sc2 : p.sc1) + (size_t)r * p.k;
+    for (int j = 0; j < p.k; ++j) {
+        float bv = s[0];
+        int bi = id[0];
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {
+            const float ov = __shfl_xor_sync(kFull, bv, o);
+            const int oi = __shfl_xor_sync(kFull, bi, o);
+            if (pred_before(ov, oi, bv, bi)) { bv = ov; bi = oi; }
+        }
+        if (id[0] == bi) {
+#pragma unroll
+            for (int u = 0; u < KT - 1; ++u) { s[u] = s[u + 1]; id[u] = id[u + 1]; }
+            s[KT - 1] = -INFINITY;
+            id[KT - 1] = 0x7fffffff;
+        }
+        if (lane == 0) { ids[j] = bi; sc[j] = bv; }
+    }
+}
+
+// what one call of the driver produces: kt = 0 counts ranks into rank1 / rank2; kt in {1, 2, 4, 8, 16} keeps the best
+// kt candidates per query and writes the first k of them to ids / scores
+struct RankOutputs {
+    int32_t* rank1; int32_t* rank2;
+    int kt, k;
+    int32_t* ids1; float* sc1; int32_t* ids2; float* sc2;
+};
+
+template <int KT>
+void predict_kernels(void (*&kern)(RankArgs), void (*&merge)(PredictMergeArgs)) { kern = k_tc_predict<KT>; merge = k_predict_merge<KT>; }
+
+// A image, forward pass in chunks of B rows (the tail chunk padded), query packing, one tcgen05 launch per pass of up to
+// RK_PASS_ROWS rows with the epilogue `o` selects (plus the merge of the partial lists for top-k)
+int launch_rank_driver(rae_engine* h, const char* what, const int32_t* indptr, const int32_t* indices, const int32_t* a1,
+                       const int32_t* a2, int64_t n_rows, const RankOutputs& o, cudaStream_t st) {
     if (n_rows == 0) return RAE_OK;
     const int B = h->B, d = h->d, DH = (d + 15) & ~15;
     const int64_t N = h->cfg.N;
-    if (N > ((int64_t)1 << 31) - 256) return fail(h, RAE_EINVAL, "rae_rank_arguments: N = %lld entities are too many", (long long)N);
+    if (N > ((int64_t)1 << 31) - 256) return fail(h, RAE_EINVAL, "%s: N = %lld entities are too many", what, (long long)N);
+    void (*kern)(RankArgs) = k_tc_rank;
+    void (*merge)(PredictMergeArgs) = nullptr;
+    switch (o.kt) {
+        case 0: break;
+        case 1: predict_kernels<1>(kern, merge); break;
+        case 2: predict_kernels<2>(kern, merge); break;
+        case 4: predict_kernels<4>(kern, merge); break;
+        case 8: predict_kernels<8>(kern, merge); break;
+        case 16: predict_kernels<16>(kern, merge); break;
+        default: return fail(h, RAE_EINVAL, "%s: no top-%d epilogue", what, o.kt);
+    }
     const int NC = (int)((N + 127) / 128);
     const size_t CB = rank_chunk_bytes(DH);
     const int nbs = (int)std::min<size_t>(RK_MAX_STAGES, ((size_t)h->max_smem_optin - 256) / CB);
-    if (nbs < 1) return fail(h, RAE_EINVAL, "rae_rank_arguments: d = %d needs %zu bytes per candidate stage", d, CB);
+    if (nbs < 1) return fail(h, RAE_EINVAL, "%s: d = %d needs %zu bytes per candidate stage", what, d, CB);
     // more than half the shared memory: one CTA per SM, so no CTA waits in tcgen05.alloc for another's 512 columns
     const size_t smem = std::max<size_t>((size_t)nbs * CB + 256, (size_t)h->max_smem_optin / 2 + 1024);
     const int64_t cpp = std::max<int64_t>(1, RK_PASS_ROWS / B);              // forward chunks of B rows per ranking pass
@@ -2561,10 +2697,13 @@ int launch_rank_arguments(rae_engine* h, const int32_t* indptr, const int32_t* i
     auto al = [](size_t x) { return (x + 255) & ~(size_t)255; };
     const size_t b_img = al((size_t)NC * CB), b_q = al((size_t)2 * Rmax * DH * 4), b_m = al((size_t)2 * Rmax * 4),
                  b_pad = al((size_t)(B + 1) * 4), b_a = al((size_t)B * 4);
-    const size_t total = 256 + b_img + b_q + 3 * b_m + b_pad + 2 * b_a;
+    // top-k partial lists: one per (item, group); items <= max(query tiles, SMs) since splits <= num_sms / n_tiles
+    const int64_t max_items = std::max<int64_t>(2 * Rmax / 128, h->num_sms);
+    const size_t b_part = o.kt ? al((size_t)max_items * 2 * o.kt * 128 * 4) : 0;
+    const size_t total = 256 + b_img + b_q + 3 * b_m + b_pad + 2 * b_a + 2 * b_part;
     uint8_t* ws = nullptr;
     cudaError_t e = cudaMallocAsync((void**)&ws, total, st);
-    if (e != cudaSuccess) return fail(h, RAE_ENOMEM, "rae_rank_arguments: %zu bytes of workspace: %s", total, cudaGetErrorString(e));
+    if (e != cudaSuccess) return fail(h, RAE_ENOMEM, "%s: %zu bytes of workspace: %s", what, total, cudaGetErrorString(e));
     uint32_t* amax = reinterpret_cast<uint32_t*>(ws);
     uint8_t* cur = ws + 256;
     auto take = [&](size_t b) { uint8_t* r = cur; cur += b; return r; };
@@ -2576,10 +2715,14 @@ int launch_rank_arguments(rae_engine* h, const int32_t* indptr, const int32_t* i
     int32_t* pad_ip = reinterpret_cast<int32_t*>(take(b_pad));
     int32_t* pad_a1 = reinterpret_cast<int32_t*>(take(b_a));
     int32_t* pad_a2 = reinterpret_cast<int32_t*>(take(b_a));
+    float* ps = reinterpret_cast<float*>(take(b_part));
+    int32_t* pi = reinterpret_cast<int32_t*>(take(b_part));
     auto body = [&]() -> int {
         int rc;
-        RAE_CUDA(h, cudaMemsetAsync(rank1, 0, sizeof(int32_t) * (size_t)n_rows, st));
-        RAE_CUDA(h, cudaMemsetAsync(rank2, 0, sizeof(int32_t) * (size_t)n_rows, st));
+        if (!o.kt) {
+            RAE_CUDA(h, cudaMemsetAsync(o.rank1, 0, sizeof(int32_t) * (size_t)n_rows, st));
+            RAE_CUDA(h, cudaMemsetAsync(o.rank2, 0, sizeof(int32_t) * (size_t)n_rows, st));
+        }
         RAE_CUDA(h, cudaMemsetAsync(amax, 0, sizeof(uint32_t), st));
         launch_pdl(k_tc_absmax, dim3(h->num_sms * 8), dim3(256), 0, st, (const float*)h->P[RAE_P_A], (size_t)N * d, (const float*)nullptr,
                    (size_t)0, (const float*)nullptr, (size_t)0, amax);
@@ -2592,7 +2735,7 @@ int launch_rank_arguments(rae_engine* h, const int32_t* indptr, const int32_t* i
         h->launches += 2;
         RAE_CUDA(h, cudaGetLastError());
         if (h->use_tc && (rc = tc_prepare_c(h, st))) return rc;
-        RAE_CUDA(h, cudaFuncSetAttribute(k_tc_rank, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        RAE_CUDA(h, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         for (int64_t row0 = 0; row0 < n_rows; row0 += pass_rows) {
             const int nr = (int)std::min<int64_t>(pass_rows, n_rows - row0);
             const int Rpad = (nr + 127) / 128 * 128;
@@ -2625,21 +2768,53 @@ int launch_rank_arguments(rae_engine* h, const int32_t* indptr, const int32_t* i
             }
             RankArgs p{};
             p.aimg = aimg; p.qimg = qimg; p.qinv = qinv; p.qthr = qthr; p.qtrue = qtrue;
-            p.out1 = rank1 + row0; p.out2 = rank2 + row0;
+            if (!o.kt) { p.out1 = o.rank1 + row0; p.out2 = o.rank2 + row0; }
+            p.ps = ps; p.pi = pi;
             p.NC = NC; p.DH = DH; p.nbs = nbs; p.Rpad = Rpad; p.nr = nr;
             p.n_tiles = 2 * Rpad / 128;
             // fewer query tiles than SMs: split the candidates, at least 8 chunks per range
             p.splits = (int)std::max<int64_t>(1, std::min<int64_t>(h->num_sms / p.n_tiles, NC / 8));
             const int G = std::min(h->num_sms, p.n_tiles * p.splits);
-            launch_pdl(k_tc_rank, dim3(G), dim3(RK_THREADS), smem, st, p);
+            launch_pdl(kern, dim3(G), dim3(RK_THREADS), smem, st, p);
             h->launches++;
             RAE_CUDA(h, cudaGetLastError());
+            if (merge) {
+                PredictMergeArgs m{};
+                m.ps = ps; m.pi = pi;
+                const size_t at = (size_t)row0 * o.k;
+                m.ids1 = o.ids1 + at; m.sc1 = o.sc1 + at; m.ids2 = o.ids2 + at; m.sc2 = o.sc2 + at;
+                m.nr = nr; m.Rpad = Rpad; m.splits = p.splits; m.k = o.k;
+                launch_pdl(merge, dim3((2 * nr + 7) / 8), dim3(256), 0, st, m);
+                h->launches++;
+                RAE_CUDA(h, cudaGetLastError());
+            }
         }
         return RAE_OK;
     };
     const int rc = body();
     cudaFreeAsync(ws, st);
     return rc;
+}
+}  // namespace
+
+int launch_rank_arguments(rae_engine* h, const int32_t* indptr, const int32_t* indices, const int32_t* a1, const int32_t* a2,
+                          int64_t n_rows, int32_t* rank1, int32_t* rank2, cudaStream_t st) {
+    RankOutputs o{};
+    o.rank1 = rank1; o.rank2 = rank2;
+    return launch_rank_driver(h, "rae_rank_arguments", indptr, indices, a1, a2, n_rows, o, st);
+}
+
+int launch_predict_arguments(rae_engine* h, const int32_t* indptr, const int32_t* indices, const int32_t* a1, const int32_t* a2,
+                             int64_t n_rows, int k, int32_t* ids1, float* scores1, int32_t* ids2, float* scores2,
+                             cudaStream_t st) {
+    if (k < 1 || k > RAE_MAX_TOPK || k > h->cfg.N)
+        return fail(h, RAE_EINVAL, "rae_predict_arguments: k = %d outside [1, min(N = %lld, %d)]", k, (long long)h->cfg.N,
+                    RAE_MAX_TOPK);
+    RankOutputs o{};
+    o.kt = 1;
+    while (o.kt < k) o.kt *= 2;              // the first k of a top-kt list are the top-k list
+    o.k = k; o.ids1 = ids1; o.sc1 = scores1; o.ids2 = ids2; o.sc2 = scores2;
+    return launch_rank_driver(h, "rae_predict_arguments", indptr, indices, a1, a2, n_rows, o, st);
 }
 
 }  // namespace rae

@@ -787,6 +787,19 @@ int rae_rank_arguments(rae_engine* h, const int32_t* indptr, const int32_t* indi
     return launch_rank_arguments(h, indptr, indices, args1, args2, n_rows, rank1, rank2, (cudaStream_t)stream);
 }
 
+int rae_predict_arguments(rae_engine* h, const int32_t* indptr, const int32_t* indices, const int32_t* args1,
+                          const int32_t* args2, int64_t n_rows, int32_t k, int32_t* ids1, float* scores1, int32_t* ids2,
+                          float* scores2, void* stream) {
+    if (!h) return RAE_EINVAL;
+    if (!h->params_bound) return fail(h, RAE_ENOTBOUND, "parameters are not bound (rae_bind_params)");
+    if (h->emit_only) return fail(h, RAE_EINVAL, "rae_predict_arguments: an emit-only handle holds compact copies of A, not the model's");
+    if (!indptr || !indices || !args1 || !args2 || !ids1 || !scores1 || !ids2 || !scores2 || n_rows < 0)
+        return fail(h, RAE_EINVAL, "rae_predict_arguments: bad argument");
+    h->launches = 0;
+    return launch_predict_arguments(h, indptr, indices, args1, args2, n_rows, k, ids1, scores1, ids2, scores2,
+                                    (cudaStream_t)stream);
+}
+
 int rae_train_step_end(rae_engine* h, void* stream) {
     int rc = check_ready(h, false, false);
     if (rc) return rc;

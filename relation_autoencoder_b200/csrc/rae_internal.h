@@ -244,6 +244,10 @@ int tc_grad_dense(rae_engine* h, cudaStream_t st);
 // rae_rank_arguments: forward in chunks of B rows, query packing, one tcgen05 ranking launch per pass (rae_decoder_tc.cu)
 int launch_rank_arguments(rae_engine* h, const int32_t* indptr, const int32_t* indices, const int32_t* a1, const int32_t* a2,
                           int64_t n_rows, int32_t* rank1, int32_t* rank2, cudaStream_t st);
+// rae_predict_arguments: the same driver with the top-k epilogue and a merge of the partial lists (rae_decoder_tc.cu)
+int launch_predict_arguments(rae_engine* h, const int32_t* indptr, const int32_t* indices, const int32_t* a1, const int32_t* a2,
+                             int64_t n_rows, int k, int32_t* ids1, float* scores1, int32_t* ids2, float* scores2,
+                             cudaStream_t st);
 
 // ---- sort / segment / updates (rae_update.cu) ----
 size_t segwork_temp_bytes(int64_t n);

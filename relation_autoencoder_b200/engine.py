@@ -231,44 +231,68 @@ class Engine:
         ids = ids[:n * k].reshape(n, k).cpu().numpy()
         return ids, (q[:n * k].reshape(n, k).cpu().numpy() if q is not None else None)
 
-    def rank_arguments(self, indptr, indices, args1, args2):
-        """Entity ranks of every row's true arguments under the bound model, from one ``rae_rank_arguments`` call ->
-        (rank1 int32 [n], rank2 int32 [n]).  rank_s = 1 + the number of other entities whose candidate score in slot s
-        (the decoder's negative-sample score with that argument replaced) exceeds the true one's.  Host or device int32
-        CSR and argument ids of any length; entity ids must lie in [0, N) and feature ids in [0, F).  The call reuses the
-        handle's per-batch scratch, so ``last_probs`` afterwards no longer shows the last training step."""
+    def _argument_inputs(self, what, indptr, indices, args1, args2):
+        """Host checks shared by rank_arguments / predict_arguments -> (n, indptr, indices, args1, args2) on the device
+        (non-null arrays for n == 0 and for rows without features)."""
         if not self.params:
-            raise RuntimeError("rank_arguments needs bound parameters (bind_params / set_params_numpy)")
+            raise RuntimeError("%s needs bound parameters (bind_params / set_params_numpy)" % what)
         ip_h = np.asarray(indptr.cpu() if isinstance(indptr, torch.Tensor) else indptr, dtype=np.int64)
         ix_h = np.asarray(indices.cpu() if isinstance(indices, torch.Tensor) else indices, dtype=np.int64)
         a1_h = np.asarray(args1.cpu() if isinstance(args1, torch.Tensor) else args1, dtype=np.int64)
         a2_h = np.asarray(args2.cpu() if isinstance(args2, torch.Tensor) else args2, dtype=np.int64)
         n = ip_h.size - 1
         if n < 0 or a1_h.shape != (n,) or a2_h.shape != (n,):
-            raise ValueError("rank_arguments: indptr has %d entries, args1 %s and args2 %s; expected n+1, (n,), (n,)"
-                             % (ip_h.size, a1_h.shape, a2_h.shape))
+            raise ValueError("%s: indptr has %d entries, args1 %s and args2 %s; expected n+1, (n,), (n,)"
+                             % (what, ip_h.size, a1_h.shape, a2_h.shape))
         if n > 0 and (np.any(np.diff(ip_h) < 0) or ip_h[0] < 0 or ip_h[-1] > ix_h.size):
-            raise ValueError("rank_arguments: indptr is not a non-decreasing offset array into %d indices" % ix_h.size)
+            raise ValueError("%s: indptr is not a non-decreasing offset array into %d indices" % (what, ix_h.size))
         for name, a in (("args1", a1_h), ("args2", a2_h)):
             if a.size and (a.min() < 0 or a.max() >= self.N):
-                raise ValueError("rank_arguments: %s holds entity ids outside [0, N = %d): min %d, max %d"
-                                 % (name, self.N, a.min(), a.max()))
+                raise ValueError("%s: %s holds entity ids outside [0, N = %d): min %d, max %d"
+                                 % (what, name, self.N, a.min(), a.max()))
         used = ix_h[ip_h[0]:ip_h[-1]] if n > 0 else ix_h[:0]
         if used.size and (used.min() < 0 or used.max() >= self.F):
-            raise ValueError("rank_arguments: indices hold feature ids outside [0, F = %d): min %d, max %d"
-                             % (self.F, used.min(), used.max()))
+            raise ValueError("%s: indices hold feature ids outside [0, F = %d): min %d, max %d"
+                             % (what, self.F, used.min(), used.max()))
         ip, ix = self._dev_i32(indptr), self._dev_i32(indices)
         a1, a2 = self._dev_i32(args1), self._dev_i32(args2)
         if ix.numel() == 0:                  # rows without features only: the library wants a non-null array
             ix = torch.zeros(1, dtype=torch.int32, device=self.device)
         if n == 0:
             a1 = a2 = torch.zeros(1, dtype=torch.int32, device=self.device)
+        return n, ip, ix, a1, a2
+
+    def rank_arguments(self, indptr, indices, args1, args2):
+        """Entity ranks of every row's true arguments under the bound model, from one ``rae_rank_arguments`` call ->
+        (rank1 int32 [n], rank2 int32 [n]).  rank_s = 1 + the number of other entities whose candidate score in slot s
+        (the decoder's negative-sample score with that argument replaced) exceeds the true one's.  Host or device int32
+        CSR and argument ids of any length; entity ids must lie in [0, N) and feature ids in [0, F).  The call reuses the
+        handle's per-batch scratch, so ``last_probs`` afterwards no longer shows the last training step."""
+        n, ip, ix, a1, a2 = self._argument_inputs("rank_arguments", indptr, indices, args1, args2)
         r1 = torch.empty(max(n, 1), dtype=torch.int32, device=self.device)
         r2 = torch.empty(max(n, 1), dtype=torch.int32, device=self.device)
         self._check(self.lib.rae_rank_arguments(self._h, _ptr(ip), _ptr(ix), _ptr(a1), _ptr(a2), n, _ptr(r1), _ptr(r2),
                                                 self._stream), "rae_rank_arguments")
         torch.cuda.synchronize(self.device)
         return r1[:n].cpu().numpy(), r2[:n].cpu().numpy()
+
+    def predict_arguments(self, indptr, indices, args1, args2, k: int):
+        """The k most likely entities of each argument slot of every row, from one ``rae_predict_arguments`` call ->
+        (ids1 int32 [n, k], scores1 float32 [n, k], ids2, scores2).  Slot 1 lists candidates for args1 (it reads args2,
+        never args1), slot 2 candidates for args2 (it reads args1, never args2); per row, score descending, equal scores by
+        ascending entity id.  Scores order a row's candidates but are not comparable across rows.  Inputs and checks as
+        :meth:`rank_arguments`, and 1 <= k <= min(N, 16).  The call reuses the handle's per-batch scratch, so
+        ``last_probs`` afterwards no longer shows the last training step."""
+        k = int(k)
+        if not 1 <= k <= min(self.N, L.RAE_MAX_TOPK):
+            raise ValueError("predict_arguments: k = %d is outside [1, min(N = %d, %d)]" % (k, self.N, L.RAE_MAX_TOPK))
+        n, ip, ix, a1, a2 = self._argument_inputs("predict_arguments", indptr, indices, args1, args2)
+        size = max(n * k, 1)
+        out = [torch.empty(size, dtype=dt, device=self.device) for dt in (torch.int32, torch.float32) * 2]
+        self._check(self.lib.rae_predict_arguments(self._h, _ptr(ip), _ptr(ix), _ptr(a1), _ptr(a2), n, k,
+                                                   *[_ptr(t) for t in out], self._stream), "rae_predict_arguments")
+        torch.cuda.synchronize(self.device)
+        return tuple(t[:n * k].reshape(n, k).cpu().numpy() for t in out)
 
     # ------------------------------------------------------------------ introspection
     def last_probs(self) -> np.ndarray:

@@ -3,7 +3,8 @@ cluster holds.  This is what the reference's ``learn(debug=True)`` pickles (``Oi
 ``compute_posteriors`` returns (``:240-250``) and ``Visualizator.print_clusters`` prints (``evaluation/Visuals.py:8-30``).
 
     python -m relation_autoencoder_b200.export train_products/m.npz sample.pk --out exported/ \\
-        [--split train --split test ...] [--tsv new_sentences.txt ...] [--top-k 3] [--rank-arguments] [--device 0]
+        [--split train --split test ...] [--tsv new_sentences.txt ...] [--top-k 3] [--rank-arguments]
+        [--predict-arguments 5] [--device 0]
 
 Every row of every labelled set is labelled, the tail batch included, by one ``rae_label_topk`` call on one GPU (the
 checkpoint does not depend on the world size it was trained on).  New sentences (``--tsv``) are featurised through the
@@ -16,6 +17,15 @@ ranked against all entities (``rae_rank_arguments``: rank 1 + the number of enti
 beats the true one's).  Per set, ``NAME.argranks.npz`` holds ``rank1`` and ``rank2`` (-1 for a row whose entity strings
 the dataset never saw: such rows cannot be ranked and are left out of the metrics), and ``summary.json`` gets
 ``sets[NAME]['arguments']``: rows ranked and skipped, and MRR, mean rank and Hits@1/3/10 per slot and over both slots.
+
+With ``--predict-arguments K`` the decoder is asked what it was trained to answer: for each example, the K entities it
+scores highest in each argument slot (``rae_predict_arguments``).  A slot is predicted whenever the argument it is
+conditioned on (the other one) is an entity the dataset knows, even if the argument it predicts is not: that is the case
+``--rank-arguments`` has to skip.  Per set, ``NAME.argpreds.npz`` holds ``ids1, scores1, ids2, scores2`` ([n, K]; ids -1
+and scores NaN for a slot that was not predicted), ``NAME.argpreds.tsv`` lists them as ``entity:score`` with the 1-based
+position of the true argument in each list (0: not in the list, -1: unknown or not predicted), and ``summary.json`` gets
+``sets[NAME]['predictions']``: rows predicted per slot and the share of those with a known true argument that list it.
+Scores order one row's candidates; they are not comparable across rows.
 """
 from __future__ import annotations
 
@@ -55,9 +65,8 @@ def csr_of(examples, F: int):
     return indptr.astype(np.int32), indices, n_features
 
 
-def cuda_labeller(ck: dict, device: int = 0):
-    """(labeller, close): ``labeller(indptr, indices, k) -> (ids, probs)`` through :meth:`Engine.label_topk` on the
-    checkpoint's parameters.  Only W and Wb are read, but the engine binds every parameter of the decoder."""
+def _engine(ck: dict, device: int):
+    """An Engine bound to the checkpoint's parameters, with the checkpoint's batch size as the forward pass's chunk."""
     from .engine import Engine
     cfg, p = ck['config'], ck['params']
     F, K = p['W'].shape
@@ -65,20 +74,28 @@ def cuda_labeller(ck: dict, device: int = 0):
     B = int(cfg.get('batch_size', 1))
     eng = Engine(cfg['decoder'], K, d, int(cfg.get('neg_samples', 1)), B, F, N, B, device=device)
     eng.set_params_numpy(p)
+    return eng
+
+
+def cuda_labeller(ck: dict, device: int = 0):
+    """(labeller, close): ``labeller(indptr, indices, k) -> (ids, probs)`` through :meth:`Engine.label_topk` on the
+    checkpoint's parameters.  Only W and Wb are read, but the engine binds every parameter of the decoder."""
+    eng = _engine(ck, device)
     return (lambda indptr, indices, k: eng.label_topk(indptr, indices, k, probs=True)), eng.close
 
 
 def cuda_ranker(ck: dict, device: int = 0):
     """(ranker, close): ``ranker(indptr, indices, args1, args2) -> (rank1, rank2)`` through :meth:`Engine.rank_arguments`
     on the checkpoint's parameters, with the checkpoint's batch size as the forward pass's chunk."""
-    from .engine import Engine
-    cfg, p = ck['config'], ck['params']
-    F, K = p['W'].shape
-    N, d = p['A'].shape
-    B = int(cfg.get('batch_size', 1))
-    eng = Engine(cfg['decoder'], K, d, int(cfg.get('neg_samples', 1)), B, F, N, B, device=device)
-    eng.set_params_numpy(p)
+    eng = _engine(ck, device)
     return eng.rank_arguments, eng.close
+
+
+def cuda_predictor(ck: dict, device: int = 0):
+    """(predictor, close): ``predictor(indptr, indices, args1, args2, k) -> (ids1, scores1, ids2, scores2)`` through
+    :meth:`Engine.predict_arguments` on the checkpoint's parameters, as :func:`cuda_ranker`."""
+    eng = _engine(ck, device)
+    return eng.predict_arguments, eng.close
 
 
 def rank_metrics(ranks: np.ndarray) -> dict:
@@ -113,6 +130,54 @@ def _rank_set(out_dir: str, name: str, examples, arg2id: Dict[str, int], F: int,
         entry['arg1'] = rank_metrics(rank1[ok])
         entry['arg2'] = rank_metrics(rank2[ok])
         entry['both'] = rank_metrics(np.concatenate([rank1[ok], rank2[ok]]))
+    return entry
+
+
+def _position(ids: np.ndarray, true: np.ndarray, known: np.ndarray) -> np.ndarray:
+    """1-based position of true[i] in ids[i] (0: not listed), -1 where known[i] is False."""
+    hit = ids == true[:, None]
+    pos = np.where(hit.any(1), hit.argmax(1) + 1, 0)
+    return np.where(known, pos, -1).astype(np.int64)
+
+
+def _predict_set(out_dir: str, name: str, examples, arg2id: Dict[str, int], id2arg, F: int, predictor, k: int,
+                 relation: np.ndarray) -> dict:
+    """Predicts each slot whose conditioning argument is known, writes NAME.argpreds.npz / .tsv and returns the summary
+    entry."""
+    n = len(examples)
+    a1 = np.array([arg2id.get(ex.arg1, -1) for ex in examples], dtype=np.int64)
+    a2 = np.array([arg2id.get(ex.arg2, -1) for ex in examples], dtype=np.int64)
+    k1, k2 = a1 >= 0, a2 >= 0
+    send = np.flatnonzero(k1 | k2)
+    ids = [np.full((n, k), -1, np.int32), np.full((n, k), -1, np.int32)]
+    scores = [np.full((n, k), np.nan, np.float32), np.full((n, k), np.nan, np.float32)]
+    if send.size:
+        indptr, indices, _ = csr_of([examples[i] for i in send], F)
+        got = predictor(indptr, indices, np.maximum(a1[send], 0).astype(np.int32), np.maximum(a2[send], 0).astype(np.int32), k)
+        got = [np.asarray(g) for g in got]
+        if len(got) != 4 or any(g.shape != (send.size, k) for g in got):
+            raise RuntimeError("the predictor returned %s for %d rows and k = %d" % ([g.shape for g in got], send.size, k))
+        # slot 1 predicts arg1 from arg2, slot 2 predicts arg2 from arg1: keep a slot only where its condition is known
+        for s, cond in ((0, k2), (1, k1)):
+            rows = send[cond[send]]
+            ids[s][rows] = got[2 * s][cond[send]]
+            scores[s][rows] = got[2 * s + 1][cond[send]]
+    np.savez(os.path.join(out_dir, name + '.argpreds.npz'), ids1=ids[0], scores1=scores[0], ids2=ids[1], scores2=scores[1])
+    pos1 = _position(ids[0], a1, k1 & k2)
+    pos2 = _position(ids[1], a2, k1 & k2)
+
+    def listing(i, s):
+        return ' '.join('%s:%.6g' % (id2arg[x], v) for x, v in zip(ids[s][i], scores[s][i]) if x >= 0)
+    with open(os.path.join(out_dir, name + '.argpreds.tsv'), 'w', encoding='utf-8') as f:
+        f.write('index\targ1\targ2\ttrigger\trelation\tpredicted_arg1\tpredicted_arg2\tposition1\tposition2\n')
+        for i, ex in enumerate(examples):
+            f.write('%d\t%s\t%s\t%s\t%d\t%s\t%s\t%d\t%d\n' % (i, ex.arg1, ex.arg2, ex.trigger, relation[i], listing(i, 0),
+                                                              listing(i, 1), pos1[i], pos2[i]))
+    entry = {'k': k}
+    for slot, pos, cond in (('arg1', pos1, k2), ('arg2', pos2, k1)):
+        known = pos >= 0
+        entry[slot] = {'rows_predicted': int(cond.sum()), 'rows_with_known_argument': int(known.sum()),
+                       'share_in_list': float(np.mean(pos[known] > 0)) if known.any() else None}
     return entry
 
 
@@ -165,14 +230,16 @@ def _write_set(out_dir: str, name: str, examples, gold, ids, probs, n_features):
 
 def export(checkpoint: str, dataset: str, out_dir: str, splits: Optional[Sequence[str]] = None, tsv: Sequence[str] = (),
            k: int = 3, device: int = 0, labeller: Optional[Callable] = None, rank_arguments: bool = False,
-           ranker: Optional[Callable] = None) -> dict:
+           ranker: Optional[Callable] = None, predict_arguments: int = 0, predictor: Optional[Callable] = None) -> dict:
     """Labels the requested splits of ``dataset`` (default: all of them) and the sentences of each ``tsv`` file with the
     k most probable relations of the model in ``checkpoint``, writes the files the module docstring lists into
     ``out_dir`` and returns the summary.  ``labeller(indptr, indices, k) -> (ids int32 [n, k], probs float32 [n, k])``
     replaces the CUDA engine (there is no CPU fallback: without a GPU and without a labeller this raises).  With
     ``rank_arguments`` every set's arguments are ranked as well (module docstring); ``ranker(indptr, indices, args1,
-    args2) -> (rank1 int32 [n], rank2 int32 [n])`` replaces the CUDA engine there in the same way.  The arguments are
-    checked before any GPU work."""
+    args2) -> (rank1 int32 [n], rank2 int32 [n])`` replaces the CUDA engine there in the same way.  With
+    ``predict_arguments = K > 0`` the K most likely entities of each argument slot are written (module docstring);
+    ``predictor(indptr, indices, args1, args2, K) -> (ids1, scores1, ids2, scores2)`` replaces the CUDA engine there.
+    The arguments are checked before any GPU work."""
     try:
         ck = load_model(checkpoint)
     except Exception as e:
@@ -199,13 +266,17 @@ def export(checkpoint: str, dataset: str, out_dir: str, splits: Optional[Sequenc
         if stem in names:
             raise ValueError("the TSV file %s would be written as set %r, which is already a set of this export" % (path, stem))
         names.append(stem)
-    arg2id = None
-    if rank_arguments:
-        _, _, arg2id = entity_index(data)
+    arg2id = id2arg = None
+    predict_arguments = int(predict_arguments)
+    if rank_arguments or predict_arguments:
+        _, id2arg, arg2id = entity_index(data)
         A = ck['params'].get('A')
         if A is None or A.ndim != 2 or A.shape[0] != len(arg2id):
             raise ValueError("the checkpoint's A has %s rows, but the dataset has %d entities: the model was not trained on "
                              "this dataset" % (None if A is None else A.shape[0], len(arg2id)))
+    if predict_arguments and not 1 <= predict_arguments <= min(len(arg2id), MAX_TOP_K):
+        raise ValueError("--predict-arguments %d is outside [1, min(N, %d)] = [1, %d]"
+                         % (predict_arguments, MAX_TOP_K, min(len(arg2id), MAX_TOP_K)))
     sets = [(s, data[s], gold.get(s, {}), True) for s in splits]
     for path, name in zip(tsv, names[len(splits):]):
         ex, g = featurize(path, lex, feats)
@@ -217,6 +288,9 @@ def export(checkpoint: str, dataset: str, out_dir: str, splits: Optional[Sequenc
     close_ranker = None
     if rank_arguments and ranker is None:
         ranker, close_ranker = cuda_ranker(ck, device)
+    close_predictor = None
+    if predict_arguments and predictor is None:
+        predictor, close_predictor = cuda_predictor(ck, device)
     os.makedirs(out_dir, exist_ok=True)
     B = int(cfg.get('batch_size', 1))
     summary = {'checkpoint': os.path.abspath(checkpoint),
@@ -241,12 +315,17 @@ def export(checkpoint: str, dataset: str, out_dir: str, splits: Optional[Sequenc
                     entry['b3_driver_rows'] = _b3(g, name, ids[:, 0], (n // B) * B)
             if rank_arguments:
                 entry['arguments'] = _rank_set(out_dir, name, examples, arg2id, F, ranker)
+            if predict_arguments:
+                entry['predictions'] = _predict_set(out_dir, name, examples, arg2id, id2arg, F, predictor, predict_arguments,
+                                                    ids[:, 0])
             summary['sets'][name] = entry
     finally:
         if close is not None:
             close()
         if close_ranker is not None:
             close_ranker()
+        if close_predictor is not None:
+            close_predictor()
     with open(os.path.join(out_dir, 'summary.json'), 'w') as f:
         json.dump(summary, f, indent=1)
     return summary
@@ -263,10 +342,14 @@ def main(argv=None):
     p.add_argument('--top-k', dest='k', type=int, default=3, help='relations kept per example (1 to min(K, 16))')
     p.add_argument('--rank-arguments', action='store_true',
                    help='also rank every example\'s true arguments against all entities (MRR, mean rank, Hits@1/3/10)')
+    p.add_argument('--predict-arguments', dest='predict_arguments', type=int, default=None, metavar='K',
+                   help='also list the K most likely entities of each argument slot of every example (1 to min(N, 16))')
     p.add_argument('--device', type=int, default=0, help='CUDA device index')
     a = p.parse_args(argv)
+    if a.predict_arguments is not None and a.predict_arguments < 1:
+        p.error('--predict-arguments %d: K must be at least 1' % a.predict_arguments)
     summary = export(a.checkpoint, a.dataset, a.out, splits=a.split, tsv=a.tsv, k=a.k, device=a.device,
-                     rank_arguments=a.rank_arguments)
+                     rank_arguments=a.rank_arguments, predict_arguments=a.predict_arguments or 0)
     for name, s in summary['sets'].items():
         b3 = s.get('b3')
         args = s.get('arguments', {}).get('both')
