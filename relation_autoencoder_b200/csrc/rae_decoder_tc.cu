@@ -76,7 +76,7 @@ __device__ int g_tc_knock = 0;
 // this CTA's segment count and whether one of its segments ends a tile (its range holds the tile's last unit)
 #define TC_TRACE_SEGS(sch, slot_n, slot_end)                                                                   \
     do {                                                                                                       \
-        TcSegIter si_(sch, blockIdx.x);                                                                        \
+        TcSegIter si_(p.segs, (sch).upt, blockIdx.x);                                                          \
         TcSeg sg_;                                                                                             \
         int n_ = 0, e_ = 0;                                                                                    \
         while (si_.next(sg_)) { ++n_; e_ |= sg_.u1 == (sch).upt; }                                             \
@@ -306,16 +306,24 @@ __device__ __forceinline__ float ldg_ordered(const float* p) {
 
 // segments of a CTA's range under the balanced schedule (rae_internal.h)
 struct TcSeg { int tile, u0, u1, slot; };
+// A CTA's range comes from the schedule's table (tc_init: tc_seg_table), one int4 per CTA: first unit, end unit, slot of
+// the first segment.  Every role of every CTA reads its entry instead of evaluating the closed form: the divisions of
+// tcs_start / tcs_first, run by all 12-20 warps of a CTA at its start, cost thousands of cycles per CTA.  Only the first
+// segment can start inside a tile; every later one starts its tile, so this CTA is the tile's first and writes slot 0.
 struct TcSegIter {
-    TcSched s; long long cur, end; int x;
-    __device__ __forceinline__ TcSegIter(TcSched s_, int x_) : s(s_), cur(tcs_start(s_, x_)), end(tcs_start(s_, x_ + 1)), x(x_) {}
+    int upt, cur, end, slot;
+    __device__ __forceinline__ TcSegIter(const int4* segs, int upt_, int x) : upt(upt_) {
+        const int4 e = __ldg(segs + x);
+        cur = e.x; end = e.y; slot = e.z;
+    }
     __device__ __forceinline__ bool next(TcSeg& g) {
         if (cur >= end) return false;
-        g.tile = (int)(cur / s.upt);
-        g.u0 = (int)(cur - (long long)g.tile * s.upt);
-        const long long len = min((long long)(s.upt - g.u0), end - cur);
-        g.u1 = g.u0 + (int)len;
-        g.slot = x - tcs_first(s, g.tile);
+        g.tile = cur / upt;
+        g.u0 = cur - g.tile * upt;
+        const int len = min(upt - g.u0, end - cur);
+        g.u1 = g.u0 + len;
+        g.slot = slot;
+        slot = 0;
         cur += len;
         return true;
     }
@@ -538,6 +546,7 @@ struct TcArgs {
     int n_sp_half;          // half chunks holding C1/C2 rows (forward only; 0 for the recompute pass)
     int nbs;                // B-operand shared-memory stages
     TcSched sch;            // units = 128-row chunks, tiles = example tiles
+    const int4* segs;       // sch's per-CTA table (TcSegIter)
 };
 
 template <int DP>
@@ -583,7 +592,7 @@ __global__ void __launch_bounds__(TC_FWD_THREADS, 1) k_tc_bilinear(TcArgs p) {
     if (warp == TC_FWD_WORKERS + 1) {
         // ===== producer: per segment the P image of its tile, then its chunks; one bulk copy per ring stage =====
         if (lane == 0) {
-            TcSegIter si(p.sch, blockIdx.x);
+            TcSegIter si(p.segs, p.sch.upt, blockIdx.x);
             TcSeg sg;
             int it = 0;
             auto fill = [&](const uint8_t* src) {
@@ -610,7 +619,7 @@ __global__ void __launch_bounds__(TC_FWD_THREADS, 1) k_tc_bilinear(TcArgs p) {
             const uint32_t a_hi = tmem_base + TC_FWD_ACOL, a_lo = a_hi + KC;
             const int ksteps = p.KH / 16;                   // 1 .. 7
             const int kmid = ksteps / 2;
-            TcSegIter si(p.sch, blockIdx.x);
+            TcSegIter si(p.segs, p.sch.upt, blockIdx.x);
             TcSeg sg;
             int it = 0, seg = 0;
             // ring positions kept incrementally (no division by the runtime stage count in the loop): operand stage s with
@@ -679,7 +688,7 @@ __global__ void __launch_bounds__(TC_FWD_THREADS, 1) k_tc_bilinear(TcArgs p) {
         constexpr int RW = (DP >= 64) ? 64 : 32;      // columns of R / w held per thread
         const int jbase = (DP == 128) ? 64 * g : 0;
         const float inv = 1.f / (TC_QSCALE * pow2_scale(p.scal[TS_AMAX_C]));      // undoes the operand scales (a power of two)
-        TcSegIter si(p.sch, blockIdx.x);
+        TcSegIter si(p.segs, p.sch.upt, blockIdx.x);
         TcSeg sg;
         int it = 0, seg = 0;
         while (si.next(sg)) {
@@ -1056,6 +1065,7 @@ struct TcDqArgs {
     int B, d, dp, K, NK;
     int n_bil_rows;         // reduction rows holding bilinear rows (a multiple of 128)
     TcSched sch;            // units = stages of 128 reduction rows, tiles = example tiles
+    const int4* segs;       // sch's per-CTA table (TcSegIter)
 };
 
 // MMAs of one dq segment: 24 kind::f16 MMAs per stage (8 k-steps of 16 reduction rows x {hi.hi, hi.lo, lo.hi}); issued by ONE
@@ -1138,7 +1148,7 @@ __global__ void __launch_bounds__(TC_BWD_THREADS, 1) k_tc_dq(TcDqArgs p) {
     }
     if (warp == TC_BWD_WORKERS + 1) {
         if (lane == 0) {
-            TcSegIter si(p.sch, blockIdx.x);
+            TcSegIter si(p.segs, p.sch.upt, blockIdx.x);
             TcSeg sg;
             int it = 0;
             while (si.next(sg)) {
@@ -1148,7 +1158,7 @@ __global__ void __launch_bounds__(TC_BWD_THREADS, 1) k_tc_dq(TcDqArgs p) {
         }
     } else if (warp == TC_BWD_WORKERS) {
         if (elect_one()) {
-            TcSegIter si(p.sch, blockIdx.x);
+            TcSegIter si(p.segs, p.sch.upt, blockIdx.x);
             TcSeg sg;
             int it = 0, seg = 0;
             while (si.next(sg)) {
@@ -1182,7 +1192,7 @@ __global__ void __launch_bounds__(TC_BWD_THREADS, 1) k_tc_dq(TcDqArgs p) {
             sG = pow2_scale(__float_as_uint(bound));
             inv = 1.f / (sG * pow2_scale(p.scal[TS_AMAX_C]));
         }
-        TcSegIter si(p.sch, blockIdx.x);
+        TcSegIter si(p.segs, p.sch.upt, blockIdx.x);
         TcSeg sg;
         int it = 0, seg = 0;
         while (si.next(sg)) {
@@ -1314,6 +1324,7 @@ struct TcDcArgs {
     int tile0;              // first 128-row tile this launch covers (the C1 / C2 tiles when k_tc_dc2 takes the bilinear rows)
     size_t split_stride;    // units*d*K
     TcSched sch;            // units = stages of 64 examples, tiles = 128-row tiles of the operand rows (from tile0 on)
+    const int4* segs;       // sch's per-CTA table (TcSegIter)
 };
 
 __global__ void __launch_bounds__(TC_BWD_THREADS, 1) k_tc_dc(TcDcArgs p) {
@@ -1333,7 +1344,7 @@ __global__ void __launch_bounds__(TC_BWD_THREADS, 1) k_tc_dc(TcDcArgs p) {
     float* sP1 = reinterpret_cast<float*>(smem_raw + TC_BSTAGES * ST_BYTES + 256);
     float* sP2 = sP1 + (size_t)nsrc * nbc;
     {
-        TcSegIter si(p.sch, blockIdx.x);
+        TcSegIter si(p.segs, p.sch.upt, blockIdx.x);
         TcSeg sg;
         int off = 0;                                        // example offset of the segment inside the staging area
         while (si.next(sg)) {
@@ -1367,7 +1378,7 @@ __global__ void __launch_bounds__(TC_BWD_THREADS, 1) k_tc_dc(TcDcArgs p) {
     }
     if (warp == TC_BWD_WORKERS + 1) {
         if (lane == 0) {
-            TcSegIter si(p.sch, blockIdx.x);
+            TcSegIter si(p.segs, p.sch.upt, blockIdx.x);
             TcSeg sg;
             int it = 0;
             while (si.next(sg)) {
@@ -1376,7 +1387,7 @@ __global__ void __launch_bounds__(TC_BWD_THREADS, 1) k_tc_dc(TcDcArgs p) {
             }
         }
     } else if (warp == TC_BWD_WORKERS) {
-        TcSegIter si(p.sch, blockIdx.x);
+        TcSegIter si(p.segs, p.sch.upt, blockIdx.x);
         TcSeg sg;
         int it = 0, seg = 0;
         while (si.next(sg)) {
@@ -1396,7 +1407,7 @@ __global__ void __launch_bounds__(TC_BWD_THREADS, 1) k_tc_dc(TcDcArgs p) {
         const uint32_t lane_base = tmem_base + ((uint32_t)(q4 * 32) << 16);
         const size_t estride = (size_t)E_NV * p.dp;
         const int src = q4 / (p.DP >> 5);
-        TcSegIter si(p.sch, blockIdx.x);
+        TcSegIter si(p.segs, p.sch.upt, blockIdx.x);
         TcSeg sg;
         int it = 0, seg = 0, off = 0;
         while (si.next(sg)) {
@@ -1529,6 +1540,7 @@ struct TcDc2Args {
     int n_bil_tiles;
     size_t split_stride;
     TcSched sch;            // units = stages of 64 examples, tiles = PAIRS of 128-row tiles
+    const int4* segs;       // sch's per-CTA table (TcSegIter)
 };
 
 __global__ void __launch_bounds__(TC_BWD_THREADS, 1) k_tc_dc2(TcDc2Args p) {
@@ -1577,7 +1589,7 @@ __global__ void __launch_bounds__(TC_BWD_THREADS, 1) k_tc_dc2(TcDc2Args p) {
     if (warp == TC_BWD_WORKERS + 1) {
         // ===== producer of the q^T operand ring =====
         if (lane == 0) {
-            TcSegIter si(p.sch, blockIdx.x);
+            TcSegIter si(p.segs, p.sch.upt, blockIdx.x);
             TcSeg sg;
             int it = 0;
             while (si.next(sg)) {
@@ -1592,7 +1604,7 @@ __global__ void __launch_bounds__(TC_BWD_THREADS, 1) k_tc_dc2(TcDc2Args p) {
     } else if (warp == TC_BWD_WORKERS + 3) {
         // ===== producer of the image ring: R image, Y2 image, and the 64-example slices of a_i / L_i of the tiles' rows =====
         if (lane == 0) {
-            TcSegIter si(p.sch, blockIdx.x);
+            TcSegIter si(p.segs, p.sch.upt, blockIdx.x);
             TcSeg sg;
             int it = 0;
             while (si.next(sg)) {
@@ -1621,7 +1633,7 @@ __global__ void __launch_bounds__(TC_BWD_THREADS, 1) k_tc_dc2(TcDc2Args p) {
         // ===== MMA issuer: one elected thread, fully unrolled (see k_tc_bilinear) =====
         if (elect_one()) {
             const uint32_t idesc = make_idesc_f16(TC_M, p.NK);
-            TcSegIter si(p.sch, blockIdx.x);
+            TcSegIter si(p.segs, p.sch.upt, blockIdx.x);
             TcSeg sg;
             int it = 0, seg = 0;
             while (si.next(sg)) {
@@ -1694,7 +1706,7 @@ __global__ void __launch_bounds__(TC_BWD_THREADS, 1) k_tc_dc2(TcDc2Args p) {
             sG = pow2_scale(__float_as_uint(fmaf(aA, aR, aL * aY)));
             inv = 1.f / (sG * TC_QSCALE);
         }
-        TcSegIter si(p.sch, blockIdx.x);
+        TcSegIter si(p.segs, p.sch.upt, blockIdx.x);
         TcSeg sg;
         int it = 0, seg = 0;
         while (si.next(sg)) {
@@ -1911,11 +1923,26 @@ extern "C" int rae_debug_set_knock(int bits) { return (int)cudaMemcpyToSymbol(g_
 namespace {
 #endif
 
+// cost weights of a schedule (TcSched): tail units, body / tail unit weight, tile-start weight
+struct TcCost { int ntail = 0, wb = 1, wt = 1, h = 0; };
+
+int sched_max_share(TcSched s) {
+    int m = 0;
+    for (int x = 0; x < s.G; ++x) m = std::max(m, tcs_start(s, x + 1) - tcs_start(s, x));
+    return m;
+}
+bool sched_nonempty(TcSched s) {
+    for (int x = 0; x < s.G; ++x)
+        if (tcs_start(s, x + 1) == tcs_start(s, x)) return false;
+    return true;
+}
+
 // balanced schedule of T = ntile * upt units: one CTA per SM, or whole waves of CTAs when a CTA's share would exceed
-// `max_share` units (accuracy bound on the MMA chain of one accumulator / capacity of a staging area)
-TcSched make_sched(int ntile, int upt, int num_sms, int max_share) {
-    TcSched s;
-    s.ntile = ntile; s.upt = upt;
+// `max_share` units (accuracy bound on the MMA chain of one accumulator / capacity of a staging area).  A CTA's share
+// of the virtual time must hold a unit: where a tile's first unit (h + wb) or a tail unit (wt) is longer than the share
+// (a few units per CTA, as at d = 30), both are capped at it.
+TcSched make_sched(int ntile, int upt, int num_sms, int max_share, TcCost c = TcCost{}) {
+    TcSched s{0, upt, ntile, std::min(c.ntail, upt), c.wb, c.wt, c.h};
     const long long T = (long long)ntile * upt;
     long long G = std::min<long long>(T, num_sms);
     if (max_share > 0 && (T + G - 1) / G > max_share) {
@@ -1923,16 +1950,26 @@ TcSched make_sched(int ntile, int upt, int num_sms, int max_share) {
         G = std::min<long long>(T, waves * num_sms);
     }
     s.G = (int)std::max<long long>(G, 1);
-    return s;
+    // terminates: each step lowers h or wt or adds a wave; with uniform weights every CTA is non-empty (G <= T) and
+    // the wave count above bounds the share
+    for (;;) {
+        if (!sched_nonempty(s)) {
+            const int share = (int)((long long)tcs_tile_len(s) * s.ntile / s.G);
+            int wt = std::max(s.wb, std::min(s.wt, share));
+            int h = std::max(0, std::min(s.h, share - s.wb));
+            if (wt == s.wt && h == s.h) { wt = std::max(s.wb, wt - 1); h = std::max(0, h - 1); }   // rounding: step down
+            s.wt = wt; s.h = h;
+        } else if (max_share > 0 && s.G < T && sched_max_share(s) > max_share) {
+            s.G = (int)std::min<long long>(T, (long long)s.G + num_sms);
+        } else {
+            return s;
+        }
+    }
 }
 int sched_max_slots(TcSched s) {
     int m = 1;
     for (int t = 0; t < s.ntile; ++t) m = std::max(m, tcs_nslots(s, t));
     return m;
-}
-int sched_max_share(TcSched s) {
-    const long long T = (long long)s.ntile * s.upt;
-    return (int)((T + s.G - 1) / s.G);
 }
 
 }  // namespace
@@ -1960,40 +1997,102 @@ int tc_supported(const rae_engine* h) {
     if (!h->hasM) return 0;
     if (h->d <= 16 || h->d > 128) return 0;
     if (h->K > 104) return 0;
+    if (h->B > (1 << 24)) return 0;     // the schedules' virtual time (TcSched) is an int: ntile * L < 2^17 * 2^11
     return 1;
 }
 
-int tc_init(rae_engine* h) {
-    const int DP = tc_dp(h->d);
-    TcState& t = h->tc;
+namespace {
+// Cost weights of the forward, recompute and dq schedules, in eighths of a body unit, fitted to the in-kernel trace at
+// K = 100 with selectional preferences on one B200 (profiles/r04_weighted_schedule.md, profiles/fit_sched_cost.py: CTA
+// life, less the body units at the pass's steady cadence, by least squares over the tail units and the extra segments of
+// each CTA).  DP = 128: the trace of the weighted schedule at T (profiles/r04_cta_life_weighted_T.csv), where CTAs of
+// 15-32 units and one or two segments pin h and wt down better than the uniform split did.  DP = 32: the trace of the
+// uniform split at cfg2 (profiles/r04_cta_life_before_cfg2.csv); make_sched caps these there anyway (two units per CTA).
+// DP = 64: the mean of the two.  Other K and shapes without selectional preferences take the same weights unmeasured.
+TcCost tc_cost(int DP, int pass, int ntail) {
+    const int di = DP == 128 ? 0 : DP == 64 ? 1 : 2;
+    static const int H[3][3] = {{64, 48, 33}, {52, 40, 29}, {76, 77, 78}};       // [pass][DP 128, 64, 32] tile start
+    static const int WT[3][3] = {{30, 57, 84}, {8, 8, 8}, {41, 32, 22}};         // [pass][DP 128, 64, 32] tail unit
+    TcCost c;
+    c.ntail = ntail; c.wb = 8; c.wt = WT[pass][di]; c.h = H[pass][di];
+    return c;
+}
+
+// geometry of the contraction operands and the forward (pass 0), recompute (1) and dq (2) schedules of a shape: host
+// arithmetic only
+void tc_plan(TcState& t, int B, int K, int d, bool hasSP, int num_sms) {
+    const int DP = tc_dp(d);
     t.DP = DP;
-    t.KH = (h->K + 15) & ~15;
+    t.KH = (K + 15) & ~15;
     // bilinear rows i padded so that the operand rows fill whole 128-row stages (DP = 64: pairs of rows, DP = 32: fours)
     const int rps = 128 / DP;
-    const int di = (h->d + rps - 1) / rps * rps;
+    const int di = (d + rps - 1) / rps * rps;
     t.n_bil_rows = di * DP;
     t.n_bil_half = t.n_bil_rows / TC_H;
-    t.n_sp_half = h->hasSP ? (2 * DP) / TC_H : 0;
-    t.n_rows_total = (t.n_bil_rows + (h->hasSP ? 2 * DP : 0) + TC_M - 1) / TC_M * TC_M;
+    t.n_sp_half = hasSP ? (2 * DP) / TC_H : 0;
+    t.n_rows_total = (t.n_bil_rows + (hasSP ? 2 * DP : 0) + TC_M - 1) / TC_M * TC_M;
     t.n_chunks_fwd = (t.n_bil_half + t.n_sp_half + 1) / 2;
     t.n_chunks_rec = t.n_bil_half / 2;
-    t.ntile = (h->B + TC_M - 1) / TC_M;
+    t.ntile = (B + TC_M - 1) / TC_M;
+    // the chunks / stages that hold C1 / C2 rows close every tile of the forward and dq passes
+    const int n_st = t.n_rows_total / TC_M;
+    t.sch_fwd = make_sched(t.ntile, t.n_chunks_fwd, num_sms, 0, tc_cost(DP, 0, t.n_chunks_fwd - t.n_chunks_rec));
+    t.sch_rec = make_sched(t.ntile, t.n_chunks_rec, num_sms, 0, tc_cost(DP, 1, 0));
+    t.slots_vw = std::max(sched_max_slots(t.sch_fwd), sched_max_slots(t.sch_rec));
+    // backward operands: NK = relations padded to a multiple of 16.  dq reduces over stages of 128 operand rows (FP16
+    // pairs), dC over stages of 64 examples (TF32 pairs): both 2 * 2 * 8 * NK * 16 bytes per stage
+    t.NK = (K + 15) & ~15;
+    // accuracy bound of the dq reduction: the measured-safe chain is 1560 MMAs into one accumulator (4.5e-6 of
+    // ||dW||_inf at the target shape); a segment never exceeds TC_DQ_MAX_STAGES stages = 1536 MMAs
+    t.sch_dq = make_sched(t.ntile, n_st, num_sms, TC_DQ_MAX_STAGES, tc_cost(DP, 2, n_st - t.n_bil_rows / TC_M));
+    t.slots_dq = sched_max_slots(t.sch_dq);
+}
+}  // namespace
+
+// The schedule tc_plan builds for one pass (0 forward, 1 recompute, 2 dq), for the tests: its seven fields
+// (G, upt, ntile, ntail, wb, wt, h) -> sched[7], the first unit of every CTA and the end -> starts[G + 1] (when
+// max_starts >= G + 1) and the partial slots of every tile -> nslots[ntile] (when max_tiles >= ntile).  Returns G, or -1
+// for a shape the tensor path does not take.  Host only: needs no device.
+extern "C" int rae_debug_tc_schedule(int B, int K, int d, int hasSP, int num_sms, int pass, int32_t* sched, int64_t* starts,
+                                     int max_starts, int32_t* nslots, int max_tiles) {
+    if (B < 1 || K < 1 || K > 104 || d <= 16 || d > 128 || num_sms < 1 || pass < 0 || pass > 2) return -1;
+    TcState t;
+    tc_plan(t, B, K, d, hasSP != 0, num_sms);
+    const TcSched s = pass == 0 ? t.sch_fwd : pass == 1 ? t.sch_rec : t.sch_dq;
+    const int f[7] = {s.G, s.upt, s.ntile, s.ntail, s.wb, s.wt, s.h};
+    if (sched != nullptr) std::copy(f, f + 7, sched);
+    if (starts != nullptr && max_starts >= s.G + 1)
+        for (int x = 0; x <= s.G; ++x) starts[x] = tcs_start(s, x);
+    if (nslots != nullptr && max_tiles >= s.ntile)
+        for (int tl = 0; tl < s.ntile; ++tl) nslots[tl] = tcs_nslots(s, tl);
+    return s.G;
+}
+
+// make_sched itself, for the tests: the schedule of ntile tiles of upt units with the given weights (wb = 0: the default
+// uniform weights) -> sched[7] as above and starts[G + 1] (when max_starts >= G + 1).  Returns G.  Host only.
+extern "C" int rae_debug_tc_make_sched(int ntile, int upt, int num_sms, int max_share, int ntail, int wb, int wt, int h,
+                                       int32_t* sched, int64_t* starts, int max_starts) {
+    if (ntile < 1 || upt < 1 || num_sms < 1 || max_share < 0 || wb < 0 || (wb > 0 && (wt < wb || h < 0 || ntail < 0))) return -1;
+    TcCost c;
+    if (wb > 0) { c.ntail = ntail; c.wb = wb; c.wt = wt; c.h = h; }
+    const TcSched s = make_sched(ntile, upt, num_sms, max_share, c);
+    const int f[7] = {s.G, s.upt, s.ntile, s.ntail, s.wb, s.wt, s.h};
+    if (sched != nullptr) std::copy(f, f + 7, sched);
+    if (starts != nullptr && max_starts >= s.G + 1)
+        for (int x = 0; x <= s.G; ++x) starts[x] = tcs_start(s, x);
+    return s.G;
+}
+
+int tc_init(rae_engine* h) {
+    TcState& t = h->tc;
+    tc_plan(t, h->B, h->K, h->d, h->hasSP, h->num_sms);
+    const int DP = t.DP;
     // forward: as many 128-row operand stages as fit (4 at K = 100: 57 KB each)
     const size_t b_bytes = (size_t)2 * (t.KH / 8) * TC_N * 16;
     t.fwd_stages = (int)std::min<size_t>(4, ((size_t)h->max_smem_optin - 256) / b_bytes);
     if (t.fwd_stages < 2) return fail(h, RAE_EINVAL, "tensor path: K=%d needs %zu bytes per operand stage, two do not fit", h->K, b_bytes);
     t.smem = (size_t)t.fwd_stages * b_bytes + 256;
-    t.sch_fwd = make_sched(t.ntile, t.n_chunks_fwd, h->num_sms, 0);
-    t.sch_rec = make_sched(t.ntile, t.n_chunks_rec, h->num_sms, 0);
-    t.slots_vw = std::max(sched_max_slots(t.sch_fwd), sched_max_slots(t.sch_rec));
-    // backward operands: NK = relations padded to a multiple of 16.  dq reduces over stages of 128 operand rows (FP16
-    // pairs), dC over stages of 64 examples (TF32 pairs): both 2 * 2 * 8 * NK * 16 bytes per stage
-    t.NK = (h->K + 15) & ~15;
     const int n_st = t.n_rows_total / TC_M;
-    // accuracy bound of the dq reduction: the measured-safe chain is 1560 MMAs into one accumulator (4.5e-6 of
-    // ||dW||_inf at the target shape); a segment never exceeds TC_DQ_MAX_STAGES stages = 1536 MMAs
-    t.sch_dq = make_sched(t.ntile, n_st, h->num_sms, TC_DQ_MAX_STAGES);
-    t.slots_dq = sched_max_slots(t.sch_dq);
     const size_t st_bytes = (size_t)2 * 2 * 8 * t.NK * 16;
     t.smem_dq = (size_t)TC_BSTAGES * st_bytes + 256;
     if (t.smem_dq > (size_t)h->max_smem_optin) return fail(h, RAE_EINVAL, "tensor path: backward operand stages do not fit in shared memory");
@@ -2054,6 +2153,24 @@ int tc_init(rae_engine* h) {
             (e = cudaMemcpy(t.tile_slots, ts.data(), ts.size() * sizeof(int32_t), cudaMemcpyHostToDevice)) != cudaSuccess)
             return fail(h, RAE_ENOMEM, "tensor-path workspace: %s", cudaGetErrorString(e));
     }
+    {
+        // per-CTA tables of the five schedules (TcSegIter): first unit, end unit, slot of the first segment
+        std::vector<int4> tab;
+        auto add = [&](const TcSched& sc) {
+            const int off = (int)tab.size();
+            for (int x = 0; x < sc.G; ++x) {
+                const int u0 = tcs_start(sc, x);
+                tab.push_back(make_int4(u0, tcs_start(sc, x + 1), x - tcs_first(sc, u0 / sc.upt), 0));
+            }
+            return off;
+        };
+        t.segs_fwd = add(t.sch_fwd); t.segs_rec = add(t.sch_rec); t.segs_dq = add(t.sch_dq);
+        if (t.dc2) t.segs_dc2 = add(t.sch_dc2);
+        if (t.dc_tiles > 0) t.segs_dc = add(t.sch_dc);
+        if ((e = cudaMalloc((void**)&t.segs, tab.size() * sizeof(int4))) != cudaSuccess ||
+            (e = cudaMemcpy(t.segs, tab.data(), tab.size() * sizeof(int4), cudaMemcpyHostToDevice)) != cudaSuccess)
+            return fail(h, RAE_ENOMEM, "tensor-path workspace: %s", cudaGetErrorString(e));
+    }
 #define RAE_TC_ATTR(KERN, BYTES)                                                                                     \
     if ((e = cudaFuncSetAttribute(KERN, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(BYTES))) != cudaSuccess) \
         return fail(h, RAE_ECUDA, "cudaFuncSetAttribute(" #KERN "): %s", cudaGetErrorString(e));
@@ -2068,7 +2185,7 @@ int tc_init(rae_engine* h) {
 
 void tc_free(rae_engine* h) {
     TcState& t = h->tc;
-    cudaFree(t.bop); cudaFree(t.pimg); cudaFree(t.vT); cudaFree(t.wT); cudaFree(t.spT); cudaFree(t.bop2); cudaFree(t.dqT); cudaFree(t.pop3); cudaFree(t.scal); cudaFree(t.pop4); cudaFree(t.Rimg); cudaFree(t.Yimg); cudaFree(t.tile_slots);
+    cudaFree(t.bop); cudaFree(t.pimg); cudaFree(t.vT); cudaFree(t.wT); cudaFree(t.spT); cudaFree(t.bop2); cudaFree(t.dqT); cudaFree(t.pop3); cudaFree(t.scal); cudaFree(t.pop4); cudaFree(t.Rimg); cudaFree(t.Yimg); cudaFree(t.tile_slots); cudaFree(t.segs);
     cudaFree(t.aT); cudaFree(t.LT); cudaFree(t.RT); cudaFree(t.cT); cudaFree(t.Y2T);
     t = TcState{};
 }
@@ -2152,6 +2269,7 @@ int tc_contract(rae_engine* h, const float* LT_in, const float* RT_in, int slotV
     p.n_bil_half = t.n_bil_half; p.n_sp_half = with_sp ? t.n_sp_half : 0;
     p.nbs = t.fwd_stages;
     p.sch = with_sp ? t.sch_fwd : t.sch_rec;
+    p.segs = t.segs + (with_sp ? t.segs_fwd : t.segs_rec);
     if (t.DP == 32) launch_pdl(k_tc_bilinear<32>, dim3(p.sch.G), dim3(TC_FWD_THREADS), t.smem, st, p);
     else if (t.DP == 64) launch_pdl(k_tc_bilinear<64>, dim3(p.sch.G), dim3(TC_FWD_THREADS), t.smem, st, p);
     else launch_pdl(k_tc_bilinear<128>, dim3(p.sch.G), dim3(TC_FWD_THREADS), t.smem, st, p);
@@ -2186,6 +2304,7 @@ int tc_backward_dq(rae_engine* h, cudaStream_t st) {
     p.B = h->B; p.d = h->d; p.dp = h->dp; p.K = h->K; p.NK = t.NK;
     p.n_bil_rows = t.n_bil_rows;
     p.sch = t.sch_dq;
+    p.segs = t.segs + t.segs_dq;
     if (t.DP == 32) launch_pdl(k_tc_dq<32>, dim3(p.sch.G), dim3(TC_BWD_THREADS), t.smem_dq, st, p);
     else if (t.DP == 64) launch_pdl(k_tc_dq<64>, dim3(p.sch.G), dim3(TC_BWD_THREADS), t.smem_dq, st, p);
     else launch_pdl(k_tc_dq<128>, dim3(p.sch.G), dim3(TC_BWD_THREADS), t.smem_dq, st, p);
@@ -2219,6 +2338,7 @@ int tc_grad_dense(rae_engine* h, cudaStream_t st) {
         p.n_bil_tiles = t.n_bil_rows / TC_M;
         p.split_stride = (size_t)h->off_gWb;
         p.sch = t.sch_dc2;
+        p.segs = t.segs + t.segs_dc2;
         launch_pdl(k_tc_dc2, dim3(p.sch.G), dim3(TC_BWD_THREADS), t.smem_dc2, st, p);
         h->launches++;
         RAE_CUDA(h, cudaGetLastError());
@@ -2233,6 +2353,7 @@ int tc_grad_dense(rae_engine* h, cudaStream_t st) {
         p.tile0 = t.dc_tile0;
         p.split_stride = (size_t)h->off_gWb;
         p.sch = t.sch_dc;
+        p.segs = t.segs + t.segs_dc;
         launch_pdl(k_tc_dc, dim3(p.sch.G), dim3(TC_BWD_THREADS), t.smem_dc, st, p);
         h->launches++;
         RAE_CUDA(h, cudaGetLastError());

@@ -452,7 +452,7 @@ int rae_create(const rae_config* cfg, rae_engine** out) {
         RAE_CREATE_RC(tc_init(h));
         h->use_tc = true;
     } else if (cfg->flags & RAE_FLAG_FORCE_TENSOR) {
-        fail(nullptr, RAE_EINVAL, "RAE_FLAG_FORCE_TENSOR: the tcgen05 path needs a bilinear model with 16 < d <= 128 and K <= 104 (K=%d d=%d)", cfg->K, cfg->d);
+        fail(nullptr, RAE_EINVAL, "RAE_FLAG_FORCE_TENSOR: the tcgen05 path needs a bilinear model with 16 < d <= 128, K <= 104 and B <= 2^24 (K=%d d=%d B=%d)", cfg->K, cfg->d, cfg->B);
         rae_destroy(h);
         return RAE_EINVAL;
     }

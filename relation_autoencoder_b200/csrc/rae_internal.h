@@ -62,21 +62,45 @@ struct FeatureCache {
 
 // Balanced schedule of the tensor-core contractions (rae_decoder_tc.cu).  The work of a contraction is `ntile` tiles of
 // `upt` units each (a unit = one streamed operand chunk / pipeline stage); the T = ntile * upt units are dealt over G
-// CTAs in contiguous ranges [start(x), start(x+1)), start(x) = floor(x T / G), so every SM gets the same number of
-// MMAs whatever the tile count.  A range is cut at tile boundaries into segments; the segment of CTA x inside tile t
-// writes its partial result into slot x - first_cta(t).  G <= T, so every CTA owns at least one unit and the CTAs that
+// CTAs in contiguous ranges [start(x), start(x+1)) of equal estimated cost, so that the CTAs end together.  The cost is
+// counted in integer weights: a unit costs wb, each of the last `ntail` units of a tile wt instead (the forward pass's
+// C1 / C2 chunks, dq's selectional-preference stages), and every tile start h more (the segment switch a CTA pays when
+// its range crosses into the tile).  Tile t spans [t L, (t + 1) L) of this virtual time, L = h + (upt - ntail) wb +
+// ntail wt; its first unit starts at t L (and so carries h), unit i > 0 at t L + h + the weights of units 0 .. i-1.
+// CTA x starts with the unit that holds the point x V / G, V = ntile L.  Uniform weights (h = 0, wt = wb) give
+// start(x) = floor(x T / G).  A range is cut at tile boundaries into segments; the segment of CTA x inside tile t
+// writes its partial result into slot x - first_cta(t).  make_sched keeps every CTA non-empty, so the CTAs that
 // overlap a tile are consecutive.  G == 0 marks the rectangular layout of the SIMT path (`upt` = uniform slot count).
-struct TcSched { int G, upt, ntile; };
-__host__ __device__ __forceinline__ long long tcs_start(TcSched s, int x) { return (long long)x * s.upt * s.ntile / s.G; }
-// the CTA whose range holds unit u: the largest x with floor(x T / G) <= u
-__host__ __device__ __forceinline__ int tcs_cta_of(TcSched s, long long u) {
-    const long long T = (long long)s.upt * s.ntile;
-    return (int)(((u + 1) * s.G + T - 1) / T) - 1;
+// Units and virtual times are ints (tc_supported bounds B so that V fits); only the products x V and G vtime are 64-bit.
+struct TcSched { int G, upt, ntile, ntail, wb, wt, h; };
+__host__ __device__ __forceinline__ int tcs_tile_len(TcSched s) { return s.h + (s.upt - s.ntail) * s.wb + s.ntail * s.wt; }
+// virtual time at which unit u starts (u = T: V)
+__host__ __device__ __forceinline__ int tcs_vtime(TcSched s, int u) {
+    const int t = u / s.upt, i = u - t * s.upt, nb = s.upt - s.ntail;
+    int a = t * tcs_tile_len(s);
+    if (i > 0) a += s.h + (i < nb ? i : nb) * s.wb + (i > nb ? i - nb : 0) * s.wt;
+    return a;
 }
-__host__ __device__ __forceinline__ int tcs_first(TcSched s, int tile) { return tcs_cta_of(s, (long long)tile * s.upt); }
+// first unit of CTA x: the last unit u with vtime(u) <= floor(x V / G)
+__host__ __device__ __forceinline__ int tcs_start(TcSched s, int x) {
+    const int L = tcs_tile_len(s);
+    const int p = (int)((long long)x * (L * s.ntile) / s.G);
+    const int t = p / L;
+    if (t >= s.ntile) return s.ntile * s.upt;
+    const int q = p - t * L - s.h;                  // time past the end of the tile-start weight
+    const int nbw = (s.upt - s.ntail) * s.wb;
+    const int i = q < 0 ? 0 : q < nbw ? q / s.wb : (s.upt - s.ntail) + (q - nbw) / s.wt;
+    return t * s.upt + i;
+}
+// the CTA whose range holds unit u: the largest x with start(x) <= u, i.e. with x V / G < vtime(u + 1)
+__host__ __device__ __forceinline__ int tcs_cta_of(TcSched s, int u) {
+    const long long V = (long long)tcs_tile_len(s) * s.ntile;
+    return (int)(((long long)tcs_vtime(s, u + 1) * s.G + V - 1) / V) - 1;
+}
+__host__ __device__ __forceinline__ int tcs_first(TcSched s, int tile) { return tcs_cta_of(s, tile * s.upt); }
 __host__ __device__ __forceinline__ int tcs_nslots(TcSched s, int tile) {
     if (s.G == 0) return s.upt;
-    return tcs_cta_of(s, (long long)(tile + 1) * s.upt - 1) - tcs_first(s, tile) + 1;
+    return tcs_cta_of(s, (tile + 1) * s.upt - 1) - tcs_first(s, tile) + 1;
 }
 
 // tensor-core (tcgen05) contraction path state (rae_decoder_tc.cu)
@@ -107,6 +131,8 @@ struct TcState {
     bool dc2 = false; int dc_tile0 = 0, dc_tiles = 0; size_t smem_dc2 = 0;   // two-tile FP16 dC kernel on the bilinear rows; tiles left to the one-tile kernel
     float4* pop4 = nullptr; float* Rimg = nullptr; float* Yimg = nullptr;     // its q^T operand and the stage images of R, Y2
     int32_t* tile_slots = nullptr;   // [n_ntiles] partial slots of every 128-row tile of dC (device; k_dense_finalize)
+    int4* segs = nullptr;   // per-CTA (first unit, end unit, first slot) of every schedule, at these offsets (TcSegIter)
+    int segs_fwd = 0, segs_rec = 0, segs_dq = 0, segs_dc = 0, segs_dc2 = 0;
     float4* pop3 = nullptr; // q^T chunks [bc][hi/lo][8][NK]
     float* aT = nullptr; float* LT = nullptr; float* RT = nullptr; float* cT = nullptr; float* Y2T = nullptr;   // [dp][B] views
 };
