@@ -361,7 +361,7 @@ int rae_get_step_stats(rae_engine* h, rae_step_stats* out);
  *  0 encoder_forward   k_encoder_forward*                      8 contract_recompute  k_tc_bilinear (M c, M^T a)
  *  1 entity_sort       k_entity_keys + CUB radix sort          9 contract_dq         k_tc_transpose_al + k_tc_dq
  *  2 feature_sort      (cached at bind time: ~0)              10 backward_finish     k_tc_bwd_finish
- *  3 operand_prep      k_tc_prep_c + k_tc_prep_qt             11 contract_dc         k_tc_dc
+ *  3 operand_prep      k_tc_prep_c + k_tc_prep_qt             11 contract_dc         k_tc_dc2 (B % 4 != 0: k_tc_dc)
  *  4 contract_forward  k_tc_bilinear                          12 dense_finalize      k_dense_finalize
  *  5 score             k_score                                13 cost                k_cost (+ k_reg_norms)
  *  6 entity_update     k_rows_chunk<1> + k_entity_long2       14 dense_apply         k_dense_apply

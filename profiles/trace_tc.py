@@ -13,7 +13,8 @@ Slots per CTA (SM clock64 values, printed relative to the kernel's entry stamp):
         segment 2: 97 X/Y loads start | 98 X/Y loaded | 99 MMA thread sees the drained accumulator | 104 its first stage
         published | values: 96 segment count, 103 the CTA ends a tile
   dC   32 entry | 33 staging + setup | 38/39 MMA stage 8 ready / issued | 43/44 same, stage 24 | 40/41/42 generator warp 0
-        stage 8 | 35 all MMAs issued | 36 generators + drain done | 37 exit
+        stage 8 | 35 all MMAs issued | 36 generators + drain done | 37 exit |
+        values: 80 segment count, 81 the CTA's range holds stages of the selectional-preference pair (the last tile pair)
 """
 import ctypes as C, os, sys
 import numpy as np, torch
@@ -75,8 +76,10 @@ KERNELS = {
                 102: "first segment drain starts", 100: "SP stages start", 101: "SP stages published", 97: "seg 2: X/Y loads start",
                 98: "seg 2: X/Y loaded", 99: "seg 2: MMA sees drained acc", 104: "seg 2: first stage published"}, 96, 103),
     "dC": (32, {32: "entry", 33: "staging+setup done", 38: "mma s8 ready", 39: "mma s8 issued", 43: "mma s24 ready", 44: "mma s24 issued",
-                40: "gen s8 wait slot", 41: "gen s8 slot acquired", 42: "gen s8 published", 35: "all MMAs issued", 36: "gen+drain done", 37: "exit"}, None, None),
+                40: "gen s8 wait slot", 41: "gen s8 slot acquired", 42: "gen s8 published", 35: "all MMAs issued", 36: "gen+drain done", 37: "exit"}, 80, 81),
 }
+# what the second per-CTA value says (CTAs are grouped by segment count and by it)
+FLAG = {"dC": ("holds SP-pair stages", "bilinear pairs only")}
 for kname, (base, names, s_nseg, s_end) in KERNELS.items():
     live = [c for c in range(NCTA) if t[c, base] != 0]
     if not live:
@@ -99,13 +102,14 @@ for kname, (base, names, s_nseg, s_end) in KERNELS.items():
             groups.setdefault((int(t[c, s_nseg]), int(t[c, s_end])), []).append(c)
         for (n, e), cs in sorted(groups.items()):
             d = [life[c] for c in cs]
+            yes, no = FLAG.get(kname, ("ends a tile", "no tile end"))
             print("   %d segment(s), %s: %3d CTAs, life min/median/max = %d / %d / %d"
-                  % (n, "ends a tile" if e else "no tile end", len(cs), min(d), int(np.median(d)), max(d)))
+                  % (n, yes if e else no, len(cs), min(d), int(np.median(d)), max(d)))
     slowest = max(live, key=lambda c: life[c])
     median_cta = sorted(live, key=lambda c: life[c])[len(live) // 2]
     for tag, cta in (("first", live[0]), ("median life", median_cta), ("slowest", slowest)):
         r = t[cta]
-        extra = "" if s_nseg is None else ", %d segment(s)%s" % (r[s_nseg], ", ends a tile" if r[s_end] else "")
+        extra = "" if s_nseg is None else ", %d segment(s)%s" % (r[s_nseg], ", " + FLAG.get(kname, ("ends a tile",))[0] if r[s_end] else "")
         print("  CTA %d, %s (entry at +%d%s)" % (cta, tag, r[base] - t0, extra))
         for slot in sorted(names, key=lambda s: r[s]):
             if r[slot]:

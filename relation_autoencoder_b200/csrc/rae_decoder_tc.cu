@@ -16,8 +16,8 @@
 // K = 16 per MMA: the same 64 cycles per instruction as a K = 8 kind::tf32 MMA, profiles/microbench/mma_power.cu, so half
 // the MMAs): an fp16 has the 11-bit significand of a TF32, and its narrow exponent is handled by scaling every operand
 // tensor by an exact power of two chosen from its measured |max| (so that |x| s < 2^12: no overflow; a value whose lo part
-// falls into the fp16 subnormals is still exact to 2^-37 of the tensor's maximum), undone in the epilogue.  The dC
-// contraction still splits into TF32 pairs (kind::tf32).
+// falls into the fp16 subnormals is still exact to 2^-37 of the tensor's maximum), undone in the epilogue.  So does the dC
+// contraction (k_tc_dc2), except its fallback for B % 4 != 0 (k_tc_dc), which splits into TF32 pairs (kind::tf32).
 //
 // The M-side (A) operand lives in TMEM (TS mode): the threads that own a TMEM lane (= an example row b, or an output row
 // n) write their row with tcgen05.st - q rows once per segment for the forward, the generated operand G stage by stage for
@@ -52,7 +52,7 @@ namespace {
 
 // optional in-kernel timeline (build with -DRAE_TRACE, never part of the shipped library): SM cycle counter of CTA-local
 // milestones, [CTA][TC_TRACE_STRIDE] slots; forward kernel slots 0.., dq 16.., dC 32.., recompute pass 64.. (the forward
-// kernel's slots + 64), dq segment / selectional-preference stamps 96.. (see profiles/trace_tc.py)
+// kernel's slots + 64), dq segment / selectional-preference stamps 96.., dC segment values 80.. (see profiles/trace_tc.py)
 #ifdef RAE_TRACE
 constexpr int TC_TRACE_STRIDE = 128;
 __device__ unsigned long long* g_tc_trace = nullptr;
@@ -61,7 +61,6 @@ __device__ unsigned long long* g_tc_trace = nullptr;
 __device__ int g_tc_knock = 0;
 #define TC_KNOCK(bit) ((g_tc_knock & (bit)) != 0)
 #define TC_TRACE_INIT() unsigned long long* const tc_trace_ptr_ = g_tc_trace
-#define TC_TRACE_INIT_IF(cond) unsigned long long* const tc_trace_ptr_ = (cond) ? g_tc_trace : nullptr
 #define TC_TRACE(slot)                                                                                         \
     do {                                                                                                       \
         if (tc_trace_ptr_ != nullptr && (slot) < TC_TRACE_STRIDE) tc_trace_ptr_[(size_t)blockIdx.x * TC_TRACE_STRIDE + (slot)] = clock64(); \
@@ -99,7 +98,6 @@ __device__ int g_tc_knock = 0;
 #define TC_TRACE_SEGS(sch, slot_n, slot_end) do { } while (0)
 #define TC_TRACE_NS(slot) do { } while (0)
 #define TC_TRACE_INIT() do { } while (0)
-#define TC_TRACE_INIT_IF(cond) do { } while (0)
 #define TC_TRACE(slot) do { } while (0)
 #endif
 
@@ -286,7 +284,8 @@ __host__ __device__ __forceinline__ float pow2_scale(uint32_t amax_bits) {
 }
 constexpr float TC_QSCALE = 4096.f;        // q in [0, 1] -> [0, 2^12]
 // device scalars of the tensor path (TcState::scal, uint32 words)
-enum TcScal { TS_AMAX_C = 0, TS_AMAX_L = 1, TS_AMAX_R = 2, TS_AMAX_A = 3, TS_AMAX_CV = 4, TS_AMAX_Y2 = 5, TS_N = 8 };
+// (TS_AMAX_SP: the selectional-preference stage images of the dC kernel, a + G2 L | c + G1 R)
+enum TcScal { TS_AMAX_C = 0, TS_AMAX_L = 1, TS_AMAX_R = 2, TS_AMAX_A = 3, TS_AMAX_CV = 4, TS_AMAX_Y2 = 5, TS_AMAX_SP = 6, TS_N = 8 };
 
 // Global load that stays where it is written: a run of these is issued back to back (ptxas keeps volatile asm in program
 // order and cannot fold the consumers in between), so a thread's 32-64 row loads cost ONE memory latency.  Plain loads were
@@ -855,12 +854,14 @@ constexpr int TC_DQ_MAX_STAGES = 64;   // dq: stages (of 64 reduction rows) per 
 // tiled transposes: job z copies src[b * stride + c] (b < B, c < cols) to dst[c * B + b], zero rows for cols <= c < cols_out,
 // and folds |max| of the job's values into *amax (bits of a non-negative float; nullptr: skip).  They give the contraction
 // kernels their [column][example] views (lane = example reads are coalesced) and the scales of the FP16 operands.
-// img != 0: the destination is a stack of STAGE IMAGES [b / 64][c < cols_out][TC_IMG_LD] (64 examples per row, padded to 68
-// floats so that 16-byte shared-memory reads of consecutive rows are conflict-free): one contiguous block per stage that the
-// dC kernel fetches with a single bulk copy
+// img_rows != 0: the destination is a stack of STAGE IMAGES [b / 64][img_rows][TC_IMG_LD], the job's columns c in its first
+// rows (64 examples per row, padded to 68 floats so that 16-byte shared-memory reads of consecutive rows are
+// conflict-free): one contiguous block per stage that the dC kernel fetches with bulk copies.
+// src2 != nullptr: the job copies src + coef[b * SC_N] * src2 instead (both rounded, as the one-tile dC kernel's generator
+// rounds them): the selectional-preference rows a + G2 L, c + G1 R of the dC operand
 constexpr int TC_IMG_LD = 68;
-struct TrJob { const float* src; size_t stride; int cols, cols_out; float* dst; uint32_t* amax; int img; };
-struct TrJobs { TrJob j[4]; int B; };
+struct TrJob { const float* src; size_t stride; int cols, cols_out; float* dst; uint32_t* amax; int img_rows; const float* src2; const float* coef; };
+struct TrJobs { TrJob j[6]; int B; };
 __global__ void __launch_bounds__(256) k_tc_transpose(TrJobs jobs) {
     pdl_enter();
     __shared__ float tile[32][33];
@@ -872,7 +873,11 @@ __global__ void __launch_bounds__(256) k_tc_transpose(TrJobs jobs) {
     uint32_t m = 0;
     for (int r = ty; r < 32; r += 8) {
         const int b = b0 + r, c = c0 + tx;
-        const float v = (b < jobs.B && c < jb.cols) ? jb.src[(size_t)b * jb.stride + c] : 0.f;
+        float v = 0.f;
+        if (b < jobs.B && c < jb.cols) {
+            v = jb.src[(size_t)b * jb.stride + c];
+            if (jb.src2 != nullptr) v = __fadd_rn(v, __fmul_rn(jb.coef[(size_t)b * SC_N], jb.src2[(size_t)b * jb.stride + c]));
+        }
         tile[r][tx] = v;
         m = max(m, __float_as_uint(fabsf(v)));
     }
@@ -885,7 +890,7 @@ __global__ void __launch_bounds__(256) k_tc_transpose(TrJobs jobs) {
     for (int r = ty; r < 32; r += 8) {
         const int c = c0 + r, b = b0 + tx;
         if (c < jb.cols_out && b < jobs.B) {
-            if (jb.img) jb.dst[((size_t)(b >> 6) * jb.cols_out + c) * TC_IMG_LD + (b & 63)] = tile[tx][r];
+            if (jb.img_rows) jb.dst[((size_t)(b >> 6) * jb.img_rows + c) * TC_IMG_LD + (b & 63)] = tile[tx][r];
             else jb.dst[(size_t)c * jobs.B + b] = tile[tx][r];
         }
     }
@@ -899,13 +904,13 @@ __global__ void __launch_bounds__(256) k_tc_transpose(TrJobs jobs) {
 //   vT [2][dp][B]        DP=128: both epilogue groups hold a half-row partial; DP=64: group j%2; DP=32: group (j/2)%2
 //   wT [slot][2][dp][B]  sum over the slots of the example's tile (DP=128: only group j/64 holds column j; else both groups)
 //   spT [2][dp][B]       c1, c2 -> ev[b][E_C1 | E_C2][j] (forward pass only; nullptr otherwise)
-// zero_amax: the forward pass's combine also clears the |max| words the NEXT transposes (a, c, Y2) accumulate into
+// zero_amax: the forward pass's combine also clears the |max| words the NEXT transposes (a, c, Y2, the SP images) accumulate into
 __global__ void __launch_bounds__(256) k_tc_combine(const float* __restrict__ vT, const float* __restrict__ wT, const float* __restrict__ spT,
                                                     float* __restrict__ ev, int B, int d, int dp, int DP, TcSched sch, int slotV, int slotW,
                                                     uint32_t* __restrict__ zero_amax) {
     pdl_enter();
     __shared__ float tv[32][33], tw[32][33], t1[32][33], t2[32][33];
-    if (zero_amax != nullptr && blockIdx.x == 0 && blockIdx.y == 0 && threadIdx.x < 3) zero_amax[TS_AMAX_A + threadIdx.x] = 0u;
+    if (zero_amax != nullptr && blockIdx.x == 0 && blockIdx.y == 0 && threadIdx.x < 4) zero_amax[TS_AMAX_A + threadIdx.x] = 0u;
     const int b0 = blockIdx.x * 32, j0 = blockIdx.y * 32;
     const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
     const int ns = tcs_nslots(sch, b0 >> 7);                    // the 32 examples of a block share a 128-example tile
@@ -957,7 +962,7 @@ struct BwdBars {
     uint64_t* a_full; uint64_t* a_empty; uint64_t* b_full; uint64_t* b_empty; uint64_t* acc_full; uint64_t* acc_empty; uint32_t* tmem_slot;
 };
 
-__device__ __forceinline__ BwdBars bwd_setup(uint8_t* smem_raw, uint32_t ST_BYTES, int warp, uint32_t& tmem_base) {
+__device__ __forceinline__ BwdBars bwd_setup(uint8_t* smem_raw, uint32_t ST_BYTES, int warp, uint32_t& tmem_base, uint32_t drain_warps) {
     BwdBars br;
     uint64_t* bars = reinterpret_cast<uint64_t*>(smem_raw + TC_BSTAGES * ST_BYTES);
     br.a_full = bars;                 // [4] 16 generator-warp arrivals
@@ -965,13 +970,13 @@ __device__ __forceinline__ BwdBars bwd_setup(uint8_t* smem_raw, uint32_t ST_BYTE
     br.b_full = bars + 8;             // [4] bulk-copy tx
     br.b_empty = bars + 12;           // [4] tcgen05.commit
     br.acc_full = bars + 16;          // tcgen05.commit behind a segment's last MMA
-    br.acc_empty = bars + 17;         // 4 drain-warp arrivals: the accumulators may be overwritten by the next segment
+    br.acc_empty = bars + 17;         // drain-warp arrivals: the accumulators may be overwritten by the next segment
     br.tmem_slot = reinterpret_cast<uint32_t*>(bars + 18);
     if (threadIdx.x == 0) {
         for (int s = 0; s < 4; ++s) { mbar_init(&br.a_full[s], 16); mbar_init(&br.a_empty[s], 1); }
         for (int s = 0; s < 4; ++s) { mbar_init(&br.b_full[s], 1); mbar_init(&br.b_empty[s], 1); }
         mbar_init(br.acc_full, 1);
-        mbar_init(br.acc_empty, 4);
+        mbar_init(br.acc_empty, drain_warps);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     if (warp == TC_BWD_WORKERS + 2) {
@@ -1000,7 +1005,7 @@ __device__ __forceinline__ void bwd_produce(const BwdBars& br, uint8_t* smB, con
 // lt % nacc, whose first MMA overwrites; the commit behind the last stage signals acc_full
 template <int NAS>
 __device__ __forceinline__ void bwd_mma_segment(const BwdBars& br, uint8_t* smB, uint32_t ST_BYTES, int NK, uint32_t tmem_base, int nst,
-                                                int it0, int nacc, int trace_base) {
+                                                int it0, int nacc) {
     TC_TRACE_INIT();
     const uint32_t idesc = make_idesc_tf32(TC_M, NK);
     const uint32_t CH_BYTES = ST_BYTES / 2;
@@ -1009,8 +1014,8 @@ __device__ __forceinline__ void bwd_mma_segment(const BwdBars& br, uint8_t* smB,
         mbar_wait(&br.a_full[as], (git / NAS) & 1);
         mbar_wait(&br.b_full[s], (git / TC_BSTAGES) & 1);
         tc_fence_after();
-        if ((threadIdx.x & 31) == 0 && git == 8) TC_TRACE(trace_base + 6);
-        if ((threadIdx.x & 31) == 0 && git == 24) TC_TRACE(trace_base + 11);
+        if ((threadIdx.x & 31) == 0 && git == 8) TC_TRACE(38);
+        if ((threadIdx.x & 31) == 0 && git == 24) TC_TRACE(43);
         if (elect_one()) {
             const uint32_t a_hi = tmem_base + TC_BWD_ACOL + 128u * as, a_lo = a_hi + 64u;
             const uint32_t acc = tmem_base + ((nacc == 2 && (lt & 1)) ? TC_BWD_ACC2 : 0u);
@@ -1034,8 +1039,8 @@ __device__ __forceinline__ void bwd_mma_segment(const BwdBars& br, uint8_t* smB,
             if (lt == nst - 1) tc_commit(br.acc_full);
         }
         __syncwarp();
-        if ((threadIdx.x & 31) == 0 && git == 8) TC_TRACE(trace_base + 7);
-        if ((threadIdx.x & 31) == 0 && git == 24) TC_TRACE(trace_base + 12);
+        if ((threadIdx.x & 31) == 0 && git == 8) TC_TRACE(39);
+        if ((threadIdx.x & 31) == 0 && git == 24) TC_TRACE(44);
     }
 }
 
@@ -1140,7 +1145,7 @@ __global__ void __launch_bounds__(TC_BWD_THREADS, 1) k_tc_dq(TcDqArgs p) {
     uint8_t* smB = smem_raw;
     uint32_t tmem_base;
     if (threadIdx.x == 0) { TC_TRACE(16); TC_TRACE_NS(30); TC_TRACE_SEGS(p.sch, 96, 103); }
-    const BwdBars br = bwd_setup(smem_raw, ST_BYTES, warp, tmem_base);
+    const BwdBars br = bwd_setup(smem_raw, ST_BYTES, warp, tmem_base, TC_BWD_WORKERS);
     if (threadIdx.x == 0) TC_TRACE(17);
 
     if (warp >= TC_BWD_WORKERS) {
@@ -1280,13 +1285,15 @@ __global__ void __launch_bounds__(TC_BWD_THREADS, 1) k_tc_dq(TcDqArgs p) {
                 if (tr0 && lt == nst - 1) TC_TRACE(101);
             }
             it += nst;
-            if (gw < 4) {
-                // ===== epilogue: accumulator row -> dq partial of this segment's slot =====
+            {
+                // ===== epilogue: accumulator row -> dq partial of this segment's slot.  All 16 warps drain: warp (q4, cg)
+                // takes the 32-column chunks 32 cg, 32 cg + 128, ... of its lane quarter (NK <= 112: one chunk each), so the
+                // next segment's MMAs - and the CTA's exit - wait for a quarter of the tcgen05.ld / store sequence =====
                 mbar_wait(br.acc_full, seg & 1);
                 tc_fence_after();
                 if (tr0 && seg == 0) TC_TRACE(102);
                 float* o = p.dqT + (size_t)sg.slot * p.NK * p.B + (ok ? b : 0);
-                for (int c0 = 0; c0 < p.NK; c0 += 32) {
+                for (int c0 = 32 * cg; c0 < p.NK; c0 += 128) {
                     float t[32];
                     tc_ld32(lane_base + (uint32_t)c0, t);
                     if (ok) {
@@ -1312,7 +1319,8 @@ __global__ void __launch_bounds__(TC_BWD_THREADS, 1) k_tc_dq(TcDqArgs p) {
     }
 }
 
-// dC: rows = operand rows n (128-row tiles), reduction over examples in stages of 64.
+// dC: rows = operand rows n (128-row tiles), reduction over examples in stages of 64, TF32 pairs.  The whole-dC fallback of
+// the two-tile kernel below: it runs only where that one cannot (B % 4 != 0, or its stages do not fit in shared memory).
 struct TcDcArgs {
     const float4* pop3;     // q^T chunks [bc][hi/lo][8][NK]
     const float* ev; const float* sc; const float* aT; const float* LT;
@@ -1321,9 +1329,8 @@ struct TcDcArgs {
     int n_bil_rows, n_rows_total, hasM;
     int nacc;               // TMEM accumulators the example stages are dealt over (1 or 2)
     int share;              // most stages one CTA handles (sizes the per-example scalar staging)
-    int tile0;              // first 128-row tile this launch covers (the C1 / C2 tiles when k_tc_dc2 takes the bilinear rows)
     size_t split_stride;    // units*d*K
-    TcSched sch;            // units = stages of 64 examples, tiles = 128-row tiles of the operand rows (from tile0 on)
+    TcSched sch;            // units = stages of 64 examples, tiles = 128-row tiles of the operand rows
     const int4* segs;       // sch's per-CTA table (TcSegIter)
 };
 
@@ -1331,7 +1338,7 @@ __global__ void __launch_bounds__(TC_BWD_THREADS, 1) k_tc_dc(TcDcArgs p) {
     pdl_enter();
     extern __shared__ __align__(128) uint8_t smem_raw[];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    TC_TRACE_INIT_IF(p.tile0 == 0);      // (as the C1 / C2 helper of k_tc_dc2 it leaves the trace slots to that kernel)
+    TC_TRACE_INIT();
     constexpr int NAS = TC_DC_ASTAGES;
     const uint32_t ST_BYTES = 2u * 2u * 8u * (uint32_t)p.NK * 16u;
     uint8_t* smB = smem_raw;
@@ -1352,7 +1359,7 @@ __global__ void __launch_bounds__(TC_BWD_THREADS, 1) k_tc_dc(TcDcArgs p) {
             for (int idx = threadIdx.x; idx < nsrc * ne; idx += blockDim.x) {
                 const int src = idx / ne, bl = idx - src * ne;
                 const int b = sg.u0 * TC_SR + bl;
-                const int n0 = (sg.tile + p.tile0) * TC_M + src * p.DP;
+                const int n0 = sg.tile * TC_M + src * p.DP;
                 float v1 = 0.f, v2 = 0.f;
                 if (b < p.B) {
                     if (n0 < p.n_bil_rows) {
@@ -1370,7 +1377,7 @@ __global__ void __launch_bounds__(TC_BWD_THREADS, 1) k_tc_dc(TcDcArgs p) {
         }
     }
     uint32_t tmem_base;
-    const BwdBars br = bwd_setup(smem_raw, ST_BYTES, warp, tmem_base);  // __syncthreads inside: staging visible
+    const BwdBars br = bwd_setup(smem_raw, ST_BYTES, warp, tmem_base, 4);  // __syncthreads inside: staging visible
     if (threadIdx.x == 0) TC_TRACE(33);
 
     if (warp >= TC_BWD_WORKERS) {
@@ -1395,7 +1402,7 @@ __global__ void __launch_bounds__(TC_BWD_THREADS, 1) k_tc_dc(TcDcArgs p) {
                 mbar_wait(br.acc_empty, (seg - 1) & 1);
                 tc_fence_after();
             }
-            bwd_mma_segment<NAS>(br, smB, ST_BYTES, p.NK, tmem_base, sg.u1 - sg.u0, it, p.nacc, p.tile0 == 0 ? 32 : 64);
+            bwd_mma_segment<NAS>(br, smB, ST_BYTES, p.NK, tmem_base, sg.u1 - sg.u0, it, p.nacc);
             it += sg.u1 - sg.u0;
             ++seg;
         }
@@ -1411,7 +1418,7 @@ __global__ void __launch_bounds__(TC_BWD_THREADS, 1) k_tc_dc(TcDcArgs p) {
         TcSeg sg;
         int it = 0, seg = 0, off = 0;
         while (si.next(sg)) {
-            const int n = (sg.tile + p.tile0) * TC_M + row;
+            const int n = sg.tile * TC_M + row;
             // decode the row once: g(b) = P1(b) * X(b) + P2(b) * Y(b)
             int type = -1, i = 0, j = 0;          // -1: padding row (zero)
             if (n < p.n_bil_rows) {
@@ -1514,7 +1521,7 @@ __global__ void __launch_bounds__(TC_BWD_THREADS, 1) k_tc_dc(TcDcArgs p) {
 }
 
 // ------------------------------------------------------------------------------------------------------------
-// dC of the bilinear rows, FP16 pairs, TWO 128-row tiles per CTA (rows n of tiles 2 tp and 2 tp + 1: the same columns j,
+// dC, FP16 pairs, TWO 128-row tiles per CTA (rows n of tiles 2 tp and 2 tp + 1: the same columns j,
 // different rows i): every R_bj / Y2_bj the generators read serves both tiles, and nothing in the loop is a per-thread
 // global load - the one-tile kernel above spent its time on lane-strided L2 reads (47 % of the MMA floor, in-kernel trace).
 //   per stage of 64 examples: bulk copies bring the stage images of R and Y2 ([j][64 examples], rows padded to 68 floats),
@@ -1523,7 +1530,10 @@ __global__ void __launch_bounds__(TC_BWD_THREADS, 1) k_tc_dc(TcDcArgs p) {
 //   per stage, both tiles; TMEM: accumulators [0,128) (tile A) and [128,256) (tile B), A stage s: tile t at
 //   [256 + 128 s + 64 t, +64) = 32 packed hi + 32 packed lo columns.  One accumulator per tile: a segment never exceeds
 //   TC_DC2_MAX_STAGES stages = 384 MMAs per accumulator (the chain bound of profiles/r01_accum_chain.md).
-// Needs B % 4 == 0 (16-byte aligned slices of the transposed copies); other batches and the C1 / C2 rows use k_tc_dc.
+// The last pair of the schedule (n_bil_pairs) is the selectional-preference pair: its stage image holds the generated rows
+// themselves, C1 rows a + G2 L then C2 rows c + G1 R ([2 DP][TC_IMG_LD], built by the transposes after scoring), so its
+// generators only scale them; DP = 128: tile A = C1, tile B = C2; DP <= 64: both in tile A.
+// Needs B % 4 == 0 (16-byte aligned slices of the transposed copies); other batches use k_tc_dc.
 // ------------------------------------------------------------------------------------------------------------
 constexpr int TC_DC2_BSTAGES = 3;      // q^T operand stages (28 KB each at K = 100)
 constexpr int TC_DC2_XSTAGES = 2;      // image stages (R, Y2: 34 KB each at d = 128, + scalars)
@@ -1533,13 +1543,14 @@ constexpr uint32_t TC_DC2_ACOL = 256;
 struct TcDc2Args {
     const uint4* pop4;      // q^T stages [st][hi/lo][oct 0..7][NK] x 16 B
     const float* Rimg; const float* Yimg;     // stage images [st][j < DP][TC_IMG_LD]
+    const float* SPimg;                       // selectional-preference stage images [st][C1 j < DP | C2 j < DP][TC_IMG_LD]
     const float* aT; const float* LT;         // [dp][B] (+ 64 floats of slack)
     float* out;             // gC_part [slot][units*d*K]
     const uint32_t* scal; float g_bound;
     int B, d, dp, K, NK, DP;
-    int n_bil_tiles;
+    int n_bil_tiles, n_bil_pairs;
     size_t split_stride;
-    TcSched sch;            // units = stages of 64 examples, tiles = PAIRS of 128-row tiles
+    TcSched sch;            // units = stages of 64 examples, tiles = PAIRS of 128-row tiles (then the SP pair, if any)
     const int4* segs;       // sch's per-CTA table (TcSegIter)
 };
 
@@ -1563,14 +1574,24 @@ __global__ void __launch_bounds__(TC_BWD_THREADS, 1) k_tc_dc2(TcDc2Args p) {
     uint64_t* x_full = bars + 10;       // [2] bulk-copy tx
     uint64_t* x_empty = bars + 12;      // [2] 16 generator-warp arrivals (their reads of the stage are done)
     uint64_t* acc_full = bars + 14;
-    uint64_t* acc_empty = bars + 15;    // 4 drain-warp arrivals
+    uint64_t* acc_empty = bars + 15;    // 16 drain-warp arrivals
     uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 16);
     if (threadIdx.x == 0) { TC_TRACE(32); TC_TRACE_NS(46); }
+#ifdef RAE_TRACE
+    if (threadIdx.x == 0) {      // segment count, and whether the CTA's range holds stages of the SP pair
+        TcSegIter si_(p.segs, p.sch.upt, blockIdx.x);
+        TcSeg sg_;
+        int n_ = 0, sp_ = 0;
+        while (si_.next(sg_)) { ++n_; sp_ |= sg_.tile == p.n_bil_pairs; }
+        TC_TRACE_VAL(80, n_);
+        TC_TRACE_VAL(81, sp_);
+    }
+#endif
     if (threadIdx.x == 0) {
         for (int i = 0; i < 2; ++i) { mbar_init(&a_full[i], 16); mbar_init(&a_empty[i], 1); mbar_init(&x_full[i], 1); mbar_init(&x_empty[i], 16); }
         for (int i = 0; i < 3; ++i) { mbar_init(&b_full[i], 1); mbar_init(&b_empty[i], 1); }
         mbar_init(acc_full, 1);
-        mbar_init(acc_empty, 4);
+        mbar_init(acc_empty, TC_BWD_WORKERS);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     if (warp == TC_BWD_WORKERS + 2) {
@@ -1602,13 +1623,15 @@ __global__ void __launch_bounds__(TC_BWD_THREADS, 1) k_tc_dc2(TcDc2Args p) {
             }
         }
     } else if (warp == TC_BWD_WORKERS + 3) {
-        // ===== producer of the image ring: R image, Y2 image, and the 64-example slices of a_i / L_i of the tiles' rows =====
+        // ===== producer of the image ring: R image, Y2 image, and the 64-example slices of a_i / L_i of the tiles' rows;
+        // for the SP pair its image alone (the same 2 IMG bytes) =====
         if (lane == 0) {
             TcSegIter si(p.segs, p.sch.upt, blockIdx.x);
             TcSeg sg;
             int it = 0;
             while (si.next(sg)) {
-                const int i0 = (2 * sg.tile * TC_M) / DP;          // first row i of tile A; tile B starts nsrc rows later
+                const bool sp = sg.tile == p.n_bil_pairs;
+                const int i0 = sp ? p.dp : (2 * sg.tile * TC_M) / DP;   // first row i of tile A; tile B starts nsrc rows later
                 for (int st = sg.u0; st < sg.u1; ++st, ++it) {
                     const int xs = it % TC_DC2_XSTAGES;
                     mbar_wait(&x_empty[xs], ((it / TC_DC2_XSTAGES) & 1) ^ 1);
@@ -1617,8 +1640,11 @@ __global__ void __launch_bounds__(TC_BWD_THREADS, 1) k_tc_dc2(TcDc2Args p) {
                         if (i0 + ts < p.dp) bytes += 512u;
                     mbar_expect_tx(&x_full[xs], bytes);
                     uint8_t* dst = smX + (size_t)xs * XST;
-                    bulk_g2s(dst, reinterpret_cast<const uint8_t*>(p.Rimg) + (size_t)st * IMG, IMG, &x_full[xs]);
-                    bulk_g2s(dst + IMG, reinterpret_cast<const uint8_t*>(p.Yimg) + (size_t)st * IMG, IMG, &x_full[xs]);
+                    const uint8_t* srcX = sp ? reinterpret_cast<const uint8_t*>(p.SPimg) + (size_t)st * 2 * IMG
+                                             : reinterpret_cast<const uint8_t*>(p.Rimg) + (size_t)st * IMG;
+                    const uint8_t* srcY = sp ? srcX + IMG : reinterpret_cast<const uint8_t*>(p.Yimg) + (size_t)st * IMG;
+                    bulk_g2s(dst, srcX, IMG, &x_full[xs]);
+                    bulk_g2s(dst + IMG, srcY, IMG, &x_full[xs]);
                     for (int ts = 0; ts < 2 * nsrc; ++ts) {
                         const int i = i0 + ts;                  // (tile, source) -> row i
                         if (i < p.dp) {
@@ -1637,7 +1663,7 @@ __global__ void __launch_bounds__(TC_BWD_THREADS, 1) k_tc_dc2(TcDc2Args p) {
             TcSeg sg;
             int it = 0, seg = 0;
             while (si.next(sg)) {
-                const bool hasB = 2 * sg.tile + 1 < p.n_bil_tiles;
+                const bool hasB = sg.tile == p.n_bil_pairs ? 2 * DP > TC_M : 2 * sg.tile + 1 < p.n_bil_tiles;
                 const int nst = sg.u1 - sg.u0;
                 if (seg > 0) {                                   // the previous segment's accumulators have been drained
                     mbar_wait(acc_empty, (seg - 1) & 1);
@@ -1699,25 +1725,35 @@ __global__ void __launch_bounds__(TC_BWD_THREADS, 1) k_tc_dc2(TcDc2Args p) {
         const int nl = q4 * 32 + lane;                          // row of the tile
         const int j = nl % DP, srcl = nl / DP;
         const uint32_t lane_base = tmem_base + ((uint32_t)(q4 * 32) << 16);
-        float sG, inv;
+        // operand scales (powers of two, undone in the epilogue): bilinear pairs from a bound of |a R + L Y2|, the SP pair
+        // from the |max| of its image
+        float sGb, invb, sGs, invs;
         {
             const float aL = __uint_as_float(p.scal[TS_AMAX_L]), aR = __uint_as_float(p.scal[TS_AMAX_R]);
             const float aA = __uint_as_float(p.scal[TS_AMAX_A]), aY = __uint_as_float(p.scal[TS_AMAX_Y2]);
-            sG = pow2_scale(__float_as_uint(fmaf(aA, aR, aL * aY)));
-            inv = 1.f / (sG * TC_QSCALE);
+            sGb = pow2_scale(__float_as_uint(fmaf(aA, aR, aL * aY)));
+            invb = 1.f / (sGb * TC_QSCALE);
+            sGs = pow2_scale(p.scal[TS_AMAX_SP]);
+            invs = 1.f / (sGs * TC_QSCALE);
         }
         TcSegIter si(p.segs, p.sch.upt, blockIdx.x);
         TcSeg sg;
         int it = 0, seg = 0;
         while (si.next(sg)) {
-            const bool hasB = 2 * sg.tile + 1 < p.n_bil_tiles;
-            const int iA = (2 * sg.tile * TC_M) / DP + srcl, iB = iA + nsrc;
-            const bool vA = iA < p.d && j < p.d, vB = hasB && iB < p.d && j < p.d;
+            // SP pair: image row nl + 128 t is C1 row j (nl < DP) or C2 row j (DP <= nl + 128 t < 2 DP), i.e. rows d and d + 1 of
+            // the slot block's [units][d][K] (the tensor path always has the bilinear units); tile A reads its C2 rows from
+            // the second image half, where the bilinear pairs keep Y2
+            const bool sp = sg.tile == p.n_bil_pairs;
+            const bool hasB = sp ? 2 * DP > TC_M : 2 * sg.tile + 1 < p.n_bil_tiles;
+            const int iA = sp ? p.d + srcl : (2 * sg.tile * TC_M) / DP + srcl, iB = iA + nsrc;
+            const bool vA = (sp ? srcl < 2 : iA < p.d) && j < p.d, vB = hasB && (sp || iB < p.d) && j < p.d;
+            const float sG = sp ? sGs : sGb, inv = sp ? invs : invb;
+            const int xrow = (sp && srcl == 1) ? nl : j;
             const int nst = sg.u1 - sg.u0;
             for (int lt = 0; lt < nst; ++lt) {
                 const int git = it + lt, xs = git & 1, as = git & 1;
                 const uint8_t* stg = smX + (size_t)xs * XST;
-                const float* Xr = reinterpret_cast<const float*>(stg) + (size_t)j * TC_IMG_LD + 16 * cg;
+                const float* Xr = reinterpret_cast<const float*>(stg) + (size_t)xrow * TC_IMG_LD + 16 * cg;
                 const float* Yr = reinterpret_cast<const float*>(stg + IMG) + (size_t)j * TC_IMG_LD + 16 * cg;
                 const float* Pa = reinterpret_cast<const float*>(stg + 2 * IMG) + (size_t)srcl * 128 + 16 * cg;     // tile A: [a | L]
                 const float* Pb = Pa + (size_t)nsrc * 128;                                                             // tile B
@@ -1735,18 +1771,26 @@ __global__ void __launch_bounds__(TC_BWD_THREADS, 1) k_tc_dc2(TcDc2Args p) {
                     y[4 * v4] = yv.x * sG; y[4 * v4 + 1] = yv.y * sG; y[4 * v4 + 2] = yv.z * sG; y[4 * v4 + 3] = yv.w * sG;
                 }
                 float gA[16], gB[16];
+                if (sp) {                                        // the image rows are the operand (zero beyond B)
 #pragma unroll
-                for (int v4 = 0; v4 < 4; ++v4) {
-                    const float4 a1 = *reinterpret_cast<const float4*>(Pa + 4 * v4), l1 = *reinterpret_cast<const float4*>(Pa + 64 + 4 * v4);
-                    const float4 a2 = *reinterpret_cast<const float4*>(Pb + 4 * v4), l2 = *reinterpret_cast<const float4*>(Pb + 64 + 4 * v4);
-                    const float pa[4] = {a1.x, a1.y, a1.z, a1.w}, pl[4] = {l1.x, l1.y, l1.z, l1.w};
-                    const float qa[4] = {a2.x, a2.y, a2.z, a2.w}, ql[4] = {l2.x, l2.y, l2.z, l2.w};
+                    for (int e = 0; e < 16; ++e) {
+                        gA[e] = (vA && !TC_KNOCK(4)) ? x[e] : 0.f;
+                        gB[e] = (vB && !TC_KNOCK(4)) ? y[e] : 0.f;
+                    }
+                } else {
 #pragma unroll
-                    for (int u = 0; u < 4; ++u) {
-                        const int e = 4 * v4 + u;
-                        const bool in = full || b0 + e < p.B;
-                        gA[e] = (vA && in && !TC_KNOCK(4)) ? fmaf(pa[u], x[e], pl[u] * y[e]) : 0.f;
-                        gB[e] = (vB && in && !TC_KNOCK(4)) ? fmaf(qa[u], x[e], ql[u] * y[e]) : 0.f;
+                    for (int v4 = 0; v4 < 4; ++v4) {
+                        const float4 a1 = *reinterpret_cast<const float4*>(Pa + 4 * v4), l1 = *reinterpret_cast<const float4*>(Pa + 64 + 4 * v4);
+                        const float4 a2 = *reinterpret_cast<const float4*>(Pb + 4 * v4), l2 = *reinterpret_cast<const float4*>(Pb + 64 + 4 * v4);
+                        const float pa[4] = {a1.x, a1.y, a1.z, a1.w}, pl[4] = {l1.x, l1.y, l1.z, l1.w};
+                        const float qa[4] = {a2.x, a2.y, a2.z, a2.w}, ql[4] = {l2.x, l2.y, l2.z, l2.w};
+#pragma unroll
+                        for (int u = 0; u < 4; ++u) {
+                            const int e = 4 * v4 + u;
+                            const bool in = full || b0 + e < p.B;
+                            gA[e] = (vA && in && !TC_KNOCK(4)) ? fmaf(pa[u], x[e], pl[u] * y[e]) : 0.f;
+                            gB[e] = (vB && in && !TC_KNOCK(4)) ? fmaf(qa[u], x[e], ql[u] * y[e]) : 0.f;
+                        }
                     }
                 }
                 // this warp's reads of the image stage are done (the values above depend on every one of them)
@@ -1775,8 +1819,9 @@ __global__ void __launch_bounds__(TC_BWD_THREADS, 1) k_tc_dc2(TcDc2Args p) {
                 if (tr) TC_TRACE(42);
             }
             it += nst;
-            if (gw < 4) {
-                // ===== epilogue: both tiles' accumulator rows -> the segment's slot of the partial gradient =====
+            {
+                // ===== epilogue: both tiles' accumulator rows -> the segment's slot of the partial gradient, drained by all
+                // 16 warps (warp (q4, cg): the 32-column chunks 32 cg, 32 cg + 128, ... of its lane quarter, as in k_tc_dq) =====
                 mbar_wait(acc_full, seg & 1);
                 tc_fence_after();
 #pragma unroll
@@ -1785,7 +1830,7 @@ __global__ void __launch_bounds__(TC_BWD_THREADS, 1) k_tc_dc2(TcDc2Args p) {
                     const bool valid = t == 0 ? vA : vB;
                     if (t == 1 && !hasB) break;
                     float* o = p.out + (size_t)sg.slot * p.split_stride + ((size_t)i * p.d + j) * p.K;
-                    for (int c0 = 0; c0 < p.NK; c0 += 32) {
+                    for (int c0 = 32 * cg; c0 < p.NK; c0 += 128) {
                         float tt[32];
                         tc_ld32(lane_base + 128u * t + (uint32_t)c0, tt);
 #pragma unroll
@@ -2047,6 +2092,45 @@ void tc_plan(TcState& t, int B, int K, int d, bool hasSP, int num_sms) {
     t.sch_dq = make_sched(t.ntile, n_st, num_sms, TC_DQ_MAX_STAGES, tc_cost(DP, 2, n_st - t.n_bil_rows / TC_M));
     t.slots_dq = sched_max_slots(t.sch_dq);
 }
+
+// the dC plan of a shape (after tc_plan; host arithmetic only).  The two-tile FP16 kernel takes every 128-row tile of the
+// operand rows - the bilinear tiles in pairs, then the C1 / C2 tiles as one more pair - when B % 4 == 0 and its stages fit
+// in shared memory; otherwise the one-tile kernel takes them all.  Uniform weights: a stage of the SP pair issues as many
+// MMAs as a bilinear pair's, except at DP <= 64 (half as many, one pair among 4 - 65).  -> tile_slots: the partial slots
+// of every tile (k_dense_finalize).  Returns 0, 1 when the backward operand stages do not fit in shared memory, 2 when the
+// one-tile kernel's staging area does not.
+int tc_plan_dc(TcState& t, int B, bool hasSP, int num_sms, int max_smem_optin, std::vector<int32_t>& tile_slots) {
+    const int DP = t.DP;
+    t.smem_dq = (size_t)TC_BSTAGES * (2 * 2 * 8 * t.NK * 16) + 256;
+    if (t.smem_dq > (size_t)max_smem_optin) return 1;
+    t.n_ntiles = t.n_rows_total / TC_M;
+    t.n_bst = (B + TC_SR - 1) / TC_SR;
+    // one-tile kernel: accuracy bound (see TC_DC_MAX_STAGES) and the capacity of the per-example scalar staging area
+    t.dc_nacc = 2;
+    const size_t per_stage = (size_t)(TC_M / DP) * 2 * TC_SR * sizeof(float);
+    const int cap = (int)(((size_t)max_smem_optin - t.smem_dq) / per_stage);
+    if (cap < 1) return 2;
+    // the two-tile kernel needs 16-byte aligned slices of the transposed copies
+    const int n_bil_tiles = t.n_bil_rows / TC_M, n_bil_pairs = (n_bil_tiles + 1) / 2;
+    t.dc2 = (B % 4 == 0) && n_bil_tiles > 0;
+    t.smem_dc2 = (size_t)TC_DC2_BSTAGES * (2 * 8 * t.NK * 16) + (size_t)TC_DC2_XSTAGES * (2 * (size_t)DP * TC_IMG_LD * 4 + 2 * (TC_M / DP) * 2 * 256) + 256;
+    if (t.smem_dc2 > (size_t)max_smem_optin) t.dc2 = false;
+    t.dc_tiles = t.dc2 ? 0 : t.n_ntiles;
+    t.dc_share = 0;
+    tile_slots.assign((size_t)t.n_ntiles, 1);
+    if (t.dc2) {
+        t.sch_dc2 = make_sched(n_bil_pairs + (hasSP ? 1 : 0), t.n_bst, num_sms, TC_DC2_MAX_STAGES);
+        t.slots_dc = sched_max_slots(t.sch_dc2);
+        for (int nt = 0; nt < t.n_ntiles; ++nt) tile_slots[nt] = tcs_nslots(t.sch_dc2, nt < n_bil_tiles ? nt / 2 : n_bil_pairs);
+    } else {
+        t.sch_dc = make_sched(t.dc_tiles, t.n_bst, num_sms, std::min(t.dc_nacc * TC_DC_MAX_STAGES, cap));
+        t.dc_share = sched_max_share(t.sch_dc);
+        t.slots_dc = sched_max_slots(t.sch_dc);
+        for (int nt = 0; nt < t.n_ntiles; ++nt) tile_slots[nt] = tcs_nslots(t.sch_dc, nt);
+    }
+    t.smem_dc = t.smem_dq + (size_t)t.dc_share * per_stage;
+    return 0;
+}
 }  // namespace
 
 // The schedule tc_plan builds for one pass (0 forward, 1 recompute, 2 dq), for the tests: its seven fields
@@ -2083,6 +2167,29 @@ extern "C" int rae_debug_tc_make_sched(int ntile, int upt, int num_sms, int max_
     return s.G;
 }
 
+// The dC plan tc_init builds, for the tests: info[4] = {two-tile kernel runs, bilinear 128-row tiles, all row tiles,
+// slots_dc}, the fields of the launched kernel's schedule -> sched[7] (as above), the first unit of every CTA and the end
+// -> starts[G + 1] (when max_starts >= G + 1) and the partial slots of every row tile -> tile_slots[n_ntiles] (when
+// max_tiles >= n_ntiles).  Returns G, or -1 for a shape the tensor path does not take or whose dC stages do not fit in
+// max_smem_optin bytes.  Host only: needs no device.
+extern "C" int rae_debug_tc_dc_plan(int B, int K, int d, int hasSP, int num_sms, int max_smem_optin, int32_t* info, int32_t* sched,
+                                    int64_t* starts, int max_starts, int32_t* tile_slots, int max_tiles) {
+    if (B < 1 || K < 1 || K > 104 || d <= 16 || d > 128 || num_sms < 1) return -1;
+    TcState t;
+    std::vector<int32_t> ts;
+    tc_plan(t, B, K, d, hasSP != 0, num_sms);
+    if (tc_plan_dc(t, B, hasSP != 0, num_sms, max_smem_optin, ts) != 0) return -1;
+    const TcSched s = t.dc2 ? t.sch_dc2 : t.sch_dc;
+    const int in[4] = {t.dc2 ? 1 : 0, t.n_bil_rows / TC_M, t.n_ntiles, t.slots_dc};
+    if (info != nullptr) std::copy(in, in + 4, info);
+    const int f[7] = {s.G, s.upt, s.ntile, s.ntail, s.wb, s.wt, s.h};
+    if (sched != nullptr) std::copy(f, f + 7, sched);
+    if (starts != nullptr && max_starts >= s.G + 1)
+        for (int x = 0; x <= s.G; ++x) starts[x] = tcs_start(s, x);
+    if (tile_slots != nullptr && max_tiles >= t.n_ntiles) std::copy(ts.begin(), ts.end(), tile_slots);
+    return s.G;
+}
+
 int tc_init(rae_engine* h) {
     TcState& t = h->tc;
     tc_plan(t, h->B, h->K, h->d, h->hasSP, h->num_sms);
@@ -2094,34 +2201,12 @@ int tc_init(rae_engine* h) {
     t.smem = (size_t)t.fwd_stages * b_bytes + 256;
     const int n_st = t.n_rows_total / TC_M;
     const size_t st_bytes = (size_t)2 * 2 * 8 * t.NK * 16;
-    t.smem_dq = (size_t)TC_BSTAGES * st_bytes + 256;
-    if (t.smem_dq > (size_t)h->max_smem_optin) return fail(h, RAE_EINVAL, "tensor path: backward operand stages do not fit in shared memory");
-    t.n_ntiles = t.n_rows_total / TC_M;
-    t.n_bst = (h->B + TC_SR - 1) / TC_SR;
-    // dC: accuracy bound (see TC_DC_MAX_STAGES) and the capacity of the per-example scalar staging area
-    t.dc_nacc = 2;
-    const size_t per_stage = (size_t)(TC_M / DP) * 2 * TC_SR * sizeof(float);
-    const int cap = (int)(((size_t)h->max_smem_optin - t.smem_dq) / per_stage);
-    if (cap < 1) return fail(h, RAE_EINVAL, "tensor path: no shared memory left for the dC staging area");
-    // the bilinear rows go to the two-tile FP16 kernel (needs 16-byte aligned slices of the transposed copies: B % 4 == 0);
-    // the C1 / C2 tiles - and everything when that kernel cannot run - to the one-tile kernel
-    const int n_bil_tiles = t.n_bil_rows / TC_M;
-    t.dc2 = (h->B % 4 == 0) && n_bil_tiles > 0;
-    t.smem_dc2 = (size_t)TC_DC2_BSTAGES * (2 * 8 * t.NK * 16) + (size_t)TC_DC2_XSTAGES * (2 * (size_t)DP * TC_IMG_LD * 4 + 2 * (TC_M / DP) * 2 * 256) + 256;
-    if (t.smem_dc2 > (size_t)h->max_smem_optin) t.dc2 = false;
-    t.dc_tile0 = t.dc2 ? n_bil_tiles : 0;
-    t.slots_dc = 1;
-    if (t.dc2) {
-        t.sch_dc2 = make_sched((n_bil_tiles + 1) / 2, t.n_bst, h->num_sms, TC_DC2_MAX_STAGES);
-        t.slots_dc = sched_max_slots(t.sch_dc2);
-    }
-    t.dc_tiles = t.n_ntiles - t.dc_tile0;                    // tiles left to the one-tile kernel (may be none: model A)
-    if (t.dc_tiles > 0) {
-        t.sch_dc = make_sched(t.dc_tiles, t.n_bst, h->num_sms, std::min(t.dc_nacc * TC_DC_MAX_STAGES, cap));
-        t.dc_share = sched_max_share(t.sch_dc);
-        t.slots_dc = std::max(t.slots_dc, sched_max_slots(t.sch_dc));
-    }
-    t.smem_dc = t.smem_dq + (size_t)t.dc_share * per_stage;
+    std::vector<int32_t> ts;
+    const int rc = tc_plan_dc(t, h->B, h->hasSP, h->num_sms, h->max_smem_optin, ts);
+    if (rc == 1) return fail(h, RAE_EINVAL, "tensor path: backward operand stages do not fit in shared memory");
+    if (rc == 2) return fail(h, RAE_EINVAL, "tensor path: no shared memory left for the dC staging area");
+    const bool sp_img = t.dc2 && h->hasSP;
+    const size_t sp_img_bytes = (size_t)t.n_bst * 2 * DP * TC_IMG_LD * sizeof(float);
     cudaError_t e;
     const size_t vec = (size_t)h->dp * h->B * sizeof(float);
     if ((e = cudaMalloc((void**)&t.bop, (size_t)t.n_chunks_fwd * b_bytes)) != cudaSuccess ||
@@ -2139,20 +2224,16 @@ int tc_init(rae_engine* h) {
         (e = cudaMalloc((void**)&t.Yimg, (size_t)t.n_bst * DP * TC_IMG_LD * sizeof(float))) != cudaSuccess ||
         (e = cudaMemset(t.Rimg, 0, (size_t)t.n_bst * DP * TC_IMG_LD * sizeof(float))) != cudaSuccess ||
         (e = cudaMemset(t.Yimg, 0, (size_t)t.n_bst * DP * TC_IMG_LD * sizeof(float))) != cudaSuccess ||
+        (sp_img && (e = cudaMalloc((void**)&t.SPimg, sp_img_bytes)) != cudaSuccess) ||
+        (sp_img && (e = cudaMemset(t.SPimg, 0, sp_img_bytes)) != cudaSuccess) ||
         (e = cudaMalloc((void**)&t.RT, vec)) != cudaSuccess || (e = cudaMalloc((void**)&t.cT, vec)) != cudaSuccess ||
         (e = cudaMalloc((void**)&t.Y2T, vec)) != cudaSuccess ||
         (e = cudaMalloc((void**)&t.scal, TS_N * sizeof(uint32_t))) != cudaSuccess ||
         (e = cudaMemset(t.scal, 0, TS_N * sizeof(uint32_t))) != cudaSuccess)
         return fail(h, RAE_ENOMEM, "tensor-path workspace: %s", cudaGetErrorString(e));
-    {
-        // partial slots of every 128-row tile: the pair's count for tiles of the two-tile kernel, the tile's own otherwise
-        std::vector<int32_t> ts((size_t)t.n_ntiles, 1);
-        for (int nt = 0; nt < t.n_ntiles; ++nt)
-            ts[nt] = (t.dc2 && nt < n_bil_tiles) ? tcs_nslots(t.sch_dc2, nt / 2) : tcs_nslots(t.sch_dc, nt - t.dc_tile0);
-        if ((e = cudaMalloc((void**)&t.tile_slots, ts.size() * sizeof(int32_t))) != cudaSuccess ||
-            (e = cudaMemcpy(t.tile_slots, ts.data(), ts.size() * sizeof(int32_t), cudaMemcpyHostToDevice)) != cudaSuccess)
-            return fail(h, RAE_ENOMEM, "tensor-path workspace: %s", cudaGetErrorString(e));
-    }
+    if ((e = cudaMalloc((void**)&t.tile_slots, ts.size() * sizeof(int32_t))) != cudaSuccess ||
+        (e = cudaMemcpy(t.tile_slots, ts.data(), ts.size() * sizeof(int32_t), cudaMemcpyHostToDevice)) != cudaSuccess)
+        return fail(h, RAE_ENOMEM, "tensor-path workspace: %s", cudaGetErrorString(e));
     {
         // per-CTA tables of the five schedules (TcSegIter): first unit, end unit, slot of the first segment
         std::vector<int4> tab;
@@ -2185,7 +2266,7 @@ int tc_init(rae_engine* h) {
 
 void tc_free(rae_engine* h) {
     TcState& t = h->tc;
-    cudaFree(t.bop); cudaFree(t.pimg); cudaFree(t.vT); cudaFree(t.wT); cudaFree(t.spT); cudaFree(t.bop2); cudaFree(t.dqT); cudaFree(t.pop3); cudaFree(t.scal); cudaFree(t.pop4); cudaFree(t.Rimg); cudaFree(t.Yimg); cudaFree(t.tile_slots); cudaFree(t.segs);
+    cudaFree(t.bop); cudaFree(t.pimg); cudaFree(t.vT); cudaFree(t.wT); cudaFree(t.spT); cudaFree(t.bop2); cudaFree(t.dqT); cudaFree(t.pop3); cudaFree(t.scal); cudaFree(t.pop4); cudaFree(t.Rimg); cudaFree(t.Yimg); cudaFree(t.SPimg); cudaFree(t.tile_slots); cudaFree(t.segs);
     cudaFree(t.aT); cudaFree(t.LT); cudaFree(t.RT); cudaFree(t.cT); cudaFree(t.Y2T);
     t = TcState{};
 }
@@ -2207,19 +2288,27 @@ int tc_prepare_c(rae_engine* h, cudaStream_t st) {
 }
 
 namespace {
-// img_slot >= 0: that slot is ALSO written as the stack of stage images the two-tile dC kernel fetches
+// img_slot >= 0: that slot is ALSO written as the stack of stage images the two-tile dC kernel fetches; sp_img: so are the
+// selectional-preference rows a + G2 L, c + G1 R of its SP pair (after scoring: a, c and G1, G2 are final)
 int tc_transpose_slots(rae_engine* h, int n, const int* slots, float* const* dst, const int* amax_word, int img_slot,
-                       float* img_dst, cudaStream_t st) {
+                       float* img_dst, bool sp_img, cudaStream_t st) {
     TcState& t = h->tc;
     TrJobs jobs{};
     jobs.B = h->B;
     int nj = 0, maxc = 0;
     for (int i = 0; i < n; ++i) {
-        jobs.j[nj++] = TrJob{h->ev + (size_t)slots[i] * h->dp, (size_t)E_NV * h->dp, h->d, h->dp, dst[i], t.scal + amax_word[i], 0};
+        jobs.j[nj++] = TrJob{h->ev + (size_t)slots[i] * h->dp, (size_t)E_NV * h->dp, h->d, h->dp, dst[i], t.scal + amax_word[i], 0, nullptr, nullptr};
         maxc = std::max(maxc, h->dp);
     }
     if (img_slot >= 0 && t.dc2) {
-        jobs.j[nj++] = TrJob{h->ev + (size_t)img_slot * h->dp, (size_t)E_NV * h->dp, h->d, t.DP, img_dst, nullptr, 1};
+        jobs.j[nj++] = TrJob{h->ev + (size_t)img_slot * h->dp, (size_t)E_NV * h->dp, h->d, t.DP, img_dst, nullptr, t.DP, nullptr, nullptr};
+        maxc = std::max(maxc, t.DP);
+    }
+    if (sp_img && t.dc2 && h->hasSP) {
+        const size_t es = (size_t)E_NV * h->dp;
+        jobs.j[nj++] = TrJob{h->ev + (size_t)E_A * h->dp, es, h->d, t.DP, t.SPimg, t.scal + TS_AMAX_SP, 2 * t.DP, h->ev + (size_t)E_L * h->dp, h->sc + SC_G2};
+        jobs.j[nj++] = TrJob{h->ev + (size_t)E_CV * h->dp, es, h->d, t.DP, t.SPimg + (size_t)t.DP * TC_IMG_LD, t.scal + TS_AMAX_SP, 2 * t.DP,
+                             h->ev + (size_t)E_R * h->dp, h->sc + SC_G1};
         maxc = std::max(maxc, t.DP);
     }
     launch_pdl(k_tc_transpose, dim3((h->B + 31) / 32, (maxc + 31) / 32, nj), dim3(256), 0, st, jobs);
@@ -2243,7 +2332,7 @@ int tc_prepare_p(rae_engine* h, const int32_t* a1, const int32_t* a2, cudaStream
     const int slots[2] = {E_L, E_R};
     float* const dst[2] = {t.LT, t.RT};
     const int words[2] = {TS_AMAX_L, TS_AMAX_R};
-    return tc_transpose_slots(h, 2, slots, dst, words, E_R, t.Rimg, st);
+    return tc_transpose_slots(h, 2, slots, dst, words, E_R, t.Rimg, false, st);
 }
 
 // the q-dependent operand alone (only the dC contraction at the end of the step needs it: prepared off the critical path)
@@ -2291,7 +2380,7 @@ int tc_backward_recompute(rae_engine* h, cudaStream_t st) {
     const int slots[3] = {E_A, E_CV, E_Y2};
     float* const dst[3] = {t.aT, t.cT, t.Y2T};
     const int words[3] = {TS_AMAX_A, TS_AMAX_CV, TS_AMAX_Y2};
-    int rc = tc_transpose_slots(h, 3, slots, dst, words, E_Y2, t.Yimg, st);
+    int rc = tc_transpose_slots(h, 3, slots, dst, words, E_Y2, t.Yimg, true, st);
     if (rc) return rc;
     return tc_contract(h, t.aT, t.cT, E_GA1, E_GA2, false, st);
 }
@@ -2326,31 +2415,30 @@ int tc_backward_finish(rae_engine* h, cudaStream_t st) {
     return RAE_OK;
 }
 
-// dC, dC1, dC2 partials on the tensor path (k_dense_finalize sums the slots of every row tile / tile pair): the bilinear
-// rows through the two-tile FP16 kernel, the C1 / C2 tiles (or everything, when B % 4 != 0) through the one-tile kernel
+// dC, dC1, dC2 partials on the tensor path (k_dense_finalize sums the slots of every row tile / tile pair): every row tile
+// through the two-tile FP16 kernel, or (B % 4 != 0, or its stages do not fit) through the one-tile kernel
 int tc_grad_dense(rae_engine* h, cudaStream_t st) {
     TcState& t = h->tc;
     if (t.dc2) {
         TcDc2Args p{};
-        p.pop4 = reinterpret_cast<const uint4*>(t.pop4); p.Rimg = t.Rimg; p.Yimg = t.Yimg; p.aT = t.aT; p.LT = t.LT; p.out = h->gC_part;
+        p.pop4 = reinterpret_cast<const uint4*>(t.pop4); p.Rimg = t.Rimg; p.Yimg = t.Yimg; p.SPimg = t.SPimg; p.aT = t.aT; p.LT = t.LT; p.out = h->gC_part;
         p.scal = t.scal; p.g_bound = (float)((double)h->S / h->Z);
         p.B = h->B; p.d = h->d; p.dp = h->dp; p.K = h->K; p.NK = t.NK; p.DP = t.DP;
         p.n_bil_tiles = t.n_bil_rows / TC_M;
+        p.n_bil_pairs = (p.n_bil_tiles + 1) / 2;
         p.split_stride = (size_t)h->off_gWb;
         p.sch = t.sch_dc2;
         p.segs = t.segs + t.segs_dc2;
         launch_pdl(k_tc_dc2, dim3(p.sch.G), dim3(TC_BWD_THREADS), t.smem_dc2, st, p);
         h->launches++;
         RAE_CUDA(h, cudaGetLastError());
-    }
-    if (t.dc_tiles > 0) {
+    } else {
         TcDcArgs p{};
         p.pop3 = t.pop3; p.ev = h->ev; p.sc = h->sc; p.aT = t.aT; p.LT = t.LT; p.out = h->gC_part;
         p.B = h->B; p.d = h->d; p.dp = h->dp; p.K = h->K; p.NK = t.NK; p.DP = t.DP;
         p.n_bil_rows = t.n_bil_rows; p.n_rows_total = t.n_rows_total; p.hasM = h->hasM ? 1 : 0;
         p.nacc = t.dc_nacc;
         p.share = t.dc_share;
-        p.tile0 = t.dc_tile0;
         p.split_stride = (size_t)h->off_gWb;
         p.sch = t.sch_dc;
         p.segs = t.segs + t.segs_dc;

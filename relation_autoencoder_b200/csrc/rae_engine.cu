@@ -205,12 +205,14 @@ static int run_step(rae_engine* h, const int32_t* indptr, const int32_t* indices
         RAE_CUDA(h, cudaEventRecord(h->ev_fork1, st));
         RAE_CUDA(h, cudaStreamWaitEvent(h->s1, h->ev_fork1, 0));
         RAE_CUDA(h, cudaStreamWaitEvent(h->s2, h->ev_fork1, 0));
+        // (each side stream's last mark goes in before its join event, so that the step's "end" mark, recorded behind
+        // the joins, is never stamped before it when the side streams finish last)
         if ((rc = launch_entity_update(h, h->ent.keys_s, h->ent.vals_s, n_occ, h->emit_only, !h->emit_only, se))) return rc;
-        RAE_CUDA(h, cudaEventRecord(h->ev_join1, h->s1));
         RAE_MARK("entity_update", h->s1, 1);
+        RAE_CUDA(h, cudaEventRecord(h->ev_join1, h->s1));
         if ((rc = launch_w_update(h, f_keys_s, f_vals_s, nnz, emit, !h->emit_only, sw))) return rc;
-        RAE_CUDA(h, cudaEventRecord(h->ev_join2, h->s2));
         RAE_MARK("w_update", h->s2, 2);
+        RAE_CUDA(h, cudaEventRecord(h->ev_join2, h->s2));
     }
     RAE_PHASE();   // 11 dense-parameter gradients: dC contraction
     if (h->use_tc) {

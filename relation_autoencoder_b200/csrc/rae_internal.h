@@ -128,8 +128,9 @@ struct TcState {
     float4* bop2 = nullptr; // Cf^T chunks [c32][hi/lo][8][NK]
     float* dqT = nullptr;   // [slots_dq][NK][B]  dq partials, transposed
     int n_ntiles = 0, n_bst = 0, dc_nacc = 2, dc_share = 0;   // dC: 128-row tiles, 64-example stages, accumulators, stages per CTA
-    bool dc2 = false; int dc_tile0 = 0, dc_tiles = 0; size_t smem_dc2 = 0;   // two-tile FP16 dC kernel on the bilinear rows; tiles left to the one-tile kernel
+    bool dc2 = false; int dc_tiles = 0; size_t smem_dc2 = 0;   // two-tile FP16 dC kernel on every row tile; else the one-tile kernel's tiles
     float4* pop4 = nullptr; float* Rimg = nullptr; float* Yimg = nullptr;     // its q^T operand and the stage images of R, Y2
+    float* SPimg = nullptr;   // ... and of the selectional-preference rows [st][a + G2 L | c + G1 R][TC_IMG_LD] (hasSP only)
     int32_t* tile_slots = nullptr;   // [n_ntiles] partial slots of every 128-row tile of dC (device; k_dense_finalize)
     int4* segs = nullptr;   // per-CTA (first unit, end unit, first slot) of every schedule, at these offsets (TcSegIter)
     int segs_fwd = 0, segs_rec = 0, segs_dq = 0, segs_dc = 0, segs_dc2 = 0;
